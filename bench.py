@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the TC-ELBO hot path (BASELINE.json metric: "TC-ELBO fwd+bwd log-densities/s (B^2*D)").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--zdim D]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--zdim D] [--dump-outputs DIR]
 
 A "step" is one compute_kl_loss-equivalent evaluation (SURVEY.md 8d): reparameterize + KL + TC
 (minibatch stratified sampling) + (beta-1)*TC + KL, mean-reduced, and its backward to mu / logvar.
@@ -11,6 +11,11 @@ all-gathered over NCCL before the sweep and its gradient reduce-scattered after 
 
 Prints ONE JSON line on rank 0 (see the keys below).  `--impl reference` times the reference's own CPU implementation on the
 host cores: the unmodified ops.py staged under oracle/_ref by __graft_entry__.build() (the oracle port if that is absent).
+
+`--dump-outputs DIR` writes what the last timed step returned -- loss.npy (one entry per rank), grad_mu.npy and
+grad_logvar.npy ([B, D], rows in global order), all float32 -- so that two builds can be compared output for output on
+the same seeded inputs.  Gradients that would exceed 64 MB are reduced to a fixed seeded sample of rows, whose indices go to
+rows.npy.
 """
 from __future__ import annotations
 
@@ -27,6 +32,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np
 import torch
 
 METRIC = "tc_elbo_fwd_bwd_log_densities_per_s"
@@ -34,6 +40,7 @@ UNIT = "log-densities/s"
 DATASET_SIZE = 16704          # UkiyoE-sized N (SURVEY.md 8d)
 BETA = 0.5
 CPU_SAMPLE_B = 1024           # bounded CPU sample: B=1024, D=128 (the reference keeps 4*B^2*D*4 bytes = 2 GiB for backward)
+DUMP_BYTES = 64 * 10**6       # --dump-outputs budget
 
 
 def synthetic_latents(b, d, seed=1234):
@@ -187,6 +194,32 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_outputs(out_dir, loss, dmu, dlogvar, world, rank):
+    """Write one step's loss and gradients, gathered over the ranks, to out_dir on rank 0 (see --dump-outputs above)."""
+    import torch.distributed as dist
+    loss = loss.detach().reshape(1)
+    if world > 1:
+        parts = []
+        for t in (loss, dmu, dlogvar):
+            out = t.new_empty((world * t.shape[0],) + tuple(t.shape[1:]))
+            dist.all_gather_into_tensor(out, t.contiguous())
+            parts.append(out)
+        loss, dmu, dlogvar = parts
+    if rank != 0:
+        return
+    arrays = {"loss": loss, "grad_mu": dmu, "grad_logvar": dlogvar}
+    b, d = dmu.shape
+    # per kept row: two float32 gradient rows and a float64 index; 4 KiB for the loss and the .npy headers
+    keep = (DUMP_BYTES - 4096 - 4 * world) // (8 * d + 8)
+    if b > keep:
+        rows = torch.randperm(b, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        idx = rows.to(dmu.device)
+        arrays.update(grad_mu=dmu[idx], grad_logvar=dlogvar[idx], rows=rows.double())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------
@@ -293,10 +326,10 @@ def run_ours(args):
         solver.peer_exchange = PeerExchange(b_loc, D, group, dev)
 
     def run_step():
+        """-> (loss, grad_mu, grad_logvar) of this step."""
         if graphed is not None:
-            graphed.replay()
-        else:
-            step(mu, lv, eps)
+            return graphed.replay()
+        return step(mu, lv, eps), mu.grad, lv.grad
     for _ in range(3):
         run_step()
     barrier()
@@ -314,11 +347,13 @@ def run_ours(args):
     for k in range(args.steps):
         flush_buf.fill_(k & 0xFF)
         starts[k].record()
-        run_step()
+        outputs = run_step()
         stops[k].record()
     barrier()
     t_wall1 = time.perf_counter()
     launches = lib.tcelbo_launch_count() - launches0
+    if args.dump_outputs:                                  # before anything below reruns the step into the same buffers
+        dump_outputs(args.dump_outputs, *outputs, world, rank)
     if graphed is not None:                                # replayed launches do not pass through the host-side counter:
         c0 = lib.tcelbo_launch_count()                     # count the kernels of one eager issue of the captured step function
         graphed._step()
@@ -542,10 +577,10 @@ def run_ours(args):
             sys.path.insert(0, os.path.join(ROOT, "tools"))
             import train_bench
             if world == 1:
-                train = train_bench.measure(64, 128, 64, steps=20, warmup=5, dev=dev)
+                train = train_bench.measure(64, 128, 64, steps=args.steps, warmup=5, dev=dev)
                 train["config"] = "BASELINE configs[1] shape: 64x64x3 synthetic images, conv arch, z_dim 128, batch 64, fp32 (no AMP in the reference)"
             else:
-                train = train_bench.measure(128, 256, 32, steps=15, warmup=5, dev=dev, group=group, peer=(exchange_note == "peer"))
+                train = train_bench.measure(128, 256, 32, steps=args.steps, warmup=5, dev=dev, group=group, peer=(exchange_note == "peer"))
                 train["config"] = f"BASELINE configs[4] shape: 128x128x3 synthetic images, z_dim 256, beta_neg 512, batch 32 per GPU, data parallel x{world}"
         except Exception as exc:
             train = {"error": f"{type(exc).__name__}: {exc}"[:300]}
@@ -611,7 +646,12 @@ def main():
     ap.add_argument("--exchange", default="auto", choices=["auto", "peer", "nccl"],
                     help="N>1: how the column operand / its gradient cross ranks (peer memory inside the kernels, or NCCL)")
     ap.add_argument("--no-graph", action="store_true", help="issue every step eagerly instead of replaying a captured CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss and gradients of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

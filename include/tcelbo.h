@@ -46,7 +46,7 @@
 extern "C" {
 #endif
 
-#define TCELBO_VERSION 2
+#define TCELBO_VERSION 3
 
 /* flags */
 #define TCELBO_EST_MSS            0u   /* minibatch stratified sampling (active in the reference) */
@@ -282,13 +282,9 @@ int tcelbo_sampling_backward(const float* log_qz_prob, int b, int d, int64_t dat
 long long tcelbo_launch_count(void);
 /* Bracket every later launch of one kernel class (1 = forward sweep, 2 = backward row sweep,
  * 3 = backward column sweep, 0 = off) with cudaEventRecord(start) / cudaEventRecord(stop) on its stream;
- * the events are cudaEvent_t handles owned by the caller. */
+ * the events are cudaEvent_t handles owned by the caller.  Environment: TCELBO_PDL=0 launches the kernels without
+ * programmatic dependent launch. */
 int tcelbo_profile_events(int kernel_id, void* start_event, void* stop_event);
-/* Tuning points for tools/tune_bwd.py; 0 restores the shipped choice of every key.  Keys: "bwd_variant" (tuning points of the fused
- * backward sweep), "bwd_seg_tiles" / "fwd_seg_tiles" (column tiles per CTA of the balanced-segment grids), "fwd_map" (1 = round 1's 32 dims
- * per lane in the forward sweep), "fwd_wave" (CTAs per SM the forward grid is sized in waves of).  Unknown key:
- * TCELBO_ERR_INVALID.  Environment: TCELBO_PDL=0 launches the kernels without programmatic dependent launch. */
-int tcelbo_set_tuning(const char* key, int value);
 /* MUFU.EX2 saturation probe: `ctas` blocks of 256 threads, 8*iters dependent-chain ex2 per thread. */
 int tcelbo_ex2_peak(float* scratch, int iters, int ctas, void* stream);
 

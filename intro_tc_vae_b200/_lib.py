@@ -87,7 +87,6 @@ _SIGNATURES = {
     "tcelbo_sampling_backward": (c_int, [_f, c_int, c_int, c_int64, c_uint32, _f, _f, _f, _f, _f, _f, c_void_p]),
     "tcelbo_launch_count": (ctypes.c_longlong, []),
     "tcelbo_profile_events": (c_int, [c_int, c_void_p, c_void_p]),
-    "tcelbo_set_tuning": (c_int, [c_char_p, c_int]),
     "tcelbo_ex2_peak": (c_int, [_f, c_int, c_int, c_void_p]),
 }
 

@@ -42,7 +42,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     """Compile the CUDA sources into intro_tc_vae_b200/libtcelbo.so; returns its path."""
     if not force and not _stale():
         return LIB_PATH
-    extra = os.environ.get("TCELBO_NVCC_FLAGS", "").split()          # e.g. -DTCELBO_ABLATIONS for tools/tune_bwd.py
+    extra = os.environ.get("TCELBO_NVCC_FLAGS", "").split()          # extra nvcc flags, e.g. -Xptxas -warn-spills
     cmd = [_nvcc()] + NVCC_FLAGS + extra + (["-Xptxas", "-v"] if verbose else []) + ["-I", INCLUDE, "-I", CSRC]
     cmd += [os.path.join(CSRC, s) for s in SOURCES] + ["-o", LIB_PATH]
     res = subprocess.run(cmd, capture_output=True, text=True)

@@ -3,7 +3,6 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
-#include <cstring>
 #include <string>
 
 #include "tc_instr.h"
@@ -560,15 +559,6 @@ int tcelbo_profile_events(int kernel_id, void* start_event, void* stop_event) {
     in.ev_start = static_cast<cudaEvent_t>(start_event);
     in.ev_stop = static_cast<cudaEvent_t>(stop_event);
     return TCELBO_OK;
-}
-
-int tcelbo_set_tuning(const char* key, int value) {
-    if (key && std::strcmp(key, "bwd_variant") == 0) { set_bwd_variant(value); return TCELBO_OK; }
-    if (key && std::strcmp(key, "fwd_seg_tiles") == 0) { fwd_seg_target() = value; return TCELBO_OK; }
-    if (key && std::strcmp(key, "bwd_seg_tiles") == 0) { set_bwd_seg_target(value); return TCELBO_OK; }
-    if (key && std::strcmp(key, "fwd_map") == 0) { fwd_map_tuning() = value; return TCELBO_OK; }
-    if (key && std::strcmp(key, "fwd_wave") == 0) { fwd_wave_tuning() = value; return TCELBO_OK; }
-    return fail(TCELBO_ERR_INVALID, "unknown tuning key");
 }
 
 int tcelbo_ex2_peak(float* scratch, int iters, int ctas, void* stream) {

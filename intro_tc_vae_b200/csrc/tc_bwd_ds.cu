@@ -42,9 +42,6 @@ struct alignas(64) BwdDsArgs {
     Weights w;
 };
 
-__device__ __forceinline__ float fset_le_ds(float a, float b) {       // 1.0f if a <= b else 0.0f (FSET.BF)
-    float y; asm("set.le.f32.f32 %0, %1, %2;" : "=f"(y) : "f"(a), "f"(b)); return y;
-}
 __device__ __forceinline__ void red_add_f32(float* addr, float v) {
     asm volatile("red.global.add.f32 [%0], %1;" :: "l"(addr), "f"(v) : "memory");
 }
@@ -54,7 +51,7 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
 }
 
 // One column for this warp's RP row pairs (this lane's dim).  kSpecial: the tile holds a stratified or a padding column.
-template <int RP, bool kSpecial, bool MSEL>
+template <int RP, bool kSpecial>
 __device__ __forceinline__ float ds_column(float mu, const float* __restrict__ gq_col, int i_glob0, int j, const Weights& w,
                                            const u64 (&zs2)[RP], const u64 (&ns2)[RP], const float (&qmx)[2 * RP],
                                            const u64 (&gps2)[RP], u64 (&A2)[RP], u64 (&CR2)[RP]) {
@@ -79,14 +76,9 @@ __device__ __forceinline__ float ds_column(float mu, const float* __restrict__ g
             e2 = fmul2(e2, pack2(r0, r1));
         }
         const u64 coef2 = ffma2(e2, gps2[p], gq2);
-        u64 r2;
-        if (MSEL) {                                  // clamp mask as FSETP + FSEL on the ALU pipe (a NaN q gives r = 0, like torch.clamp's backward)
-            float k0, k1;
-            unpack2(coef2, k0, k1);
-            r2 = pack2(q0 <= qmx[2 * p] ? k0 : 0.0f, q1 <= qmx[2 * p + 1] ? k1 : 0.0f);
-        } else {                                     // FSET.BF + one packed multiply on the FMA pipe
-            r2 = fmul2(coef2, pack2(fset_le_ds(q0, qmx[2 * p]), fset_le_ds(q1, qmx[2 * p + 1])));
-        }
+        float k0, k1;                                // clamp mask as FSETP + FSEL on the ALU pipe (a NaN q gives r = 0, like torch.clamp's backward)
+        unpack2(coef2, k0, k1);
+        const u64 r2 = pack2(q0 <= qmx[2 * p] ? k0 : 0.0f, q1 <= qmx[2 * p + 1] ? k1 : 0.0f);
         const u64 t2 = fmul2(r2, dl2);
         A2[p] = fadd2(A2[p], t2);
         CR2[p] = ffma2(r2, q2, CR2[p]);
@@ -97,45 +89,7 @@ __device__ __forceinline__ float ds_column(float mu, const float* __restrict__ g
     return lo + hi;
 }
 
-// Two adjacent columns in lockstep: per row pair the two columns' chains are independent and share the row constants
-// (same zs2 / ns2 / gps2 operands in consecutive instructions), which doubles the instruction-level parallelism inside a warp.
-template <int RP>
-__device__ __forceinline__ void ds_column_x2(float mu_a, float mu_b, const float* __restrict__ gq_a, const float* __restrict__ gq_b,
-                                             const u64 (&zs2)[RP], const u64 (&ns2)[RP], const float (&qmx)[2 * RP],
-                                             const u64 (&gps2)[RP], u64 (&A2)[RP], u64 (&CR2)[RP], float& g_a, float& g_b) {
-    const u64 mua2 = pack2(mu_a, mu_a), mub2 = pack2(mu_b, mu_b);
-    const u64 nk2 = pack2(-kInvTwoLn2, -kInvTwoLn2);
-    u64 Ga = 0ull, Gb = 0ull;
-#pragma unroll
-    for (int p = 0; p < RP; ++p) {
-        const u64 gqa2 = *reinterpret_cast<const u64*>(gq_a + 2 * p);
-        const u64 gqb2 = *reinterpret_cast<const u64*>(gq_b + 2 * p);
-        const u64 dla2 = ffma2(mua2, ns2[p], zs2[p]);
-        const u64 dlb2 = ffma2(mub2, ns2[p], zs2[p]);
-        const u64 qa2 = ffma2(dla2, dla2, nk2);
-        const u64 qb2 = ffma2(dlb2, dlb2, nk2);
-        float qa0, qa1, qb0, qb1;
-        unpack2(qa2, qa0, qa1); unpack2(qb2, qb0, qb1);
-        const u64 ea2 = pack2(ex2(-qa0), ex2(-qa1));
-        const u64 eb2 = pack2(ex2(-qb0), ex2(-qb1));
-        const u64 ma2 = pack2(fset_le_ds(qa0, qmx[2 * p]), fset_le_ds(qa1, qmx[2 * p + 1]));
-        const u64 mb2 = pack2(fset_le_ds(qb0, qmx[2 * p]), fset_le_ds(qb1, qmx[2 * p + 1]));
-        const u64 ra2 = fmul2(ffma2(ea2, gps2[p], gqa2), ma2);
-        const u64 rb2 = fmul2(ffma2(eb2, gps2[p], gqb2), mb2);
-        const u64 ta2 = fmul2(ra2, dla2);
-        const u64 tb2 = fmul2(rb2, dlb2);
-        A2[p] = fadd2(A2[p], fadd2(ta2, tb2));
-        CR2[p] = ffma2(rb2, qb2, ffma2(ra2, qa2, CR2[p]));
-        Ga = ffma2(ta2, ns2[p], Ga);
-        Gb = ffma2(tb2, ns2[p], Gb);
-    }
-    float lo, hi;
-    unpack2(Ga, lo, hi); g_a = lo + hi;
-    unpack2(Gb, lo, hi); g_b = lo + hi;
-}
-
-// UNR: columns per basic block; X2: 1 = two columns in lockstep; MSEL: clamp mask by select (ALU pipe) instead of a packed multiply
-template <int RP, int CH, int NW, int MINB, int JT, int UNR, int X2, bool MSEL>
+template <int RP, int CH, int NW, int MINB, int JT>
 __global__ void __launch_bounds__(NW * 32, MINB)
 tc_bwd_ds_kernel(const __grid_constant__ BwdDsArgs a) {
     pdl_trigger(); pdl_wait();                               // programmatic dependent launch, tc_common.cuh
@@ -285,23 +239,14 @@ tc_bwd_ds_kernel(const __grid_constant__ BwdDsArgs a) {
         if (special) {
 #pragma unroll 2
             for (int jj = 0; jj < JT; ++jj) {
-                const float g = ds_column<RP, true, MSEL>(tile[jj * DPS], gq + jj * RW, a.row_offset + row0, jt0 + jj, a.w, zs2, ns2, qmx, gps2, A2, CR2);
+                const float g = ds_column<RP, true>(tile[jj * DPS], gq + jj * RW, a.row_offset + row0, jt0 + jj, a.w, zs2, ns2, qmx, gps2, A2, CR2);
                 red_add_f32(gptr, g);
                 gptr += pitch;
             }
-        } else if (X2 == 1) {
-#pragma unroll(UNR / 2)
-            for (int jj = 0; jj < JT; jj += 2) {
-                float ga, gb;
-                ds_column_x2<RP>(tile[jj * DPS], tile[(jj + 1) * DPS], gq + jj * RW, gq + (jj + 1) * RW, zs2, ns2, qmx, gps2, A2, CR2, ga, gb);
-                red_add_f32(gptr, ga);
-                red_add_f32(gptr + pitch, gb);
-                gptr += 2 * pitch;
-            }
         } else {
-#pragma unroll(UNR)
+#pragma unroll 8
             for (int jj = 0; jj < JT; ++jj) {
-                const float g = ds_column<RP, false, MSEL>(tile[jj * DPS], gq + jj * RW, 0, 0, a.w, zs2, ns2, qmx, gps2, A2, CR2);
+                const float g = ds_column<RP, false>(tile[jj * DPS], gq + jj * RW, 0, 0, a.w, zs2, ns2, qmx, gps2, A2, CR2);
                 red_add_f32(gptr, g);
                 gptr += pitch;
             }
@@ -342,15 +287,12 @@ static bool make_map_2d(CUtensorMap* m, const float* base, uint64_t rows, uint64
                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static int g_ds_seg_target = 0;
-void set_bwd_seg_target(int v) { g_ds_seg_target = v; }
-
-template <int RP, int CH, int NW, int MINB, int JT, int UNR = 8, int X2 = 0, bool MSEL = false>
+template <int RP, int CH, int NW, int MINB, int JT>
 static cudaError_t launch_bwd_ds_t(const Plan& p, const BwdFusedArgs& u, BwdFinArgs* fin, cudaStream_t st) {
     constexpr int ROWS = (NW / CH) * 2 * RP, DPS = 32 * CH;
     const size_t smem = ((size_t)kStages * JT * DPS + (size_t)kStages * ROWS * JT + (size_t)NW * JT * 2 * RP + (size_t)NW * 2 * RP * 2) * sizeof(float)
                         + 2 * kStages * sizeof(uint64_t);
-    auto kern = tc_bwd_ds_kernel<RP, CH, NW, MINB, JT, UNR, X2, MSEL>;
+    auto kern = tc_bwd_ds_kernel<RP, CH, NW, MINB, JT>;
     static PerDevice ctas_on;
     int& ctas_per_sm = ctas_on.cur();
     if (ctas_per_sm == 0) {
@@ -364,7 +306,7 @@ static cudaError_t launch_bwd_ds_t(const Plan& p, const BwdFusedArgs& u, BwdFinA
     const int n_rb = (p.bl_pad + ROWS - 1) / ROWS;
     const int n_slices = p.dp / DPS;
     const int T = p.bg_pad / JT;
-    const Segments seg = plan_segments((int64_t)n_rb * n_slices, T, p.sms * ctas_per_sm, g_ds_seg_target > 0 ? g_ds_seg_target : 2048 / JT);     // 128 tiles of 16 columns per CTA (profiles/r2_notes.md)
+    const Segments seg = plan_segments((int64_t)n_rb * n_slices, T, p.sms * ctas_per_sm, 2048 / JT);     // 128 tiles of 16 columns per CTA (profiles/r2_notes.md)
     fin->seg = seg; fin->tiles_per_block = T; fin->n_rb = n_rb; fin->rows_per_block = ROWS; fin->slice_dp = DPS;
     if (u.plan_only) return cudaSuccess;
     BwdDsArgs a;
@@ -547,32 +489,17 @@ __global__ void bwd_fused_finalize_v4_kernel(const BwdFinArgs a) {
     }
 }
 
-// variant 0 is the shipped configuration; the others are tuning points kept for tools/tune_bwd.py (profiles/r2_bwd_ds_sweep.md)
-static cudaError_t launch_bwd_ds(const Plan& p, const BwdFusedArgs& a, BwdFinArgs* fin, int variant, cudaStream_t st) {
-    if (p.small) {                       // B = 3 / 64-sized batches: 4 rows per warp so that row blocks x tiles covers more SMs
-        if (p.dp >= 128) return launch_bwd_ds_t<2, 4, 8, 2, 16, 8, false, true>(p, a, fin, st);
-        if (p.dp == 64) return launch_bwd_ds_t<2, 2, 8, 2, 16, 8, false, true>(p, a, fin, st);
-        return launch_bwd_ds_t<2, 1, 8, 2, 16, 8, false, true>(p, a, fin, st);
-    }
-    if (p.dp >= 128) {
-        switch (variant) {           // tools/tune_bwd.py: the tuning points that bracket the shipped one (profiles/r2_bwd_ds_sweep.md)
-            case 1:  return launch_bwd_ds_t<6, 4, 8, 2, 16, 8, false, true>(p, a, fin, st);    // 12 rows/warp, 16 warps/SM (128 regs)
-            case 2:  return launch_bwd_ds_t<5, 4, 8, 2, 16, 8, false, true>(p, a, fin, st);    // 10 rows/warp, 16 warps/SM
-            case 3:  return launch_bwd_ds_t<8, 4, 12, 1, 16, 8>(p, a, fin, st);                // shipped shape, clamp mask by multiply
-            case 4:  return launch_bwd_ds_t<6, 4, 8, 2, 16, 4, 1>(p, a, fin, st);              // two columns in lockstep
-            default: return launch_bwd_ds_t<8, 4, 12, 1, 16, 8, false, true>(p, a, fin, st);   // 16 rows/warp, 12 warps/SM (168 regs),
-        }                                                                                       // 8 columns per basic block, mask by select
-    }
-    if (p.dp == 64) return launch_bwd_ds_t<8, 2, 12, 1, 16, 8, false, true>(p, a, fin, st);
-    return launch_bwd_ds_t<8, 1, 12, 1, 16, 8, false, true>(p, a, fin, st);
-}
-
-
-static int g_bwd_variant = 0;       // 0: shipped configuration; set through tcelbo_set_tuning("bwd_variant", v) by tools/tune_bwd.py
-void set_bwd_variant(int v) { g_bwd_variant = v < 0 ? 0 : v; }
-
+// Shipped configurations; the measured alternatives they beat are in profiles/r2_bwd_ds_sweep.md
 cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, BwdFinArgs* fin, cudaStream_t st) {
-    return launch_bwd_ds(p, a, fin, g_bwd_variant, st);
+    if (p.small) {                       // B = 3 / 64-sized batches: 4 rows per warp so that row blocks x tiles covers more SMs
+        if (p.dp >= 128) return launch_bwd_ds_t<2, 4, 8, 2, 16>(p, a, fin, st);
+        if (p.dp == 64) return launch_bwd_ds_t<2, 2, 8, 2, 16>(p, a, fin, st);
+        return launch_bwd_ds_t<2, 1, 8, 2, 16>(p, a, fin, st);
+    }
+    // 16 rows per warp, 12 warps per SM (168 registers), 8 columns per basic block, clamp mask by select
+    if (p.dp >= 128) return launch_bwd_ds_t<8, 4, 12, 1, 16>(p, a, fin, st);
+    if (p.dp == 64) return launch_bwd_ds_t<8, 2, 12, 1, 16>(p, a, fin, st);
+    return launch_bwd_ds_t<8, 1, 12, 1, 16>(p, a, fin, st);
 }
 
 cudaError_t launch_bwd_fused_finalize(const Plan& p, const BwdFinArgs& a, cudaStream_t st) {

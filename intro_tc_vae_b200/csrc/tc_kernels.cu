@@ -232,8 +232,7 @@ __device__ __forceinline__ void fwd_tile(const float* __restrict__ tile, int jt,
 
 // JTS: columns per tile (0 = as many as fit kTileFloats, at most 32); KCH: 16-byte chunks (4 dims) per lane -- 4 in the shipped
 // mapping (16 dims per lane, 128 registers, 16 warps per SM), 8 (32 dims per lane, 168 registers, 3 CTAs of 4 warps per SM) in the
-// small-problem instantiation and the fwd_map = 1 tuning point; MINB: CTAs per SM; NWF: warps per CTA (8 for D >= 256, so that
-// a CTA keeps 16 / 8 rows)
+// small-problem instantiation; MINB: CTAs per SM; NWF: warps per CTA (8 for D >= 256, so that a CTA keeps 16 / 8 rows)
 template <int LPR, int JTS, int KCH = 8, int MINB = 3, int NWF = kFwdWarps>
 __global__ void __launch_bounds__(NWF * 32, MINB)
 tc_fwd_kernel(const FwdArgs a) {
@@ -252,7 +251,7 @@ tc_fwd_kernel(const FwdArgs a) {
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int l = lane % LPR, rw = lane / LPR;
-    // Work = row blocks x T column tiles, linearised block-major and cut into equal contiguous segments of a.seg_tiles
+    // Work = row blocks x T column tiles, linearised block-major and cut into equal contiguous segments of a.seg.base
     // (+1) tiles, one per CTA (tc_layout.h: plan_segments): every CTA carries the same load whatever the batch shape.  A
     // segment that crosses into the next row block flushes its partial sums and reloads the row constants.
     const int T = a.bg_pad / JT;
@@ -570,22 +569,12 @@ cudaError_t launch_fwd(const Plan& p, const FwdArgs& a, cudaStream_t st) {
             default: return cudaErrorInvalidValue;
         }
     }
-    if (p.fwd_kch == 4) {                // 16 dims per lane, 16 warps per SM (<= 128 registers)
-        switch (p.fwd_lpr) {
-            case 2:  return launch_fwd_t<2, 0, 4, 4>(p, a, st);
-            case 4:  return launch_fwd_t<4, 0, 4, 4>(p, a, st);
-            case 8:  return launch_fwd_t<8, 0, 4, 4>(p, a, st);
-            case 16: return launch_fwd_t<16, 0, 4, 2, 8>(p, a, st);      // D = 256 / 512: 8 warps per CTA keep 16 / 8 rows per CTA
-            case 32: return launch_fwd_t<32, 0, 4, 2, 8>(p, a, st);
-            default: return cudaErrorInvalidValue;
-        }
-    }
-    switch (p.dpt) {
-        case 1:  return launch_fwd_t<1, 0>(p, a, st);
-        case 2:  return launch_fwd_t<2, 0>(p, a, st);
-        case 4:  return launch_fwd_t<4, 0>(p, a, st);
-        case 8:  return launch_fwd_t<8, 0>(p, a, st);
-        case 16: return launch_fwd_t<16, 0>(p, a, st);
+    switch (p.fwd_lpr) {                 // 16 dims per lane, 16 warps per SM (<= 128 registers)
+        case 2:  return launch_fwd_t<2, 0, 4, 4>(p, a, st);
+        case 4:  return launch_fwd_t<4, 0, 4, 4>(p, a, st);
+        case 8:  return launch_fwd_t<8, 0, 4, 4>(p, a, st);
+        case 16: return launch_fwd_t<16, 0, 4, 2, 8>(p, a, st);      // D = 256 / 512: 8 warps per CTA keep 16 / 8 rows per CTA
+        case 32: return launch_fwd_t<32, 0, 4, 2, 8>(p, a, st);
         default: return cudaErrorInvalidValue;
     }
 }

@@ -100,8 +100,6 @@ struct BwdUpstream {
 cudaError_t launch_bwd_prep(const Plan& p, const BwdUpstream& u, const float* S, float* gps, float* gj, float* gk,
                             float* zero, size_t zero_n, cudaStream_t st);
 cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, BwdFinArgs* fin, cudaStream_t st);   // fills fin's segment fields
-void set_bwd_variant(int v);          // tools/tune_bwd.py: tuning points of the fused sweep (tc_bwd_ds.cu)
-void set_bwd_seg_target(int v);       // tools/tune_bwd.py: column tiles per CTA segment (0 = default)
 // column-variance ("full" path) variant, tc_colvar.cu
 cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* lv_all, int64_t ldlv,
                                const Plan& p, float* colpack, float* zpad, float* shift, cudaStream_t st);

@@ -3,7 +3,6 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
-#include <cstdlib>
 
 namespace tcelbo {
 
@@ -110,11 +109,6 @@ inline Segments plan_segments(int64_t n_blocks, int tiles_per_block, int slots, 
     return s;
 }
 
-inline int& fwd_seg_target() { static int v = 0; return v; }    // tuning: forward segment length in column tiles (0 = default)
-// tools/tune_bwd.py --fwd-map (or TCELBO_FWD_MAP): 1 = 32 dims per lane everywhere (round-1 mapping)
-inline int& fwd_map_tuning() { static int v = [] { const char* e = std::getenv("TCELBO_FWD_MAP"); return e ? std::atoi(e) : 0; }(); return v; }
-inline int& fwd_wave_tuning() { static int v = 0; return v; }   // tuning: CTAs per SM the forward grid is sized for (0 = as resident: 4 / 3)
-
 // `sms` = multiprocessor count of the current device (148 on B200).
 inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int sms) {
     if (b_loc < 1 || b_glob < 1 || d < 1 || d > 512) return false;
@@ -145,11 +139,11 @@ inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int
     if (p.jt > 32) p.jt = 32;
     p.small = !p.var_col && (int64_t)p.n_rb_fwd * (p.bg_pad / p.jt) < sms;
     if (p.small) p.jt = kSmallTile;
-    else if (!p.var_col && fwd_map_tuning() == 0) set_map(dp / 16, 4, dp <= 128 ? kFwdWarps : 8);
-    const int fwd_res = fwd_wave_tuning() > 0 ? fwd_wave_tuning() : (p.fwd_kch == 4 ? 16 / p.fwd_warps : 3);   // resident CTAs per SM: wave size
+    else if (!p.var_col) set_map(dp / 16, 4, dp <= 128 ? kFwdWarps : 8);
+    const int fwd_res = p.fwd_kch == 4 ? 16 / p.fwd_warps : 3;   // resident CTAs per SM: wave size
     choose_splits(p.n_rb_fwd, sms * 3, p.bg_pad, p.jt, 4, p.n_js_fwd, p.js_len_fwd);
     p.tiles_fwd = p.bg_pad / p.jt;
-    p.seg_fwd = plan_segments(p.n_rb_fwd, p.tiles_fwd, sms * fwd_res, fwd_seg_target() > 0 ? fwd_seg_target() : 21);
+    p.seg_fwd = plan_segments(p.n_rb_fwd, p.tiles_fwd, sms * fwd_res, 21);    // column tiles per CTA: 16 / 21 / 32 time the same (profiles/r2_notes.md)
     p.slots_fwd = (p.tiles_fwd - 1) / p.seg_fwd.base + 2;
     if (p.slots_fwd > kMaxSplits) p.slots_fwd = kMaxSplits;
     // ---- fused backward sweep: its launcher plans the column split for the CTA shape it runs (<= kMaxSplits)

@@ -24,7 +24,7 @@ def test_library_exports_every_declared_symbol():
     for name in declared:
         assert hasattr(lib, name), f"{name} declared in include/tcelbo.h but not exported by libtcelbo.so"
     assert set(declared) == set(_lib.EXPORTED_SYMBOLS)
-    assert lib.tcelbo_version() == 2
+    assert lib.tcelbo_version() == 3
 
 
 def test_workspace_planner_without_gpu():
@@ -39,26 +39,6 @@ def test_workspace_planner_without_gpu():
     assert shard < 8 * 1024 ** 3
     assert lib.tcelbo_workspace_bytes(64, 64, 513, 0) == 0  # d > 512 is outside the built kernels
     assert lib.tcelbo_workspace_bytes(0, 64, 16, 0) == 0
-
-
-def test_tuning_keys_without_gpu():
-    """tcelbo_set_tuning: the documented keys are accepted, an unknown key is an error; the forward mapping key changes the
-    planner's row padding for D <= 128 (16 rows per CTA with 16 dims per lane, 32 with 32 dims per lane)."""
-    from intro_tc_vae_b200 import _lib
-    lib = _lib.load()
-    flags = _lib.SAVE_FOR_BACKWARD
-    try:
-        for key in (b"bwd_variant", b"bwd_seg_tiles", b"fwd_seg_tiles", b"fwd_map", b"fwd_wave"):
-            assert lib.tcelbo_set_tuning(key, 0) == 0
-        assert lib.tcelbo_set_tuning(b"no_such_key", 1) == _lib.ERR_INVALID
-        assert lib.tcelbo_set_tuning(None, 1) == _lib.ERR_INVALID
-        shipped = [lib.tcelbo_workspace_bytes(1000, 8192, d, flags) for d in (20, 64, 128, 512)]
-        assert lib.tcelbo_set_tuning(b"fwd_map", 1) == 0
-        wide = [lib.tcelbo_workspace_bytes(1000, 8192, d, flags) for d in (20, 64, 128, 512)]
-        assert all(w > 0 for w in shipped + wide)
-        assert shipped[:3] != wide[:3]
-    finally:
-        lib.tcelbo_set_tuning(b"fwd_map", 0)
 
 
 def test_argument_validation_returns_status_not_crash():

@@ -186,9 +186,8 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     fa.b_loc = b_loc; fa.bl_pad = p.bl_pad; fa.bg_pad = p.bg_pad; fa.row_offset = row_offset; fa.js_len = p.js_len_fwd;
     fa.seg = p.seg_fwd; fa.n_rb = p.n_rb_fwd;
     fa.w = w;
-    int n_js_used = p.n_js_fwd;
     if (p.var_col) {
-        if ((e = launch_fwd_colvar(p, fa, &n_js_used, st)) != cudaSuccess) return fail_cuda(e, "tc_fwd_colvar");
+        if ((e = launch_fwd_colvar(p, fa, st)) != cudaSuccess) return fail_cuda(e, "tc_fwd_colvar");
     } else {
         if ((e = launch_fwd(p, fa, st)) != cudaSuccess) return fail_cuda(e, "tc_fwd");
     }
@@ -197,7 +196,7 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     fin.Spart = Spart; fin.Jpart = Jpart; fin.shift = shift;
     fin.S = at<float>(workspace, p.off_S); fin.J2 = at<float>(workspace, p.off_J2);
     fin.log_qz = log_qz; fin.log_qz_prod = log_qz_prod;
-    fin.b_loc = b_loc; fin.bl_pad = p.bl_pad; fin.d = d; fin.dp = p.dp; fin.n_js = n_js_used; fin.lw_u = w.lw_u;
+    fin.b_loc = b_loc; fin.bl_pad = p.bl_pad; fin.d = d; fin.dp = p.dp; fin.n_js = p.n_js_fwd; fin.lw_u = w.lw_u;
     fin.seg = p.seg_fwd; if (p.var_col) fin.seg.n_ctas = 0;
     fin.tiles_per_block = p.tiles_fwd; fin.rows_per_block = p.fwd_rows;
     fin.lv = nullptr; fin.ldlv = 0; fin.mu_loc = nullptr; fin.ldmu = 0; fin.beta = lf.beta; fin.loss_rows = nullptr; fin.kl_rows = nullptr;
@@ -257,44 +256,48 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
     float* CRpart = at<float>(scratch, p.boff_CR);
     float* Gpart = at<float>(scratch, p.boff_G);
 
-    const size_t zero_n = (size_t)(p.var_col ? 2 : 1) * p.bg_pad * p.dp;
-    BwdUpstream up;
-    up.g_log_qz = g_log_qz; up.g_log_qz_prod = g_log_qz_prod; up.g_loss = lf.g_loss; up.g_kl = lf.g_kl;
-    up.g_loss_mean = lf.fz.g_loss_mean; up.g_kl_mean = lf.fz.g_kl_mean; up.g_expelbo = lf.fz.g_expelbo; up.e_rows = lf.fz.e_rows;
-    up.scale = lf.fz.scale; up.g_rec_rows = lf.fz.g_rec_rows; up.beta = lf.beta;
-    up.epoch = (peers.on() && peers.sync.on()) ? peers.sync.state + 1 : nullptr;
-    if ((peers.phase & 1) && (e = launch_bwd_prep(p, up, S, gps, gj, lf.on ? gk : nullptr, Gpart, zero_n, st)) != cudaSuccess)
-        return fail_cuda(e, "bwd_prep");
+    float* Glv = Gpart + (size_t)p.bg_pad * p.dp;                  // column-variance plans: the logvar column sums
 
-    BwdFinArgs fa;
-    fa.Apart = Apart; fa.CRpart = CRpart; fa.Gpart = Gpart; fa.ns = ns; fa.vr = vr;
-    fa.grad_z = grad_z; fa.ldgz = ldgz; fa.grad_lv = grad_logvar; fa.ldglv = ldglv; fa.grad_mu = grad_mu_all; fa.ldgmu = ldgmu;
-    fa.b_loc = b_loc; fa.b_glob = b_glob; fa.bl_pad = p.bl_pad; fa.bg_pad = p.bg_pad; fa.d = d; fa.dp = p.dp;
-    fa.n_js = 1; fa.n_is = 1;
-    fa.seg = Segments{0, 0, 0}; fa.tiles_per_block = 0; fa.n_rb = 0; fa.rows_per_block = 0; fa.slice_dp = 0;
-    fa.gk = lf.on ? gk : nullptr; fa.lv = logvar; fa.ldlv = ldlv; fa.mu_all = mu_all; fa.ldmu = ldmu; fa.row_offset = row_offset;
-    fa.scratch_parts = peers.on() ? peers.scratch_parts : nullptr; fa.g_off = p.boff_G; fa.n_ranks = peers.n_ranks;
-    fa.eps = lf.fz.eps; fa.ldeps = lf.fz.ldeps;
-    fa.sync = peers.sync;
+    // phase 1: prologue and sweep into the scratch
+    if (peers.phase & 1) {
+        const size_t zero_n = (size_t)(p.var_col ? 2 : 1) * p.bg_pad * p.dp;
+        BwdUpstream up;
+        up.g_log_qz = g_log_qz; up.g_log_qz_prod = g_log_qz_prod; up.g_loss = lf.g_loss; up.g_kl = lf.g_kl;
+        up.g_loss_mean = lf.fz.g_loss_mean; up.g_kl_mean = lf.fz.g_kl_mean; up.g_expelbo = lf.fz.g_expelbo; up.e_rows = lf.fz.e_rows;
+        up.scale = lf.fz.scale; up.g_rec_rows = lf.fz.g_rec_rows; up.beta = lf.beta;
+        up.epoch = (peers.on() && peers.sync.on()) ? peers.sync.state + 1 : nullptr;
+        if ((e = launch_bwd_prep(p, up, S, gps, gj, lf.on ? gk : nullptr, Gpart, zero_n, st)) != cudaSuccess) return fail_cuda(e, "bwd_prep");
 
-    BwdFusedArgs ua;
-    ua.zs = zs; ua.ns = ns; ua.qmax = qmax; ua.gps = gps; ua.gj = gj; ua.J2 = J2; ua.mu_pad = mu_pad;
-    ua.s2 = s2; ua.ld_s2 = p.ld_s2; ua.Apart = Apart; ua.CRpart = CRpart; ua.Gacc = Gpart; ua.Gacc2 = nullptr;
-    ua.b_loc = b_loc; ua.bl_pad = p.bl_pad; ua.bg_pad = p.bg_pad; ua.row_offset = row_offset; ua.js_len = 0; ua.w = w;
-    ua.seg = Segments{0, 0, 0}; ua.n_blocks = 0; ua.n_rb = 0;
-    ua.plan_only = (peers.phase & 1) ? 0 : 1;
-
-    if (p.var_col) {
-        float* Glv = Gpart + (size_t)p.bg_pad * p.dp;
-        ua.Gacc2 = Glv;
-        if ((e = launch_bwd_colvar(p, ua, &fa.n_js, st)) != cudaSuccess) return fail_cuda(e, "tc_bwd_colvar");
-        if ((e = launch_bwd_colvar_finalize(p, fa, mu_pad, Glv, st)) != cudaSuccess) return fail_cuda(e, "bwd_colvar_finalize");
-        return TCELBO_OK;
+        BwdFusedArgs ua;
+        ua.zs = zs; ua.ns = ns; ua.qmax = qmax; ua.gps = gps; ua.gj = gj; ua.J2 = J2; ua.mu_pad = mu_pad;
+        ua.s2 = s2; ua.ld_s2 = p.ld_s2; ua.Apart = Apart; ua.CRpart = CRpart; ua.Gacc = Gpart; ua.Gacc2 = p.var_col ? Glv : nullptr;
+        ua.b_loc = b_loc; ua.bl_pad = p.bl_pad; ua.bg_pad = p.bg_pad; ua.row_offset = row_offset; ua.js_len = p.js_len_bwd; ua.w = w;
+        if (p.var_col) {
+            if ((e = launch_bwd_colvar(p, ua, st)) != cudaSuccess) return fail_cuda(e, "tc_bwd_colvar");
+        } else {
+            // single fused sweep: row-local sums in registers, column sums via red.global
+            if ((e = launch_bwd_fused(p, ua, st)) != cudaSuccess) return fail_cuda(e, "tc_bwd_fused");
+        }
     }
-    // single fused sweep: row-local sums in registers, column sums via smem staging + red.global
-    if ((e = launch_bwd_fused(p, ua, &fa, st)) != cudaSuccess) return fail_cuda(e, "tc_bwd_fused");
-    if (!(peers.phase & 2)) return TCELBO_OK;
-    if ((e = launch_bwd_fused_finalize(p, fa, st)) != cudaSuccess) return fail_cuda(e, "bwd_fused_finalize");
+
+    // phase 2: finalize (with peers: once every rank's sweep has filled its scratch)
+    if (peers.phase & 2) {
+        BwdFinArgs fa;
+        fa.Apart = Apart; fa.CRpart = CRpart; fa.Gpart = Gpart; fa.ns = ns; fa.vr = vr;
+        fa.grad_z = grad_z; fa.ldgz = ldgz; fa.grad_lv = grad_logvar; fa.ldglv = ldglv; fa.grad_mu = grad_mu_all; fa.ldgmu = ldgmu;
+        fa.b_loc = b_loc; fa.b_glob = b_glob; fa.bl_pad = p.bl_pad; fa.bg_pad = p.bg_pad; fa.d = d; fa.dp = p.dp;
+        fa.n_js = p.n_js_bwd; fa.n_is = 1;
+        fa.seg = p.seg_bwd; fa.tiles_per_block = p.tiles_bwd; fa.n_rb = p.n_rb_bwd; fa.rows_per_block = p.bwd_rows; fa.slice_dp = p.slice_bwd;
+        fa.gk = lf.on ? gk : nullptr; fa.lv = logvar; fa.ldlv = ldlv; fa.mu_all = mu_all; fa.ldmu = ldmu; fa.row_offset = row_offset;
+        fa.scratch_parts = peers.on() ? peers.scratch_parts : nullptr; fa.g_off = p.boff_G; fa.n_ranks = peers.n_ranks;
+        fa.eps = lf.fz.eps; fa.ldeps = lf.fz.ldeps;
+        fa.sync = peers.sync;
+        if (p.var_col) {
+            if ((e = launch_bwd_colvar_finalize(p, fa, mu_pad, Glv, st)) != cudaSuccess) return fail_cuda(e, "bwd_colvar_finalize");
+        } else {
+            if ((e = launch_bwd_fused_finalize(p, fa, st)) != cudaSuccess) return fail_cuda(e, "bwd_fused_finalize");
+        }
+    }
     return TCELBO_OK;
 }
 

@@ -287,37 +287,23 @@ static bool make_map_2d(CUtensorMap* m, const float* base, uint64_t rows, uint64
                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int RP, int CH, int NW, int MINB, int JT>
-static cudaError_t launch_bwd_ds_t(const Plan& p, const BwdFusedArgs& u, BwdFinArgs* fin, cudaStream_t st) {
-    constexpr int ROWS = (NW / CH) * 2 * RP, DPS = 32 * CH;
+template <int K>
+static cudaError_t launch_bwd_ds_t(const Plan& p, const BwdFusedArgs& u, cudaStream_t st) {
+    constexpr BwdDsConfig c = kBwdDsConfigs[K];
+    constexpr int RP = c.rp, CH = c.ch, NW = c.nw, JT = c.jt, ROWS = (NW / CH) * 2 * RP, DPS = 32 * CH;
+    constexpr auto kern = tc_bwd_ds_kernel<RP, CH, NW, c.minb, JT>;
     const size_t smem = ((size_t)kStages * JT * DPS + (size_t)kStages * ROWS * JT + (size_t)NW * JT * 2 * RP + (size_t)NW * 2 * RP * 2) * sizeof(float)
                         + 2 * kStages * sizeof(uint64_t);
-    auto kern = tc_bwd_ds_kernel<RP, CH, NW, MINB, JT>;
-    static PerDevice ctas_on;
-    int& ctas_per_sm = ctas_on.cur();
-    if (ctas_per_sm == 0) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int occ = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NW * 32, smem);
-        if (e != cudaSuccess) return e;
-        ctas_per_sm = occ > 0 ? occ : 1;
-    }
-    const int n_rb = (p.bl_pad + ROWS - 1) / ROWS;
-    const int n_slices = p.dp / DPS;
-    const int T = p.bg_pad / JT;
-    const Segments seg = plan_segments((int64_t)n_rb * n_slices, T, p.sms * ctas_per_sm, 2048 / JT);     // 128 tiles of 16 columns per CTA (profiles/r2_notes.md)
-    fin->seg = seg; fin->tiles_per_block = T; fin->n_rb = n_rb; fin->rows_per_block = ROWS; fin->slice_dp = DPS;
-    if (u.plan_only) return cudaSuccess;
+    if (cudaError_t e = allow_dynamic_smem<kern>(smem)) return e;
     BwdDsArgs a;
     if (!make_map_2d(&a.map_mu, u.mu_pad, (uint64_t)p.bg_pad, (uint64_t)p.dp, (uint64_t)p.dp, JT, DPS)) return cudaErrorNotSupported;
     if (!make_map_2d(&a.map_s2, u.s2, (uint64_t)p.bl_pad, (uint64_t)p.bg_pad, (uint64_t)u.ld_s2, ROWS, JT)) return cudaErrorNotSupported;
     a.zs = u.zs; a.ns = u.ns; a.qmax = u.qmax; a.gps = u.gps; a.gj = u.gj; a.J2 = u.J2;
     a.Apart = u.Apart; a.CRpart = u.CRpart; a.Gacc = u.Gacc;
     a.b_loc = u.b_loc; a.bl_pad = u.bl_pad; a.bg_pad = u.bg_pad; a.row_offset = u.row_offset; a.pitch = p.dp;
-    a.seg = seg; a.n_rb = n_rb; a.w = u.w;
+    a.seg = p.seg_bwd; a.n_rb = p.n_rb_bwd; a.w = u.w;
     LaunchScope scope(kKernBwdRow, st);
-    return launch_pdl(kern, dim3(seg.n_ctas), dim3(NW * 32), smem, st, a);
+    return launch_pdl(kern, dim3(p.seg_bwd.n_ctas), dim3(NW * 32), smem, st, a);
 }
 
 // Elementwise over [B,D]: sum the column-split partials of the row-local sums (8 independent loads in flight), scale,
@@ -489,17 +475,16 @@ __global__ void bwd_fused_finalize_v4_kernel(const BwdFinArgs a) {
     }
 }
 
-// Shipped configurations; the measured alternatives they beat are in profiles/r2_bwd_ds_sweep.md
-cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, BwdFinArgs* fin, cudaStream_t st) {
-    if (p.small) {                       // B = 3 / 64-sized batches: 4 rows per warp so that row blocks x tiles covers more SMs
-        if (p.dp >= 128) return launch_bwd_ds_t<2, 4, 8, 2, 16>(p, a, fin, st);
-        if (p.dp == 64) return launch_bwd_ds_t<2, 2, 8, 2, 16>(p, a, fin, st);
-        return launch_bwd_ds_t<2, 1, 8, 2, 16>(p, a, fin, st);
+cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, cudaStream_t st) {
+    switch (p.bwd_cfg) {
+        case 0: return launch_bwd_ds_t<0>(p, a, st);
+        case 1: return launch_bwd_ds_t<1>(p, a, st);
+        case 2: return launch_bwd_ds_t<2>(p, a, st);
+        case 3: return launch_bwd_ds_t<3>(p, a, st);
+        case 4: return launch_bwd_ds_t<4>(p, a, st);
+        case 5: return launch_bwd_ds_t<5>(p, a, st);
+        default: return cudaErrorInvalidValue;
     }
-    // 16 rows per warp, 12 warps per SM (168 registers), 8 columns per basic block, clamp mask by select
-    if (p.dp >= 128) return launch_bwd_ds_t<8, 4, 12, 1, 16>(p, a, fin, st);
-    if (p.dp == 64) return launch_bwd_ds_t<8, 2, 12, 1, 16>(p, a, fin, st);
-    return launch_bwd_ds_t<8, 1, 12, 1, 16>(p, a, fin, st);
 }
 
 cudaError_t launch_bwd_fused_finalize(const Plan& p, const BwdFinArgs& a, cudaStream_t st) {

@@ -17,9 +17,6 @@
 
 namespace tcelbo {
 
-__device__ __forceinline__ float fset_ge_cv(float a, float b) {
-    float y; asm("set.ge.f32.f32 %0, %1, %2;" : "=f"(y) : "f"(a), "f"(b)); return y;
-}
 __device__ __forceinline__ void red_add_v4_cv(float* addr, float a, float b, float c, float d) {
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" :: "l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
@@ -98,7 +95,7 @@ __device__ __forceinline__ float cv_fwd_one_column(const float* __restrict__ col
 }
 
 template <int LPR>
-__global__ void __launch_bounds__(kFwdWarps * 32, 2)
+__global__ void __launch_bounds__(kFwdWarps * 32, kColvarFwdRes)
 tc_fwd_colvar_kernel(const FwdArgs a) {
     using GEO = CvGeom<LPR>;
     constexpr int DP = GEO::DP, JT = GEO::JT, TILE = GEO::TILE;
@@ -219,7 +216,7 @@ template <int DPT> struct CvBwdGeom {
 };
 
 template <int DPT, int RI>
-__global__ void __launch_bounds__(kBwdWarps * 32, 1)
+__global__ void __launch_bounds__(kBwdWarps * 32, colvar_bwd_res(DPT))
 tc_bwd_colvar_kernel(const BwdFusedArgs a) {
     using GEO = CvBwdGeom<DPT>;
     constexpr int VEC = GEO::VEC, NCH = GEO::NCH, DP = GEO::DP, CH = GEO::CH, JT = GEO::JT, JS = GEO::JS;
@@ -414,74 +411,46 @@ cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all,
 }
 
 template <int LPR>
-static cudaError_t launch_fwd_colvar_t(const Plan& p, FwdArgs a, int* n_js_out, cudaStream_t st) {
-    using GEO = CvGeom<LPR>;
-    const size_t smem = (size_t)kStages * GEO::TILE * sizeof(float) + 2 * kStages * sizeof(uint64_t);
-    static PerDevice ctas_on;
-    int& ctas_per_sm = ctas_on.cur();
-    if (ctas_per_sm == 0) {
-        cudaError_t e = cudaFuncSetAttribute(tc_fwd_colvar_kernel<LPR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int occ = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, tc_fwd_colvar_kernel<LPR>, kFwdWarps * 32, smem);
-        if (e != cudaSuccess) return e;
-        ctas_per_sm = occ > 0 ? occ : 1;
-    }
-    int n_js, js_len;
-    choose_splits(p.n_rb_fwd, p.sms * ctas_per_sm, p.bg_pad, p.jt, 4, n_js, js_len);
-    if (n_js > p.n_js_fwd) { n_js = p.n_js_fwd; js_len = p.js_len_fwd; }       // scratch is sized for the row-variant plan
-    a.js_len = js_len;
-    *n_js_out = n_js;
+static cudaError_t launch_fwd_colvar_t(const Plan& p, const FwdArgs& a, cudaStream_t st) {
+    constexpr auto kern = tc_fwd_colvar_kernel<LPR>;
+    const size_t smem = (size_t)kStages * CvGeom<LPR>::TILE * sizeof(float) + 2 * kStages * sizeof(uint64_t);
+    if (cudaError_t e = allow_dynamic_smem<kern>(smem)) return e;
     LaunchScope scope(kKernFwd, st);
-    tc_fwd_colvar_kernel<LPR><<<dim3(p.n_rb_fwd, n_js), kFwdWarps * 32, smem, st>>>(a);
+    kern<<<dim3(p.n_rb_fwd, p.n_js_fwd), kFwdWarps * 32, smem, st>>>(a);
     return cudaGetLastError();
 }
 
-cudaError_t launch_fwd_colvar(const Plan& p, const FwdArgs& a, int* n_js_out, cudaStream_t st) {
+cudaError_t launch_fwd_colvar(const Plan& p, const FwdArgs& a, cudaStream_t st) {
     switch (p.dpt) {
-        case 1:  return launch_fwd_colvar_t<1>(p, a, n_js_out, st);
-        case 2:  return launch_fwd_colvar_t<2>(p, a, n_js_out, st);
-        case 4:  return launch_fwd_colvar_t<4>(p, a, n_js_out, st);
-        case 8:  return launch_fwd_colvar_t<8>(p, a, n_js_out, st);
-        case 16: return launch_fwd_colvar_t<16>(p, a, n_js_out, st);
+        case 1:  return launch_fwd_colvar_t<1>(p, a, st);
+        case 2:  return launch_fwd_colvar_t<2>(p, a, st);
+        case 4:  return launch_fwd_colvar_t<4>(p, a, st);
+        case 8:  return launch_fwd_colvar_t<8>(p, a, st);
+        case 16: return launch_fwd_colvar_t<16>(p, a, st);
         default: return cudaErrorInvalidValue;
     }
 }
 
-template <int DPT, int RI>
-static cudaError_t launch_bwd_colvar_t(const Plan& p, BwdFusedArgs a, int* n_js_out, cudaStream_t st) {
+template <int DPT>
+static cudaError_t launch_bwd_colvar_t(const Plan& p, const BwdFusedArgs& a, cudaStream_t st) {
     using GEO = CvBwdGeom<DPT>;
-    constexpr int ROWS = kBwdWarps * RI;
+    constexpr int RI = colvar_bwd_rows_per_warp(DPT), ROWS = kBwdWarps * RI;
+    constexpr auto kern = tc_bwd_colvar_kernel<DPT, RI>;
     const size_t smem = ((size_t)kStages * GEO::JT * 3 * GEO::DP + (size_t)kStages * ROWS * GEO::JT + (size_t)kBwdWarps * RI * GEO::JT
                          + (size_t)kBwdWarps * GEO::JS * 2 * GEO::DP) * sizeof(float) + 2 * kStages * sizeof(uint64_t);
-    static PerDevice ctas_on;
-    int& ctas_per_sm = ctas_on.cur();
-    if (ctas_per_sm == 0) {
-        auto kern = tc_bwd_colvar_kernel<DPT, RI>;
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        int occ = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kBwdWarps * 32, smem);
-        if (e != cudaSuccess) return e;
-        ctas_per_sm = occ > 0 ? occ : 1;
-    }
-    const int n_rb = (p.bl_pad + ROWS - 1) / ROWS;
-    int n_js, js_len;
-    choose_splits(n_rb, p.sms * ctas_per_sm, p.bg_pad, p.jt, 4, n_js, js_len);
-    a.js_len = js_len;
-    *n_js_out = n_js;
+    if (cudaError_t e = allow_dynamic_smem<kern>(smem)) return e;
     LaunchScope scope(kKernBwdRow, st);
-    tc_bwd_colvar_kernel<DPT, RI><<<dim3(n_rb, n_js), kBwdWarps * 32, smem, st>>>(a);
+    kern<<<dim3(p.n_rb_bwd, p.n_js_bwd), kBwdWarps * 32, smem, st>>>(a);
     return cudaGetLastError();
 }
 
-cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, int* n_js_out, cudaStream_t st) {
+cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, cudaStream_t st) {
     switch (p.dpt) {
-        case 1:  return launch_bwd_colvar_t<1, 4>(p, a, n_js_out, st);
-        case 2:  return launch_bwd_colvar_t<2, 4>(p, a, n_js_out, st);
-        case 4:  return launch_bwd_colvar_t<4, 4>(p, a, n_js_out, st);
-        case 8:  return launch_bwd_colvar_t<8, 2>(p, a, n_js_out, st);
-        case 16: return launch_bwd_colvar_t<16, 1>(p, a, n_js_out, st);
+        case 1:  return launch_bwd_colvar_t<1>(p, a, st);
+        case 2:  return launch_bwd_colvar_t<2>(p, a, st);
+        case 4:  return launch_bwd_colvar_t<4>(p, a, st);
+        case 8:  return launch_bwd_colvar_t<8>(p, a, st);
+        case 16: return launch_bwd_colvar_t<16>(p, a, st);
         default: return cudaErrorInvalidValue;
     }
 }

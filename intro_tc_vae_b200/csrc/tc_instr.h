@@ -25,11 +25,23 @@ struct LaunchScope {                        // RAII: count the launch, record ev
     ~LaunchScope() { if (timed) cudaEventRecord(instr().ev_stop, st); }
 };
 
-// One cached int per CUDA device (cudaFuncSetAttribute and occupancy are per device: a process that drives several GPUs
-// must configure every kernel on each of them).  Races are benign: every thread computes the same value.
+// One cached int per CUDA device (cudaFuncSetAttribute is per device: a process that drives several GPUs must configure
+// every kernel on each of them).  Races are benign: every thread computes the same value.
 struct PerDevice {
     int v[64] = {};
     int& cur() { int d = 0; if (cudaGetDevice(&d) != cudaSuccess) d = 0; return v[d & 63]; }
 };
+
+// Let `kern` use `smem` bytes of dynamic shared memory (every launch of a kernel asks for the same amount), once per device.
+// One instantiation, and so one cache, per kernel.
+template <auto kern>
+inline cudaError_t allow_dynamic_smem(size_t smem) {
+    static PerDevice done_on;
+    int& done = done_on.cur();
+    if (done) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) done = 1;
+    return e;
+}
 
 }  // namespace tcelbo

@@ -521,16 +521,11 @@ template <int LPR, int JTS, int KCH = 8, int MINB = 3, int NWF = kFwdWarps>
 static cudaError_t launch_fwd_t(const Plan& p, const FwdArgs& a, cudaStream_t st) {
     constexpr int DP = 4 * KCH * LPR;
     constexpr int JT = JTS > 0 ? JTS : ((kTileFloats / DP) > 32 ? 32 : (kTileFloats / DP));
+    constexpr auto kern = tc_fwd_kernel<LPR, JTS, KCH, MINB, NWF>;
     const size_t smem = (size_t)kStages * JT * DP * sizeof(float) + 2 * kStages * sizeof(uint64_t);
-    static PerDevice configured_on;
-    int& configured = configured_on.cur();
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(tc_fwd_kernel<LPR, JTS, KCH, MINB, NWF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        configured = 1;
-    }
+    if (cudaError_t e = allow_dynamic_smem<kern>(smem)) return e;
     LaunchScope scope(kKernFwd, st);
-    return launch_pdl(tc_fwd_kernel<LPR, JTS, KCH, MINB, NWF>, dim3(p.seg_fwd.n_ctas), dim3(NWF * 32), smem, st, a);
+    return launch_pdl(kern, dim3(p.seg_fwd.n_ctas), dim3(NWF * 32), smem, st, a);
 }
 
 cudaError_t launch_publish(const float* src, int64_t ld, int b_loc, int d, float* dst, unsigned int* epoch, cudaStream_t st) {

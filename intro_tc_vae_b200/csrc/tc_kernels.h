@@ -14,8 +14,9 @@ struct FwdArgs {
     float* Spart;                                          // [n_js][bl_pad][dp]
     float* Jpart;                                          // [n_js][bl_pad] (m, s) pairs
     int b_loc, bl_pad, bg_pad, row_offset, js_len;
-    Segments seg; int n_rb;                                // balanced segments (row-variance sweep; tc_layout.h: plan_segments)
-    Weights w;
+    Segments seg;                                          // balanced segments (row-variance sweep; tc_layout.h: plan_segments)
+    int n_rb;                                              // read by no kernel, but dropping it moves `w` and with it changes the
+    Weights w;                                             // register allocation (and spills) of the forward sweep kernels
 };
 
 struct FinArgs {
@@ -57,9 +58,6 @@ struct BwdFusedArgs {
     float* Gacc;                                                             // [bg_pad][dp], zeroed by the caller
     float* Gacc2;                                                            // column-variance variant: logvar column sums
     int b_loc, bl_pad, bg_pad, row_offset, js_len;
-    int pitch;                                                               // floats per row of the [*, dp] arrays
-    Segments seg; int n_blocks, n_rb;                                        // balanced segments (fused sweep; tc_layout.h: plan_segments)
-    int plan_only;                                                           // host-side: compute the column split, launch nothing
     Weights w;
 };
 
@@ -99,12 +97,12 @@ struct BwdUpstream {
 };
 cudaError_t launch_bwd_prep(const Plan& p, const BwdUpstream& u, const float* S, float* gps, float* gj, float* gk,
                             float* zero, size_t zero_n, cudaStream_t st);
-cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, BwdFinArgs* fin, cudaStream_t st);   // fills fin's segment fields
+cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, cudaStream_t st);
 // column-variance ("full" path) variant, tc_colvar.cu
 cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* lv_all, int64_t ldlv,
                                const Plan& p, float* colpack, float* zpad, float* shift, cudaStream_t st);
-cudaError_t launch_fwd_colvar(const Plan& p, const FwdArgs& a, int* n_js_out, cudaStream_t st);
-cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, int* n_js_out, cudaStream_t st);
+cudaError_t launch_fwd_colvar(const Plan& p, const FwdArgs& a, cudaStream_t st);
+cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, cudaStream_t st);
 cudaError_t launch_bwd_colvar_finalize(const Plan& p, const BwdFinArgs& a, const float* colpack, const float* Glv, cudaStream_t st);
 cudaError_t launch_bwd_fused_finalize(const Plan& p, const BwdFinArgs& a, cudaStream_t st);
 

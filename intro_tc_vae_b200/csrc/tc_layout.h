@@ -46,9 +46,21 @@ TCELBO_HD inline int seg_slots(const Segments& s, int64_t q, int tiles_per_block
     return seg_of(s, (q + 1) * tiles_per_block - 1) - seg_of(s, q * tiles_per_block) + 1;
 }
 
+// Shipped configurations of the backward row-variance sweep, tc_bwd_ds_kernel<RP, CH, NW, MINB, JT> (tc_bwd_ds.cu): RP row
+// pairs per warp, CH warps per 32*CH-dim slice, NW warps per CTA, MINB resident CTAs per SM (the launch bounds, and the wave
+// size the segment plan assumes), JT columns per tile.  The measured alternatives they beat are in profiles/r2_bwd_ds_sweep.md.
+struct BwdDsConfig { int rp, ch, nw, minb, jt; };
+constexpr BwdDsConfig kBwdDsConfigs[6] = {
+    {8, 4, 12, 1, 16}, {8, 2, 12, 1, 16}, {8, 1, 12, 1, 16},   // 16 rows per warp, 12 warps per SM (168 registers); dp >= 128 / 64 / 32
+    {2, 4, 8, 2, 16},  {2, 2, 8, 2, 16},  {2, 1, 8, 2, 16},    // small problems: 4 rows per warp, so that row blocks x tiles covers more SMs
+};
+// Column-variance sweeps (tc_colvar.cu), DPT = dp / 32: resident CTAs per SM (the kernels' launch bounds) and, backward, rows per warp
+constexpr int kColvarFwdRes = 3;
+constexpr int colvar_bwd_rows_per_warp(int dpt) { return dpt <= 4 ? 4 : 16 / dpt; }
+constexpr int colvar_bwd_res(int dpt) { return dpt <= 2 ? 2 : 1; }
+
 struct Plan {
     // padded problem
-    int sms;
     int d, dp, dpt;            // dp = power of two >= max(d, 32); dpt = dp / 32 (floats per lane / lanes per row)
     int b_loc, b_glob, bl_pad, bg_pad;
     int jt;                    // column-tile height (rows of mu per stage) = kTileFloats / dp
@@ -56,6 +68,11 @@ struct Plan {
     int fwd_rows, n_rb_fwd, n_js_fwd, js_len_fwd;            // uniform split (column-variance sweep)
     Segments seg_fwd; int tiles_fwd, slots_fwd;               // balanced segments (row-variance sweep)
     int n_part_fwd;                                           // partial-sum slots the scratch holds
+    // backward sweep: n_rb_bwd row blocks of bwd_rows rows
+    int bwd_rows, n_rb_bwd;
+    int n_js_bwd, js_len_bwd;                                 // uniform split: grid (n_rb_bwd, n_js_bwd) (column-variance sweep)
+    int bwd_cfg, slice_bwd, n_slices_bwd;                     // kBwdDsConfigs entry, dims per slice (row-variance sweep) ...
+    Segments seg_bwd; int tiles_bwd;                          // ... balanced segments over blocks q = slice * n_rb_bwd + row block
     // workspace (byte offsets)
     size_t off_mu, off_zs, off_ns, off_qmax, off_shift, off_vr;   // [bg_pad|bl_pad][dp]
     size_t off_S, off_J2;                                         // persistent forward results
@@ -112,6 +129,7 @@ inline Segments plan_segments(int64_t n_blocks, int tiles_per_block, int slots, 
 // `sms` = multiprocessor count of the current device (148 on B200).
 inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int sms) {
     if (b_loc < 1 || b_glob < 1 || d < 1 || d > 512) return false;
+    p = Plan();
     p.d = d;
     int dp = 32; while (dp < d) dp <<= 1;
     p.dp = dp; p.dpt = dp / 32;
@@ -141,13 +159,27 @@ inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int
     if (p.small) p.jt = kSmallTile;
     else if (!p.var_col) set_map(dp / 16, 4, dp <= 128 ? kFwdWarps : 8);
     const int fwd_res = p.fwd_kch == 4 ? 16 / p.fwd_warps : 3;   // resident CTAs per SM: wave size
-    choose_splits(p.n_rb_fwd, sms * 3, p.bg_pad, p.jt, 4, p.n_js_fwd, p.js_len_fwd);
+    // the column-variance grid; row-variance plans size their forward partials with it too
+    choose_splits(p.n_rb_fwd, sms * kColvarFwdRes, p.bg_pad, p.jt, 4, p.n_js_fwd, p.js_len_fwd);
     p.tiles_fwd = p.bg_pad / p.jt;
     p.seg_fwd = plan_segments(p.n_rb_fwd, p.tiles_fwd, sms * fwd_res, 21);    // column tiles per CTA: 16 / 21 / 32 time the same (profiles/r2_notes.md)
     p.slots_fwd = (p.tiles_fwd - 1) / p.seg_fwd.base + 2;
     if (p.slots_fwd > kMaxSplits) p.slots_fwd = kMaxSplits;
-    // ---- fused backward sweep: its launcher plans the column split for the CTA shape it runs (<= kMaxSplits)
-    p.sms = sms;
+    // ---- backward sweep: the partial-sum slots it writes per row block fit the kMaxSplits of the backward scratch
+    if (p.var_col) {
+        p.bwd_rows = kBwdWarps * colvar_bwd_rows_per_warp(p.dpt);
+        p.n_rb_bwd = (p.bl_pad + p.bwd_rows - 1) / p.bwd_rows;
+        choose_splits(p.n_rb_bwd, sms * colvar_bwd_res(p.dpt), p.bg_pad, p.jt, 4, p.n_js_bwd, p.js_len_bwd);
+    } else {
+        p.bwd_cfg = (p.small ? 3 : 0) + (dp >= 128 ? 0 : dp == 64 ? 1 : 2);
+        const BwdDsConfig& c = kBwdDsConfigs[p.bwd_cfg];
+        p.bwd_rows = c.nw / c.ch * 2 * c.rp;
+        p.n_rb_bwd = (p.bl_pad + p.bwd_rows - 1) / p.bwd_rows;
+        p.slice_bwd = 32 * c.ch;
+        p.n_slices_bwd = dp / p.slice_bwd;
+        p.tiles_bwd = p.bg_pad / c.jt;
+        p.seg_bwd = plan_segments((int64_t)p.n_rb_bwd * p.n_slices_bwd, p.tiles_bwd, sms * c.minb, 2048 / c.jt);   // 128 tiles of 16 columns per CTA (profiles/r2_notes.md)
+    }
 
     // ---- workspace
     size_t off = 0;

@@ -1,5 +1,6 @@
 """Host-side work planner (csrc/tc_layout.h): balanced segments must tile the (row block x column tile) space exactly,
-differ by at most one tile, stay within the partial-slot budget, and number the slots of every block 0..n-1."""
+differ by at most one tile, stay within the partial-slot budget, and number the slots of every block 0..n-1.  Whole plans:
+the forward and backward grids of both sweeps write no more partial-sum slots than the workspace and the scratch hold."""
 import os
 import subprocess
 import textwrap
@@ -13,8 +14,7 @@ SRC = textwrap.dedent(r"""
     #include <cstdio>
     #include <vector>
     using namespace tcelbo;
-    static int check(int64_t n_blocks, int T, int slots, int target) {
-        const Segments s = plan_segments(n_blocks, T, slots, target);
+    static int check_tiling(const Segments& s, int64_t n_blocks, int T) {
         const int64_t total = n_blocks * T;
         if (s.n_ctas < 1 || s.base < 1) return 1;
         if (seg_begin(s, s.n_ctas - 1) + seg_len(s, s.n_ctas - 1) != total) return 2;      // covers everything, no overlap
@@ -28,6 +28,11 @@ SRC = textwrap.dedent(r"""
             const int n = seg_slots(s, q, T);
             if (n < 1 || n > kMaxSplits) return 6;
         }
+        return 0;
+    }
+    static int check(int64_t n_blocks, int T, int slots, int target) {
+        const Segments s = plan_segments(n_blocks, T, slots, target);
+        if (const int rc = check_tiling(s, n_blocks, T)) return rc;
         if (s.n_ctas > slots && s.n_ctas % slots != 0) return 7;                           // whole waves once past one wave
         return 0;
     }
@@ -42,14 +47,29 @@ SRC = textwrap.dedent(r"""
         }
         // whole plans for shapes the tests and the bench use
         const int shapes[][3] = {{8192, 8192, 128}, {1024, 8192, 128}, {2, 2, 4}, {37, 37, 20}, {24, 24, 512}, {4096, 32768, 512}, {1, 8, 3},
-                                   {4096, 4096, 64}, {4000, 4000, 20}, {1000, 1000, 128}, {512, 4096, 256}, {64, 64, 128}, {3, 3, 128}};
+                                   {4096, 4096, 64}, {4000, 4000, 20}, {1000, 1000, 128}, {512, 4096, 256}, {64, 64, 128}, {3, 3, 128},
+                                   {64, 64, 64}};
+        int cfgs_seen = 0;
         for (auto& sh : shapes) {
+            // row variance: balanced segments; the backward ones index Apart / CRpart, which hold kMaxSplits slots per row
             Plan p;
             if (!make_plan(p, sh[0], sh[1], sh[2], 4u, 148)) { std::printf("FAIL make_plan\n"); return 1; }
             if (p.slots_fwd > p.n_part_fwd || p.slots_fwd > kMaxSplits) { std::printf("FAIL slots\n"); return 1; }
             for (int q = 0; q < p.n_rb_fwd; ++q)
                 if (seg_slots(p.seg_fwd, q, p.tiles_fwd) > p.slots_fwd) { std::printf("FAIL fwd slots %d %d\n", sh[0], sh[1]); return 1; }
+            if (p.n_rb_bwd * p.bwd_rows < p.bl_pad || p.n_slices_bwd * p.slice_bwd != p.dp) { std::printf("FAIL bwd blocks %d %d\n", sh[0], sh[1]); return 1; }
+            if (const int rc = check_tiling(p.seg_bwd, (int64_t)p.n_rb_bwd * p.n_slices_bwd, p.tiles_bwd)) {
+                std::printf("FAIL bwd segments rc=%d %d %d %d\n", rc, sh[0], sh[1], sh[2]); return 1;
+            }
+            cfgs_seen |= 1 << p.bwd_cfg;
+            // column variance: uniform splits, one partial-sum slot per split
+            if (!make_plan(p, sh[0], sh[1], sh[2], 6u, 148)) { std::printf("FAIL make_plan\n"); return 1; }
+            if (p.n_js_fwd > p.n_part_fwd || p.n_js_bwd > kMaxSplits) { std::printf("FAIL colvar splits %d %d %d\n", sh[0], sh[1], sh[2]); return 1; }
+            if ((int64_t)p.n_js_fwd * p.js_len_fwd < p.bg_pad || (int64_t)p.n_js_bwd * p.js_len_bwd < p.bg_pad || p.n_rb_bwd * p.bwd_rows < p.bl_pad) {
+                std::printf("FAIL colvar coverage %d %d %d\n", sh[0], sh[1], sh[2]); return 1;
+            }
         }
+        if (cfgs_seen != (1 << 6) - 1) { std::printf("FAIL backward configurations covered: %x\n", cfgs_seen); return 1; }
         std::printf("OK\n");
         return 0;
     }

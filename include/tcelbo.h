@@ -160,6 +160,32 @@ int tcelbo_klloss_backward_ex(const float* z, int64_t ldz, const float* mu_all, 
                               const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream);
 
 /*
+ * Fused MI / TC / dimension-wise KL decomposition of TCSovler._compute_kl_loss_full (solvers/tc.py:91-144), the beta-TCVAE
+ * loss, on the column-variance density: flags must contain TCELBO_VAR_COL.  Per local row i, global row r = row_offset + i,
+ * lp = the clamped un-floored density of tcelbo_rowdensity_forward:
+ *   condx_i = sum_d lp(z_id; mu_rd, logvar_rd)       pz_i = sum_d lp(z_id; 0, 0)
+ *   mi_rows[i] = condx_i - log_qz[i]   tc_rows[i] = log_qz[i] - log_qz_prod[i]   dimkl_rows[i] = log_qz_prod[i] - pz_i
+ *   loss_rows[i] = mi_rows[i] + beta * tc_rows[i] + dimkl_rows[i]
+ * Same arguments as tcelbo_klloss_forward_ex / _backward_ex with logvar [b_glob, D] (all rows, like mu_all); workspace and
+ * scratch sizes come from tcelbo_workspace_bytes / tcelbo_backward_scratch_bytes with the same flags.  `means` (optional, DEVICE
+ * float[4]) receives the means of loss, mi, tc, dimkl over this rank's b_loc rows, summed in a fixed order inside the finalize
+ * kernel.  The backward takes dLoss/d of the four per-row outputs and g_means (DEVICE float[4], dLoss/d of the four means); each
+ * may be NULL (= zero) as long as one is given.  It adds the gradients of condx and pz to grad_z, to grad_logvar [b_glob, D] and to
+ * rows [row_offset, row_offset + b_loc) of grad_mu_all, so no row-density or elementwise kernels are launched: 3 kernels forward,
+ * 3 backward.  The peer-memory exchange and the fused reparameterize cover the row-variance density only.
+ */
+int tcelbo_decomp_forward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                          int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                          float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                          void* workspace, size_t workspace_bytes, void* stream);
+int tcelbo_decomp_backward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                           int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                           const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                           const float* g_means,
+                           float* grad_z, int64_t ldgz, float* grad_mu_all, int64_t ldgmu, float* grad_logvar, int64_t ldglv,
+                           const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream);
+
+/*
  * Peer-memory exchange for the row-sharded fused loss (one process per GPU; SURVEY.md 8e).  Replaces the NCCL all-gather of
  * the column operand and the reduce-scatter of its gradient (what a torch DistributedDataParallel port of solvers/tc.py:69-89
  * would issue around ops.py:52-89) by loads over NVLink inside the library's own prep / finalize kernels:

@@ -58,6 +58,11 @@ _SIGNATURES = {
     "tcelbo_klloss_backward_ex": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32, c_float,
                                           _f, _f, _f, _f, POINTER(Fusion), _f, c_int64, _f, c_int64, _f, c_int64, c_void_p, c_size_t,
                                           c_void_p, c_size_t, c_void_p]),
+    "tcelbo_decomp_forward": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32, c_float,
+                                      _f, _f, _f, _f, _f, c_void_p, c_size_t, c_void_p]),
+    "tcelbo_decomp_backward": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32, c_float,
+                                       _f, _f, _f, _f, _f, _f, c_int64, _f, c_int64, _f, c_int64, c_void_p, c_size_t, c_void_p,
+                                       c_size_t, c_void_p]),
     "tcelbo_peer_publish": (c_int, [_f, c_int64, c_int, c_int, _f, POINTER(PeerSyncArgs), c_void_p]),
     "tcelbo_klloss_forward_peer": (c_int, [_f, c_int64, _f, c_int64, c_void_p, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64,
                                            c_uint32, c_float, _f, _f, _f, _f, POINTER(Fusion), POINTER(PeerSyncArgs), c_void_p, c_size_t, c_void_p]),

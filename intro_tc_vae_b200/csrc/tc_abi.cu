@@ -120,6 +120,11 @@ struct LossFusion {            // solvers/tc.py:83-89 folded into the finalize k
     const float* g_loss = nullptr; const float* g_kl = nullptr;           // backward inputs
     bool on = false;
     tcelbo_fusion fz = {};                                                // optional prologue / epilogue fusions (tcelbo.h)
+    // MI + beta*TC + dimension-wise KL of solvers/tc.py:91-144, column-variance density (tcelbo_decomp_*; exclusive with `on`)
+    bool decomp = false;
+    float* mi_rows = nullptr; float* tc_rows = nullptr; float* dimkl_rows = nullptr; float* means = nullptr;   // forward outputs
+    const float* g_mi = nullptr; const float* g_tc = nullptr; const float* g_dimkl = nullptr;                    // backward inputs
+    const float* g_means = nullptr;
 };
 
 // Peer-memory exchange (tcelbo_*_peer): the column operand / the column accumulators live in n_ranks allocations that
@@ -138,7 +143,7 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
                         float* log_qz, float* log_qz_prod, const LossFusion& lf,
                         void* workspace, size_t workspace_bytes, void* stream, const Peers& peers = Peers()) {
     if (int rc = check_common(z, mu_all, logvar, b_loc, b_glob, row_offset, d, dataset_size, flags, ldz, ldmu, ldlv, lf.fz.eps != nullptr)) return rc;
-    if (!log_qz || !log_qz_prod) return fail(TCELBO_ERR_INVALID, "null output pointer");
+    if (!lf.decomp && (!log_qz || !log_qz_prod)) return fail(TCELBO_ERR_INVALID, "null output pointer");
     if (lf.fz.eps && (lf.fz.ldeps < d || (lf.fz.z_out && lf.fz.ldz_out < d))) return fail(TCELBO_ERR_INVALID, "eps / z_out row pitch smaller than d");
     if (lf.fz.eps && (flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_UNSUPPORTED, "the fused reparameterize covers the row-variance density");
     if (lf.fz.expelbo && (!lf.fz.rec_rows || !lf.fz.e_rows)) return fail(TCELBO_ERR_INVALID, "expelbo needs rec_rows and e_rows");
@@ -162,9 +167,9 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     float* Jpart = Spart + (size_t)p.n_part_fwd * p.bl_pad * p.dp;
 
     const tcelbo_fusion& fz = lf.fz;
-    unsigned int* ticket = at<unsigned int>(workspace, p.off_red) + 3 * (size_t)p.n_fin_ctas;
+    unsigned int* ticket = at<unsigned int>(workspace, p.off_red) + 4 * (size_t)p.n_fin_ctas;
     if (p.var_col) {
-        if ((e = launch_colvar_prep(z, ldz, mu_all, ldmu, logvar, ldlv, p, mu_pad, zs, shift, st)) != cudaSuccess) return fail_cuda(e, "colvar_prep");
+        if ((e = launch_colvar_prep(z, ldz, mu_all, ldmu, logvar, ldlv, p, mu_pad, zs, shift, ticket, st)) != cudaSuccess) return fail_cuda(e, "colvar_prep");
     } else {
         PrepArgs pa;
         pa.mu_all = mu_all; pa.ldmu = ldmu;
@@ -202,6 +207,13 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     fin.lv = nullptr; fin.ldlv = 0; fin.mu_loc = nullptr; fin.ldmu = 0; fin.beta = lf.beta; fin.loss_rows = nullptr; fin.kl_rows = nullptr;
     fin.loss_mean = nullptr; fin.kl_mean = nullptr; fin.rec_rows = nullptr; fin.scale = 0.0f; fin.expelbo = nullptr; fin.e_rows = nullptr;
     fin.red_part = nullptr; fin.ticket = nullptr;
+    fin.dz = nullptr; fin.lddz = 0; fin.dmu = nullptr; fin.lddmu = 0; fin.dlv = nullptr; fin.lddlv = 0; fin.row_offset = row_offset;
+    fin.dec_loss = fin.dec_mi = fin.dec_tc = fin.dec_dimkl = fin.dec_means = nullptr;
+    if (lf.decomp) {
+        fin.dz = z; fin.lddz = ldz; fin.dmu = mu_all; fin.lddmu = ldmu; fin.dlv = logvar; fin.lddlv = ldlv;
+        fin.dec_loss = lf.loss_rows; fin.dec_mi = lf.mi_rows; fin.dec_tc = lf.tc_rows; fin.dec_dimkl = lf.dimkl_rows;
+        if (lf.means) { fin.dec_means = lf.means; fin.red_part = at<float>(workspace, p.off_red); fin.ticket = ticket; }
+    }
     if (lf.on) {
         fin.lv = logvar; fin.ldlv = ldlv; fin.mu_loc = peers.on() ? mu_all : mu_all + (int64_t)row_offset * ldmu; fin.ldmu = ldmu;
         fin.loss_rows = lf.loss_rows; fin.kl_rows = lf.kl_rows;
@@ -227,7 +239,7 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
     if (lf.fz.g_expelbo && !lf.fz.e_rows) return fail(TCELBO_ERR_INVALID, "g_expelbo needs the e_rows the forward wrote");
     if (!(flags & TCELBO_SAVE_FOR_BACKWARD)) return fail(TCELBO_ERR_INVALID, "backward needs the workspace of a forward run with TCELBO_SAVE_FOR_BACKWARD");
     if (!grad_z || !grad_mu_all || !grad_logvar) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
-    if (!lf.on && (!g_log_qz || !g_log_qz_prod)) return fail(TCELBO_ERR_INVALID, "null upstream gradient pointer");
+    if (!lf.on && !lf.decomp && (!g_log_qz || !g_log_qz_prod)) return fail(TCELBO_ERR_INVALID, "null upstream gradient pointer");
     if (ldgz < d || ldgmu < d || ldglv < d) return fail(TCELBO_ERR_INVALID, "gradient row pitch smaller than d");
     Plan p;
     if (!make_plan(p, b_loc, b_glob, d, flags, sm_count())) return fail(TCELBO_ERR_INVALID, "cannot plan this shape");
@@ -255,6 +267,7 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
     float* Apart = at<float>(scratch, p.boff_A);
     float* CRpart = at<float>(scratch, p.boff_CR);
     float* Gpart = at<float>(scratch, p.boff_G);
+    float* gpz = at<float>(scratch, p.boff_gpz);
 
     float* Glv = Gpart + (size_t)p.bg_pad * p.dp;                  // column-variance plans: the logvar column sums
 
@@ -266,7 +279,10 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
         up.g_loss_mean = lf.fz.g_loss_mean; up.g_kl_mean = lf.fz.g_kl_mean; up.g_expelbo = lf.fz.g_expelbo; up.e_rows = lf.fz.e_rows;
         up.scale = lf.fz.scale; up.g_rec_rows = lf.fz.g_rec_rows; up.beta = lf.beta;
         up.epoch = (peers.on() && peers.sync.on()) ? peers.sync.state + 1 : nullptr;
-        if ((e = launch_bwd_prep(p, up, S, gps, gj, lf.on ? gk : nullptr, Gpart, zero_n, st)) != cudaSuccess) return fail_cuda(e, "bwd_prep");
+        up.g_mi = lf.g_mi; up.g_tc = lf.g_tc; up.g_dimkl = lf.g_dimkl; up.g_dec_means = lf.g_means ? lf.g_means + 1 : nullptr;
+        up.gpz = lf.decomp ? gpz : nullptr;
+        if (lf.decomp) { up.g_loss = lf.g_loss; up.g_loss_mean = lf.g_means; }    // g_means[0]: the loss mean's gradient
+        if ((e = launch_bwd_prep(p, up, S, gps, gj, (lf.on || lf.decomp) ? gk : nullptr, Gpart, zero_n, st)) != cudaSuccess) return fail_cuda(e, "bwd_prep");
 
         BwdFusedArgs ua;
         ua.zs = zs; ua.ns = ns; ua.qmax = qmax; ua.gps = gps; ua.gj = gj; ua.J2 = J2; ua.mu_pad = mu_pad;
@@ -292,6 +308,7 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
         fa.scratch_parts = peers.on() ? peers.scratch_parts : nullptr; fa.g_off = p.boff_G; fa.n_ranks = peers.n_ranks;
         fa.eps = lf.fz.eps; fa.ldeps = lf.fz.ldeps;
         fa.sync = peers.sync;
+        fa.gc = lf.decomp ? gk : nullptr; fa.gpz = lf.decomp ? gpz : nullptr; fa.z = z; fa.ldz = ldz;   // gk holds gc (bwd_prep)
         if (p.var_col) {
             if ((e = launch_bwd_colvar_finalize(p, fa, mu_pad, Glv, st)) != cudaSuccess) return fail_cuda(e, "bwd_colvar_finalize");
         } else {
@@ -363,6 +380,41 @@ int tcelbo_klloss_backward_ex(const float* z, int64_t ldz, const float* mu_all, 
         return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
     return backward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
                          g_log_qz, g_log_qz_prod, lf, grad_z, ldgz, grad_mu_all, ldgmu, grad_logvar, ldglv,
+                         workspace, workspace_bytes, scratch, scratch_bytes, stream);
+}
+
+// Checked before anything touches the device, so that a wrong call fails the same way on a machine without a GPU.
+static int check_decomp(uint32_t flags, const void* z, const void* mu_all, const void* logvar) {
+    if (!(flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_INVALID, "the decomposition uses the column-variance density: flags need TCELBO_VAR_COL");
+    if (!z || !mu_all || !logvar) return fail(TCELBO_ERR_INVALID, "null input pointer");
+    return TCELBO_OK;
+}
+
+int tcelbo_decomp_forward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                          int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                          float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+    if (int rc = check_decomp(flags, z, mu_all, logvar)) return rc;
+    if (!loss_rows || !mi_rows || !tc_rows || !dimkl_rows) return fail(TCELBO_ERR_INVALID, "null output pointer");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.loss_rows = loss_rows; lf.mi_rows = mi_rows; lf.tc_rows = tc_rows; lf.dimkl_rows = dimkl_rows; lf.means = means;
+    return forward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
+                        nullptr, nullptr, lf, workspace, workspace_bytes, stream);
+}
+
+int tcelbo_decomp_backward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                           int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                           const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                           const float* g_means,
+                           float* grad_z, int64_t ldgz, float* grad_mu_all, int64_t ldgmu, float* grad_logvar, int64_t ldglv,
+                           const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream) {
+    if (int rc = check_decomp(flags, z, mu_all, logvar)) return rc;
+    if (!grad_z || !grad_mu_all || !grad_logvar) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
+    if (!g_loss_rows && !g_mi_rows && !g_tc_rows && !g_dimkl_rows && !g_means) return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.g_loss = g_loss_rows; lf.g_mi = g_mi_rows; lf.g_tc = g_tc_rows; lf.g_dimkl = g_dimkl_rows; lf.g_means = g_means;
+    return backward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
+                         nullptr, nullptr, lf, grad_z, ldgz, grad_mu_all, ldgmu, grad_logvar, ldglv,
                          workspace, workspace_bytes, scratch, scratch_bytes, stream);
 }
 

@@ -21,12 +21,15 @@ __device__ __forceinline__ void red_add_v4_cv(float* addr, float a, float b, flo
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" :: "l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
-// column operands: colpack[j][0..2][dp] = (sj, nmus, c2); rows: zpad[i][dp] (zero padded), shift[i][dp] = 0
+// column operands: colpack[j][0..2][dp] = (sj, nmus, c2); rows: zpad[i][dp] (zero padded), shift[i][dp] = 0; zeroes the
+// ticket of the finalize kernel's batch means (the workspace may be fresh, uninitialised memory)
 __global__ void colvar_prep_kernel(const float* __restrict__ z, int64_t ldz, const float* __restrict__ mu_all, int64_t ldmu,
                                    const float* __restrict__ lv_all, int64_t ldlv, int b_loc, int b_glob, int d,
                                    int bl_pad, int bg_pad, int dp,
-                                   float* __restrict__ colpack, float* __restrict__ zpad, float* __restrict__ shift) {
+                                   float* __restrict__ colpack, float* __restrict__ zpad, float* __restrict__ shift,
+                                   unsigned int* __restrict__ ticket) {
     const int64_t n_col = (int64_t)bg_pad * dp, n_row = (int64_t)bl_pad * dp;
+    if (blockIdx.x == 0 && threadIdx.x == 0) *ticket = 0u;
     for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n_col + n_row; idx += (int64_t)gridDim.x * blockDim.x) {
         if (idx < n_col) {
             const int j = (int)(idx / dp), dd = (int)(idx % dp);
@@ -376,6 +379,10 @@ tc_bwd_colvar_kernel(const BwdFusedArgs a) {
     }
 }
 
+// With the decomposition (a.gc != nullptr) the row-local densities of solvers/tc.py:107,112 add their gradients, the terms of
+// rowdensity_bwd_kernel: condx_i = sum_d lp(z_id; mu_rd, lv_rd) to grad_z[i] and to row r = row_offset + i of grad_mu / grad_lv
+// (the thread that owns (r, d) of the column part adds them, so no two threads write one element), pz_i = sum_d lp(z_id; 0, 0)
+// to grad_z[i].
 __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __restrict__ colpack, const float* __restrict__ Glv) {
     const int64_t n_row = (int64_t)a.b_loc * a.d;
     const int64_t n_col = (int64_t)a.b_glob * a.d;
@@ -385,14 +392,34 @@ __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __re
             const size_t o = (size_t)i * a.dp + dd;
             float sa = 0.0f;
             for (int s = 0; s < a.n_js; ++s) sa += a.Apart[(size_t)s * a.bl_pad * a.dp + o];
-            a.grad_z[(int64_t)i * a.ldgz + dd] = -kTwoLn2 * sa;
+            float gz = -kTwoLn2 * sa;
+            if (a.gc != nullptr) {
+                const int64_t r = (int64_t)a.row_offset + i;
+                const float x = a.z[(int64_t)i * a.ldz + dd];
+                float t, iv, t0, iv0;
+                const float lp = lp_unfloored(x, a.mu_all[r * a.ldmu + dd], a.lv[r * a.ldlv + dd], t, iv);
+                const float lp0 = lp_unfloored(x, 0.0f, 0.0f, t0, iv0);
+                const float gc = lp_passes_grad(lp) ? a.gc[i] : 0.0f, gp = lp_passes_grad(lp0) ? a.gpz[i] : 0.0f;
+                gz += -gc * t * iv + -gp * t0 * iv0;
+            }
+            a.grad_z[(int64_t)i * a.ldgz + dd] = gz;
         } else {
             const int64_t k = idx - n_row;
             const int j = (int)(k / a.d), dd = (int)(k % a.d);
             const size_t o = (size_t)j * a.dp + dd;
             const float sj = colpack[(size_t)j * 3 * a.dp + dd];
-            a.grad_mu[(int64_t)j * a.ldgmu + dd] = kTwoLn2 * sj * a.Gpart[o];
-            a.grad_lv[(int64_t)j * a.ldglv + dd] = Glv[o];
+            float gmu = kTwoLn2 * sj * a.Gpart[o], glv = Glv[o];
+            const int i = j - a.row_offset;
+            if (a.gc != nullptr && i >= 0 && i < a.b_loc) {
+                const float m = a.mu_all[(int64_t)j * a.ldmu + dd], l = a.lv[(int64_t)j * a.ldlv + dd];
+                float t, iv;
+                const float lp = lp_unfloored(a.z[(int64_t)i * a.ldz + dd], m, l, t, iv);
+                const float gc = lp_passes_grad(lp) ? a.gc[i] : 0.0f;
+                gmu += gc * t * iv;
+                glv += gc * 0.5f * (t * t * iv - 1.0f);
+            }
+            a.grad_mu[(int64_t)j * a.ldgmu + dd] = gmu;
+            a.grad_lv[(int64_t)j * a.ldglv + dd] = glv;
         }
     }
 }
@@ -401,12 +428,12 @@ __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __re
 // launchers
 // ------------------------------------------------------------------------------------------------------
 cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* lv_all, int64_t ldlv,
-                               const Plan& p, float* colpack, float* zpad, float* shift, cudaStream_t st) {
+                               const Plan& p, float* colpack, float* zpad, float* shift, unsigned int* ticket, cudaStream_t st) {
     const int64_t n = (int64_t)(p.bg_pad + p.bl_pad) * p.dp;
     int64_t g = (n + 255) / 256; if (g > 148 * 16) g = 148 * 16;
     LaunchScope scope(kKernNone, st);
     colvar_prep_kernel<<<(int)g, 256, 0, st>>>(z, ldz, mu_all, ldmu, lv_all, ldlv, p.b_loc, p.b_glob, p.d, p.bl_pad, p.bg_pad, p.dp,
-                                                colpack, zpad, shift);
+                                                colpack, zpad, shift, ticket);
     return cudaGetLastError();
 }
 

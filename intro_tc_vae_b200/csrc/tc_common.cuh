@@ -55,6 +55,20 @@ __device__ __forceinline__ float fmax_nan(float a, float b) {
     float y; asm("max.NaN.f32 %0, %1, %2;" : "=f"(y) : "f"(a), "f"(b)); return y;
 }
 
+// ---- un-floored Gaussian log-density of one element (ops.py:24-29), shared by the row-density kernels and the column-variance
+//      finalize kernels so that their terms agree bit for bit ----------------------------------------------------------------
+// lp = -0.5 * ((x - mu)^2 * exp(-lv) + lv + log 2pi), before the -50 clamp; t = x - mu and iv = exp(-lv) are returned for the
+// gradient.  The roundings are spelled out so that constant operands (the prior: mu = lv = 0) cannot change them.  With
+// lv < -88.7 and x == mu the product is 0 * inf = NaN, as in the reference.
+__device__ __forceinline__ float lp_unfloored(float x, float mu, float lv, float& t, float& iv) {
+    t = x - mu;
+    iv = expf(-lv);
+    return -0.5f * __fadd_rn(fmaf(__fmul_rn(t, t), iv, lv), kLog2Pi);
+}
+// the clamped value (max.NaN: a NaN term stays NaN, like torch.clamp) and the gradient mask of the clamp
+__device__ __forceinline__ float lp_clamped(float lp) { return fmax_nan(lp, kLogpFloor); }
+__device__ __forceinline__ bool lp_passes_grad(float lp) { return lp >= kLogpFloor; }
+
 // ---- mbarrier + 1-D bulk TMA (cp.async.bulk -> UBLKCP) -------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));

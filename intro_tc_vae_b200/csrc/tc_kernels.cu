@@ -344,7 +344,8 @@ tc_fwd_kernel(const FwdArgs a) {
 }
 
 // One warp per row: sum the column-split partials (float4 per lane, 8 independent loads in flight), take logs,
-// emit log_qz / log_qz_prod and, when asked, the fused KL and (beta-1)*TC + KL of solvers/tc.py:83-89.
+// emit log_qz / log_qz_prod and, when asked, either the fused KL and (beta-1)*TC + KL of solvers/tc.py:83-89 (a.lv) or the
+// MI / TC / dimension-wise KL decomposition of solvers/tc.py:91-144 (a.dz).  Neither mode computes the other's terms.
 __global__ void fwd_finalize_kernel(const FinArgs a) {
     pdl_trigger(); pdl_wait();                               // programmatic dependent launch, tc_common.cuh
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -384,13 +385,25 @@ __global__ void fwd_finalize_kernel(const FinArgs a) {
             kl += 1.0f + l - expf(l) - m * m;
         }
     }
+    float condx = 0.0f, pz = 0.0f;                           // decomposition: log q(z_i|x_i) and log p(z_i), summed over d in
+    if (a.dz != nullptr) {                                   // the order of rowdensity_fwd_kernel, so they equal ops.row_log_density
+        const int64_t r = (int64_t)a.row_offset + row;
+        for (int dd = lane; dd < a.d; dd += 32) {
+            const float x = a.dz[(int64_t)row * a.lddz + dd];
+            float t, iv;
+            condx += lp_clamped(lp_unfloored(x, a.dmu[r * a.lddmu + dd], a.dlv[r * a.lddlv + dd], t, iv));
+            pz += lp_clamped(lp_unfloored(x, 0.0f, 0.0f, t, iv));
+        }
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         P += __shfl_xor_sync(0xffffffffu, P, o);
         C += __shfl_xor_sync(0xffffffffu, C, o);
         kl += __shfl_xor_sync(0xffffffffu, kl, o);
+        condx += __shfl_xor_sync(0xffffffffu, condx, o);
+        pz += __shfl_xor_sync(0xffffffffu, pz, o);
     }
-    float loss_i = 0.0f, kl_i = 0.0f, e_i = 0.0f;
+    float red[4] = {0.0f, 0.0f, 0.0f, 0.0f};                // this row's share of the batch means
     if (lane == 0 && row_ok) {
         const float2* pj = reinterpret_cast<const float2*>(a.Jpart);
         float m = kNegBig, s = 0.0f;
@@ -403,51 +416,65 @@ __global__ void fwd_finalize_kernel(const FinArgs a) {
         const float J2 = m + log2f(s);
         const float lq = kLn2 * J2 + C + a.lw_u;
         a.J2[row] = J2;
-        a.log_qz[row] = lq;
-        a.log_qz_prod[row] = P;
-        if (a.lv != nullptr) {
+        if (a.log_qz != nullptr) a.log_qz[row] = lq;
+        if (a.log_qz_prod != nullptr) a.log_qz_prod[row] = P;
+        if (a.lv != nullptr) {                               // red = (loss, kl, exp-ELBO, -)
             kl *= -0.5f;
             a.kl_rows[row] = kl;
-            loss_i = (a.beta - 1.0f) * (lq - P) + kl;
-            kl_i = kl;
+            const float loss_i = (a.beta - 1.0f) * (lq - P) + kl;
+            red[0] = loss_i; red[1] = kl;
             a.loss_rows[row] = loss_i;
             if (a.rec_rows != nullptr) {
-                e_i = expf(-2.0f * a.scale * (a.rec_rows[row] + loss_i));
-                a.e_rows[row] = e_i;
+                red[2] = expf(-2.0f * a.scale * (a.rec_rows[row] + loss_i));
+                a.e_rows[row] = red[2];
             }
+        } else if (a.dz != nullptr) {                        // red = (loss, mi, tc, dimkl)
+            const float mi = condx - lq, tc = lq - P, dimkl = P - pz;
+            red[0] = mi + a.beta * tc + dimkl; red[1] = mi; red[2] = tc; red[3] = dimkl;
+            a.dec_loss[row] = red[0]; a.dec_mi[row] = mi; a.dec_tc[row] = tc; a.dec_dimkl[row] = dimkl;
         }
     }
     if (a.red_part == nullptr) return;
     // ---- batch means: per-CTA partials in a fixed slot, summed in fixed order by the last CTA to arrive (deterministic)
-    __shared__ float sh[3][kFinWarps];
+    __shared__ float sh[4][kFinWarps];
     __shared__ bool last;
-    if (lane == 0) { sh[0][warp] = loss_i; sh[1][warp] = kl_i; sh[2][warp] = e_i; }
+    if (lane == 0) {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) sh[q][warp] = red[q];
+    }
     __syncthreads();
     if (threadIdx.x == 0) {
-        float t0 = 0.0f, t1 = 0.0f, t2 = 0.0f;
-        for (int w = 0; w < kFinWarps; ++w) { t0 += sh[0][w]; t1 += sh[1][w]; t2 += sh[2][w]; }
-        a.red_part[blockIdx.x] = t0; a.red_part[gridDim.x + blockIdx.x] = t1; a.red_part[2 * gridDim.x + blockIdx.x] = t2;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            float tq = 0.0f;
+            for (int w = 0; w < kFinWarps; ++w) tq += sh[q][w];
+            a.red_part[q * gridDim.x + blockIdx.x] = tq;
+        }
         __threadfence();
         last = (atomicAdd(a.ticket, 1u) == gridDim.x - 1);
     }
     __syncthreads();
     if (!last || warp != 0) return;
     __threadfence();
-    float t[3] = {0.0f, 0.0f, 0.0f};
+    float t[4] = {0.0f, 0.0f, 0.0f, 0.0f};
     for (int k = lane; k < (int)gridDim.x; k += 32) {
 #pragma unroll
-        for (int q = 0; q < 3; ++q) t[q] += *(volatile float*)(a.red_part + q * gridDim.x + k);
+        for (int q = 0; q < 4; ++q) t[q] += *(volatile float*)(a.red_part + q * gridDim.x + k);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
-        for (int q = 0; q < 3; ++q) t[q] += __shfl_xor_sync(0xffffffffu, t[q], o);
+        for (int q = 0; q < 4; ++q) t[q] += __shfl_xor_sync(0xffffffffu, t[q], o);
     }
     if (lane == 0) {
         const float inv_b = 1.0f / (float)a.b_loc;
         if (a.loss_mean) a.loss_mean[0] = t[0] * inv_b;
         if (a.kl_mean) a.kl_mean[0] = t[1] * inv_b;
         if (a.expelbo) a.expelbo[0] = t[2] * inv_b;
+        if (a.dec_means) {
+#pragma unroll
+            for (int q = 0; q < 4; ++q) a.dec_means[q] = t[q] * inv_b;
+        }
         *a.ticket = 0u;
     }
 }
@@ -469,6 +496,10 @@ __global__ void bwd_prep_kernel(const BwdUpstream u, const float* __restrict__ S
     const float gl_mean = u.g_loss_mean ? u.g_loss_mean[0] * inv_b : 0.0f;
     const float gk_mean = u.g_kl_mean ? u.g_kl_mean[0] * inv_b : 0.0f;
     const float ge = u.g_expelbo ? u.g_expelbo[0] * (-2.0f * u.scale * inv_b) : 0.0f;
+    const float gm_mean = u.g_dec_means ? u.g_dec_means[0] * inv_b : 0.0f;      // decomposition: d/d of the mi, tc, dimkl means
+    const float gt_mean = u.g_dec_means ? u.g_dec_means[1] * inv_b : 0.0f;
+    const float gd_mean = u.g_dec_means ? u.g_dec_means[2] * inv_b : 0.0f;
+    auto g_term = [](const float* rows, float mean, int i) { return (rows ? rows[i] : 0.0f) + mean; };
     if (u.epoch != nullptr && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(u.epoch, 1u);   // opens the backward exchange's barrier
     auto g_loss_of = [&](int i, float& g_rec) {                 // dLoss/dloss_rows[i]; g_rec = its exp-ELBO part (= dLoss/drec_rows[i])
         g_rec = u.g_expelbo ? ge * u.e_rows[i] : 0.0f;
@@ -486,6 +517,7 @@ __global__ void bwd_prep_kernel(const BwdUpstream u, const float* __restrict__ S
             float g_rec, gP = 0.0f;
             if (u.g_log_qz_prod) gP += u.g_log_qz_prod[i];
             gP -= (u.beta - 1.0f) * g_loss_of(i, g_rec);
+            if (u.gpz) gP += g_term(u.g_dimkl, gd_mean, i) - g_term(u.g_tc, gt_mean, i);
             const float4 sv = reinterpret_cast<const float4*>(S)[idx];
             o = make_float4(gP / sv.x, gP / sv.y, gP / sv.z, gP / sv.w);
         }
@@ -501,6 +533,12 @@ __global__ void bwd_prep_kernel(const BwdUpstream u, const float* __restrict__ S
             k = gl + gk_mean;
             if (u.g_kl) k += u.g_kl[idx];
             if (u.g_rec_rows) u.g_rec_rows[idx] = g_rec;
+            if (u.gpz) {                                                  // k is gc, the coefficient of condx
+                const float gm = g_term(u.g_mi, gm_mean, (int)idx), gd = g_term(u.g_dimkl, gd_mean, (int)idx);
+                gJ += g_term(u.g_tc, gt_mean, (int)idx) - gm;
+                k = gl + gm;
+                u.gpz[idx] = -(gl + gd);
+            }
         }
         gj[idx] = gJ;
         if (gk) gk[idx] = k;

@@ -32,7 +32,15 @@ struct FinArgs {
     //   loss_mean = mean_i loss_rows[i], kl_mean = mean_i kl_rows[i]               (solvers/tc.py:83-89 with reduce="mean")
     //   e_rows[i] = exp(-2*scale*(rec_rows[i] + loss_rows[i])), expelbo = mean_i e_rows[i]   (solvers/intro.py:102-103)
     float* loss_mean; float* kl_mean; const float* rec_rows; float scale; float* expelbo; float* e_rows;
-    float* red_part; unsigned int* ticket;                       // [3][gridDim.x] partial sums, arrival counter (zeroed by the prologue)
+    // optional MI / TC / dimension-wise KL decomposition of solvers/tc.py:91-144 (column-variance plans; dz == nullptr: off),
+    // per local row i with global row r = row_offset + i:
+    //   condx_i = sum_d lp(z_id; mu_rd, lv_rd), pz_i = sum_d lp(z_id; 0, 0)      (lp: tc_common.cuh lp_unfloored, clamped)
+    //   mi_i = condx_i - log_qz_i, tc_i = log_qz_i - log_qz_prod_i, dimkl_i = log_qz_prod_i - pz_i, loss_i = mi_i + beta*tc_i + dimkl_i
+    //   dec_means[0..3] = the batch means of loss, mi, tc, dimkl (nullptr: none)
+    const float* dz; int64_t lddz; const float* dmu; int64_t lddmu; const float* dlv; int64_t lddlv;   // z rows; mu / logvar [b_glob]
+    int row_offset;
+    float* dec_loss; float* dec_mi; float* dec_tc; float* dec_dimkl; float* dec_means;
+    float* red_part; unsigned int* ticket;                       // [4][gridDim.x] partial sums, arrival counter (zeroed by the prologue)
 };
 
 // One prologue kernel: pads / gathers the column operand, derives the per-(i,d) row constants, optionally forms
@@ -77,6 +85,9 @@ struct BwdFinArgs {
     // receives grad_z * eps * 0.5 * exp(logvar / 2), i.e. the outputs are the gradients w.r.t. the encoder's mu / logvar
     const float* eps; int64_t ldeps;
     PeerSync sync;                                               // peer exchange: barrier between the ranks' sweeps and this reduce
+    // column-variance decomposition (BwdUpstream::gpz): the row-local gradients of condx_i (coefficient gc_i) and pz_i (gpz_i),
+    // masked where lp < -50, on grad_z[i] and on row r = row_offset + i of grad_mu / grad_lv (nullptr: off)
+    const float* gc; const float* gpz; const float* z; int64_t ldz;
 };
 
 cudaError_t launch_prep(const PrepArgs& a, cudaStream_t st);
@@ -94,13 +105,19 @@ struct BwdUpstream {
     float* g_rec_rows;
     float beta;
     unsigned int* epoch;          // peer exchange with in-kernel barriers: the backward barrier counter this prologue advances
+    // MI / TC / dimension-wise KL decomposition (FinArgs::dz; gpz == nullptr: off).  g_loss / g_loss_mean carry the loss's
+    // gradient as above, g_mi / g_tc / g_dimkl [b_loc] (any may be null) and g_dec_means[0..2] (the mi, tc, dimkl means; may be
+    // null) the terms'; with gX_i = g_X[i] + g_dec_means[X]/b_loc:
+    //   gJ_i = (beta-1)*gl_i - g_mi_i + g_tc_i,  gP_i = (1-beta)*gl_i - g_tc_i + g_dimkl_i,
+    //   gk_i = gl_i + g_mi_i (coefficient of condx_i),  gpz[i] = -(gl_i + g_dimkl_i) (coefficient of pz_i)
+    const float* g_mi; const float* g_tc; const float* g_dimkl; const float* g_dec_means; float* gpz;
 };
 cudaError_t launch_bwd_prep(const Plan& p, const BwdUpstream& u, const float* S, float* gps, float* gj, float* gk,
                             float* zero, size_t zero_n, cudaStream_t st);
 cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, cudaStream_t st);
 // column-variance ("full" path) variant, tc_colvar.cu
 cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* lv_all, int64_t ldlv,
-                               const Plan& p, float* colpack, float* zpad, float* shift, cudaStream_t st);
+                               const Plan& p, float* colpack, float* zpad, float* shift, unsigned int* ticket, cudaStream_t st);
 cudaError_t launch_fwd_colvar(const Plan& p, const FwdArgs& a, cudaStream_t st);
 cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, cudaStream_t st);
 cudaError_t launch_bwd_colvar_finalize(const Plan& p, const BwdFinArgs& a, const float* colpack, const float* Glv, cudaStream_t st);

@@ -81,7 +81,7 @@ struct Plan {
     size_t off_scratch;                                           // forward split partials (S, J)
     size_t total_bytes;                                           // forward workspace (read-only in backward)
     // backward scratch (its own buffer, so the forward workspace stays immutable and backward can be re-run)
-    size_t boff_gps, boff_gj, boff_gk, boff_A, boff_CR, boff_G, bwd_bytes;
+    size_t boff_gps, boff_gj, boff_gk, boff_A, boff_CR, boff_G, boff_gpz, bwd_bytes;
     bool save, var_col;
     int fwd_lpr, fwd_kch, fwd_warps;   // forward sweep mapping: lanes per row, 16-byte chunks (4 dims) per lane, warps per CTA
     bool small;                // fewer work units than SMs with the standard tiles: small-tile / few-rows instantiations
@@ -194,7 +194,7 @@ inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int
     p.off_S = off;     off = align256(off + row_arr);
     p.off_J2 = off;    off = align256(off + (size_t)p.bl_pad * sizeof(float));
     p.n_fin_ctas = (b_loc + kFinWarps - 1) / kFinWarps;
-    p.off_red = off;   off = align256(off + ((size_t)3 * p.n_fin_ctas + 4) * sizeof(float));
+    p.off_red = off;   off = align256(off + ((size_t)4 * p.n_fin_ctas + 4) * sizeof(float));    // 4 means per CTA, then the ticket
     p.ld_s2 = p.bg_pad;
     p.off_s2 = off;    off = align256(off + (p.save ? (size_t)p.bl_pad * p.ld_s2 * sizeof(float) : 0));
     const int n_part = p.n_js_fwd > p.slots_fwd ? p.n_js_fwd : p.slots_fwd;
@@ -210,6 +210,7 @@ inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int
     p.boff_A = b;   b = align256(b + (size_t)kMaxSplits * row_arr);          // row-local partial sums per column split
     p.boff_CR = b;  b = align256(b + (size_t)kMaxSplits * row_arr);
     p.boff_G = b;   b = align256(b + 2 * col_arr);                           // column accumulators (mu [, logvar])
+    p.boff_gpz = b; b = align256(b + (p.var_col ? (size_t)p.bl_pad * sizeof(float) : 0));   // decomposition: coefficient of log p(z_i)
     p.bwd_bytes = b;
     return true;
 }

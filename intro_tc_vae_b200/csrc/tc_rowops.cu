@@ -67,7 +67,8 @@ __global__ void reparam_bwd_kernel(const float* __restrict__ lv, int64_t ldlv, c
     }
 }
 
-// lp = max(-0.5*((x-mu)^2*exp(-lv) + lv + log2pi), -50); the reference's log 2pi is an fp32 constant (ops.py:25)
+// lp = max(-0.5*((x-mu)^2*exp(-lv) + lv + log2pi), -50) (tc_common.cuh: lp_unfloored); the reference's log 2pi is an fp32
+// constant (ops.py:25)
 __global__ void rowdensity_fwd_kernel(const float* __restrict__ x, int64_t ldx, const float* __restrict__ mu, int64_t ldmu,
                                       const float* __restrict__ lv, int64_t ldlv, int b, int d, float* __restrict__ out) {
     const int row = blockIdx.x * kRowWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -77,9 +78,8 @@ __global__ void rowdensity_fwd_kernel(const float* __restrict__ x, int64_t ldx, 
         const float xv = x[(int64_t)row * ldx + dd];
         const float m = mu ? mu[(int64_t)row * ldmu + dd] : 0.0f;
         const float l = lv ? lv[(int64_t)row * ldlv + dd] : 0.0f;
-        const float t = xv - m;
-        const float lp = -0.5f * (t * t * expf(-l) + l + kLog2Pi);
-        acc += fmax_nan(lp, kLogpFloor);
+        float t, iv;
+        acc += lp_clamped(lp_unfloored(xv, m, l, t, iv));
     }
     acc = warp_sum(acc);
     if (lane == 0) out[row] = acc;
@@ -95,9 +95,9 @@ __global__ void rowdensity_bwd_kernel(const float* __restrict__ x, int64_t ldx, 
         const float xv = x[(int64_t)i * ldx + dd];
         const float m = mu ? mu[(int64_t)i * ldmu + dd] : 0.0f;
         const float l = lv ? lv[(int64_t)i * ldlv + dd] : 0.0f;
-        const float t = xv - m, iv = expf(-l);
-        const float lp = -0.5f * (t * t * iv + l + kLog2Pi);
-        const float g = (lp >= kLogpFloor) ? g_rows[i] : 0.0f;            // clamp passes gradient where lp >= -50
+        float t, iv;
+        const float lp = lp_unfloored(xv, m, l, t, iv);
+        const float g = lp_passes_grad(lp) ? g_rows[i] : 0.0f;            // clamp passes gradient where lp >= -50
         if (gx) gx[(int64_t)i * ldgx + dd] = -g * t * iv;
         if (gmu) gmu[(int64_t)i * ldgmu + dd] = g * t * iv;
         if (glv) glv[(int64_t)i * ldglv + dd] = g * 0.5f * (t * t * iv - 1.0f);

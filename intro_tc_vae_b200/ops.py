@@ -8,6 +8,7 @@ returns ``(log_qz_prod, log_qz)`` directly and recomputes tiles in backward.
 Reference map (file:line in the reference repository):
     total_correlation            ops.py:52-89
     tc_terms                     ops.py:80-84 + 104-115 / 92-101 fused (and solvers/tc.py:114-119 for var_of="col")
+    tc_decomp_loss_*             solvers/tc.py:91-144 fused (MI + beta*TC + dimension-wise KL)
     kl_divergence / kl_no_reduce ops.py:136-163   (argument order: logvar, mu)
     reparameterize               ops.py:166-185
     log_importance_weight_matrix ops.py:32-49
@@ -26,7 +27,8 @@ from .losses import reconstruction_loss          # ops.py:188-236 lives in ops i
 from .sharding import gather_rows, shard_rows
 
 __all__ = [
-    "total_correlation", "tc_terms", "kl_tc_loss_terms", "kl_tc_loss_mean", "reconstruction_loss", "kl_divergence", "kl_no_reduce", "reparameterize",
+    "total_correlation", "tc_terms", "kl_tc_loss_terms", "kl_tc_loss_mean", "tc_decomp_loss_terms", "tc_decomp_loss_mean",
+    "reconstruction_loss", "kl_divergence", "kl_no_reduce", "reparameterize",
     "log_importance_weight_matrix", "row_log_density", "gaussian_log_density_torch", "gaussian_log_density",
     "minibatch_stratified_sampling", "minibatch_weighted_sampling",
 ]
@@ -303,6 +305,138 @@ def kl_tc_loss_mean(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, be
     if loss_mean is None:                                        # peer-memory path: per-row outputs only
         return loss.mean(), kl.mean()
     return loss_mean, kl_mean
+
+
+# --------------------------------------------------------------------------------------------------
+# fused MI / TC / dimension-wise KL decomposition:  torch.ops.tcelbo.decomp_forward / decomp_backward
+# --------------------------------------------------------------------------------------------------
+@torch.library.custom_op("tcelbo::decomp_forward", mutates_args=(), device_types="cuda")
+def _decomp_forward(z: Tensor, mu_all: Tensor, logvar_all: Tensor, row_offset: int, dataset_size: int, flags: int,
+                    beta: float) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """-> (loss [B], mi [B], tc [B], dimkl [B], means [4], workspace): the per-sample terms of solvers/tc.py:91-144 on the
+    column-variance density and their batch means (loss, mi, tc, dimkl), reduced inside the finalize kernel."""
+    lib = _lib.load()
+    z, mu_all, logvar_all = _rows(z), _rows(mu_all), _rows(logvar_all)
+    b_loc, d = z.shape
+    b_glob = mu_all.shape[0]
+    nbytes = lib.tcelbo_workspace_bytes(b_loc, b_glob, d, flags)
+    if nbytes == 0:
+        raise NotImplementedError(f"tcelbo: unsupported shape b_loc={b_loc} b_glob={b_glob} d={d} (d must be <= 512)")
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=z.device)
+    out = [torch.empty(b_loc, dtype=torch.float32, device=z.device) for _ in range(4)]   # loss, mi, tc, dimkl
+    means = torch.empty(4, dtype=torch.float32, device=z.device)
+    with torch.cuda.device(z.device):
+        st = lib.tcelbo_decomp_forward(z.data_ptr(), z.stride(0), mu_all.data_ptr(), mu_all.stride(0),
+                                       logvar_all.data_ptr(), logvar_all.stride(0), b_loc, b_glob, row_offset, d, dataset_size,
+                                       flags, beta, *(t.data_ptr() for t in out), means.data_ptr(), ws.data_ptr(), nbytes, _stream(z))
+    _lib.check(st, "tcelbo_decomp_forward")
+    return out[0], out[1], out[2], out[3], means, ws
+
+
+@_decomp_forward.register_fake
+def _(z, mu_all, logvar_all, row_offset, dataset_size, flags, beta):
+    nbytes = _lib.load().tcelbo_workspace_bytes(z.shape[0], mu_all.shape[0], z.shape[1], flags)
+    b = z.shape[0]
+    return (z.new_empty(b), z.new_empty(b), z.new_empty(b), z.new_empty(b), z.new_empty(4), z.new_empty(nbytes, dtype=torch.uint8))
+
+
+@torch.library.custom_op("tcelbo::decomp_backward", mutates_args=(), device_types="cuda")
+def _decomp_backward(z: Tensor, mu_all: Tensor, logvar_all: Tensor, row_offset: int, dataset_size: int, flags: int, beta: float,
+                     g_loss: Optional[Tensor], g_mi: Optional[Tensor], g_tc: Optional[Tensor], g_dimkl: Optional[Tensor],
+                     g_means: Optional[Tensor], workspace: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    _alert_not_deterministic("tcelbo::decomp_backward")
+    lib = _lib.load()
+    z, mu_all, logvar_all = _rows(z), _rows(mu_all), _rows(logvar_all)
+    b_loc, d = z.shape
+    b_glob = mu_all.shape[0]
+    ups = [t.contiguous() if t is not None else None for t in (g_loss, g_mi, g_tc, g_dimkl, g_means)]
+    grad_z = torch.empty(b_loc, d, dtype=torch.float32, device=z.device)
+    grad_mu = torch.empty(b_glob, d, dtype=torch.float32, device=z.device)
+    grad_lv = torch.empty(b_glob, d, dtype=torch.float32, device=z.device)
+    nscratch = lib.tcelbo_backward_scratch_bytes(b_loc, b_glob, d, flags)
+    scratch = torch.empty(nscratch, dtype=torch.uint8, device=z.device)
+    with torch.cuda.device(z.device):
+        st = lib.tcelbo_decomp_backward(z.data_ptr(), z.stride(0), mu_all.data_ptr(), mu_all.stride(0),
+                                        logvar_all.data_ptr(), logvar_all.stride(0), b_loc, b_glob, row_offset, d, dataset_size,
+                                        flags, beta, *(t.data_ptr() if t is not None else None for t in ups),
+                                        grad_z.data_ptr(), d, grad_mu.data_ptr(), d, grad_lv.data_ptr(), d,
+                                        workspace.data_ptr(), workspace.numel(), scratch.data_ptr(), nscratch, _stream(z))
+    _lib.check(st, "tcelbo_decomp_backward")
+    return grad_z, grad_mu, grad_lv
+
+
+@_decomp_backward.register_fake
+def _(z, mu_all, logvar_all, row_offset, dataset_size, flags, beta, g_loss, g_mi, g_tc, g_dimkl, g_means, workspace):
+    return (z.new_empty(z.shape), mu_all.new_empty(mu_all.shape), logvar_all.new_empty(logvar_all.shape))
+
+
+def _decomp_setup_context(ctx, inputs, output):
+    ctx.set_materialize_grads(False)          # unused outputs arrive as None instead of zero-filled tensors
+    z, mu_all, logvar_all, row_offset, dataset_size, flags, beta = inputs
+    ctx.save_for_backward(z, mu_all, logvar_all, output[5])
+    ctx.meta = (row_offset, dataset_size, flags, beta)
+
+
+def _decomp_autograd_backward(ctx, g_loss, g_mi, g_tc, g_dimkl, g_means, _g_ws):
+    z, mu_all, logvar_all, ws = ctx.saved_tensors
+    row_offset, dataset_size, flags, beta = ctx.meta
+    if not flags & _lib.SAVE_FOR_BACKWARD:
+        raise RuntimeError("tcelbo: forward ran without TCELBO_SAVE_FOR_BACKWARD but a gradient was requested")
+    if all(g is None for g in (g_loss, g_mi, g_tc, g_dimkl, g_means)):
+        return None, None, None, None, None, None, None
+    gz, gmu, glv = _decomp_backward(z, mu_all, logvar_all, row_offset, dataset_size, flags, beta,
+                                    g_loss, g_mi, g_tc, g_dimkl, g_means, ws)
+    return gz, gmu, glv, None, None, None, None
+
+
+_decomp_forward.register_autograd(_decomp_autograd_backward, setup_context=_decomp_setup_context)
+
+
+def _decomp(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str, group):
+    """Shared front end of :func:`tc_decomp_loss_terms` / :func:`tc_decomp_loss_mean` -> the op's 5 tensor outputs."""
+    for name, t in (("z", z), ("mu", mu), ("logvar", logvar)):
+        _check(name, t)
+    if not (z.shape == mu.shape == logvar.shape):
+        raise ValueError(f"z, mu, logvar must have one shape, got {tuple(z.shape)}, {tuple(mu.shape)}, {tuple(logvar.shape)}")
+    if estimator not in ("mss", "mws"):
+        raise ValueError(f"estimator must be 'mss' or 'mws', got {estimator!r}")
+    flags = (_lib.EST_MSS if estimator == "mss" else _lib.EST_MWS) | _lib.VAR_COL
+    if torch.is_grad_enabled() and (z.requires_grad or mu.requires_grad or logvar.requires_grad):
+        flags |= _lib.SAVE_FOR_BACKWARD
+    row_offset, mu_all, lv_all = 0, mu, logvar
+    if group is not None:
+        import torch.distributed as dist
+        if dist.get_world_size(group) > 1:
+            row_offset, _ = shard_rows(group, z.shape[0], z.device)
+            mu_all = gather_rows(mu, group)
+            lv_all = gather_rows(logvar, group)
+    if estimator == "mss" and mu_all.shape[0] == 1:
+        raise ZeroDivisionError("float division by zero")       # ops.py:44 with M = B-1 = 0
+    return _decomp_forward(z, mu_all, lv_all, row_offset, int(dataset_size), flags, float(beta))[:5]
+
+
+def tc_decomp_loss_terms(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str = "mss",
+                         group=None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """One fused evaluation of ``TCSovler._compute_kl_loss_full`` (solvers/tc.py:91-144), the beta-TCVAE loss, per sample:
+
+        mi_i = log q(z_i|x_i) - log q(z_i),  tc_i = log q(z_i) - sum_d log q(z_id),  dimkl_i = sum_d log q(z_id) - log p(z_i)
+        loss_i = mi_i + beta * tc_i + dimkl_i
+
+    on the column-variance density (``tc_terms(..., var_of="col")``; ``log q(z_i|x_i)`` and ``log p(z_i)`` as in
+    :func:`row_log_density`).  Returns ``(loss [B], mi [B], tc [B], dimkl [B])``.  The two row densities and the combine are
+    folded into the TC kernels' finalize steps, forward and backward: three kernels each way.  ``group`` row-shards the batch
+    exactly as :func:`tc_terms` with ``var_of="col"`` does (``mu`` and ``logvar`` all-gathered, column gradients
+    reduce-scattered); outputs cover the local rows.
+    """
+    return _decomp(z, mu, logvar, dataset_size, beta, estimator, group)[:4]
+
+
+def tc_decomp_loss_mean(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str = "mss",
+                        group=None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """``reduce="mean"`` form of :func:`tc_decomp_loss_terms`: 0-d ``(mean loss, mean mi, mean tc, mean dimkl)``.  The means
+    come out of the finalize kernel (deterministic last-CTA reduction) and their gradients enter the backward prologue as
+    device scalars.  Row-sharded calls return the means over the local rows."""
+    return tuple(_decomp(z, mu, logvar, dataset_size, beta, estimator, group)[4].unbind(0))
 
 
 def tc_terms(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, estimator: str = "mss",

@@ -69,25 +69,22 @@ class TCLossMixin:
 
     def _compute_kl_loss_full(self, z: Optional[Tensor], mu: Tensor, logvar: Tensor, reduce: str = "mean",
                               beta: float = None, write: bool = False) -> Tensor:
-        """solvers/tc.py:91-144: MI + beta * TC + dimension-wise KL, column-variance density, MSS."""
+        """solvers/tc.py:91-144: MI + beta * TC + dimension-wise KL, column-variance density, MSS.  One fused op: the row
+        densities, the combine and (for reduce="mean") the batch means ride in the TC kernels' finalize steps."""
         if beta is None:
             beta = self.beta_kl
         dataset_size = len(self.dataset)
-        logqz_condx = ops.row_log_density(z, mu, logvar)
-        logpz = ops.row_log_density(z)
-        logqz_prodmarginals, log_qz = ops.tc_terms(z, mu, logvar, dataset_size, "mss", "col",
-                                                   getattr(self, "process_group", None))
-        mi_loss = logqz_condx - log_qz
-        tc_loss = log_qz - logqz_prodmarginals
-        kl_loss = logqz_prodmarginals - logpz
+        group = getattr(self, "process_group", None)
         sw = _singleton_writer()
         if reduce == "mean":
-            mi_loss, tc_loss, kl_loss = mi_loss.mean(), tc_loss.mean(), kl_loss.mean()
+            loss, mi_loss, tc_loss, kl_loss = ops.tc_decomp_loss_mean(z, mu, logvar, dataset_size, beta, "mss", group)
             if sw.writer:
                 sw.writer.add_scalars(
                     "tc_decomp",
                     {"mi": mi_loss.data.item(), "tc": tc_loss.data.item(), "kl": kl_loss.data.item()},
                     global_step=sw.cur_iter)
+        else:
+            loss, mi_loss, tc_loss, kl_loss = ops.tc_decomp_loss_terms(z, mu, logvar, dataset_size, beta, "mss", group)
         if write:
             self.write_scalar(sw.cur_iter, "kl_loss_unscaled", mi_loss + tc_loss + kl_loss)
-        return mi_loss + beta * tc_loss + kl_loss
+        return loss

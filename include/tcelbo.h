@@ -172,7 +172,8 @@ int tcelbo_klloss_backward_ex(const float* z, int64_t ldz, const float* mu_all, 
  * kernel.  The backward takes dLoss/d of the four per-row outputs and g_means (DEVICE float[4], dLoss/d of the four means); each
  * may be NULL (= zero) as long as one is given.  It adds the gradients of condx and pz to grad_z, to grad_logvar [b_glob, D] and to
  * rows [row_offset, row_offset + b_loc) of grad_mu_all, so no row-density or elementwise kernels are launched: 3 kernels forward,
- * 3 backward.  The peer-memory exchange and the fused reparameterize cover the row-variance density only.
+ * 3 backward.  The row-sharded peer-memory form is tcelbo_decomp_forward_peer / _backward_peer below; the fused reparameterize
+ * (tcelbo_fusion.eps) covers the row-variance density only.
  */
 int tcelbo_decomp_forward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
                           int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
@@ -198,8 +199,9 @@ int tcelbo_decomp_backward(const float* z, int64_t ldz, const float* mu_all, int
  *             scratch buffers of all ranks (`scratch_parts`, DEVICE array of n_ranks scratch base pointers) and writes
  *             grad_z, grad_logvar and grad_mu_loc [b_loc, d] (the already reduce-scattered gradient of mu, KL term included).
  * A scratch (and a published mu buffer) may be reused two exchanges later (double-buffer them), never by the very next one.
- * `mu_loc` is this rank's rows of mu (the KL term reads it).  Row-variance density only.  `fusion` as in the _ex entry points
- * (NULL = none): with `eps`, z is formed in the prologue and grad_mu_loc / grad_logvar are the gradients w.r.t. the encoder outputs.
+ * `mu_loc` is this rank's rows of mu (the KL term reads it).  Row-variance density only (the column-variance decomposition has its
+ * own peer entry points below).  `fusion` as in the _ex entry points (NULL = none): with `eps`, z is formed in the prologue and
+ * grad_mu_loc / grad_logvar are the gradients w.r.t. the encoder outputs.
  */
 /* Optional in-kernel barriers for the two exchange steps (NULL: the CALLER puts a cross-rank barrier on the stream before
  * tcelbo_klloss_forward_peer and before the TCELBO_PEER_FINISH call, as described above).  With it, the prologue kernel signals
@@ -236,6 +238,38 @@ int tcelbo_klloss_backward_peer(int phase, const float* z, int64_t ldz, const fl
                                 const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
                                 const void* const* scratch_parts, const tcelbo_fusion* fusion, const tcelbo_peer_sync* sync,
                                 void* stream);
+
+/*
+ * The decomposition (tcelbo_decomp_forward / _backward) row-sharded with the same peer-memory exchange.  The column-variance
+ * density needs the logvar of every row as well, so both column operands are exchanged:
+ *   forward : every rank publishes its [b_loc, d] rows of mu AND logvar in mapped buffers (tcelbo_peer_publish_mu_logvar: one
+ *             kernel, one forward barrier); the column-prep kernel gathers them through `mu_parts` and `lv_parts` (DEVICE tables
+ *             of n_ranks pointers, row pitch ld_part floats).  `mu_loc` / `logvar_loc` are this rank's rows (condx reads them).
+ *             The outputs and `means` are those of tcelbo_decomp_forward for this rank's rows.
+ *   backward: as tcelbo_klloss_backward_peer, with the upstream gradients of tcelbo_decomp_backward.  TCELBO_PEER_FINISH sums this
+ *             rank's rows of the mu and the logvar column sums over all ranks' scratch (in rank order) and writes grad_z,
+ *             grad_mu_loc and grad_logvar_loc [b_loc, d], already reduce-scattered, the gradients of condx and pz included.
+ * flags must contain TCELBO_VAR_COL; scratch comes from tcelbo_backward_scratch_bytes with those flags (larger than the
+ * row-variance scratch: it holds the logvar column sums too).  b_glob = n_ranks * b_loc, row_offset = rank * b_loc.  Buffer reuse,
+ * `sync` and the call order are as for the klloss peer entry points; both losses may share one set of buffers and barrier
+ * counters.  3 kernels forward (after the publish), 2 in the sweep phase, 1 in the finish.
+ */
+int tcelbo_peer_publish_mu_logvar(const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv, int b_loc, int d,
+                                  float* mu_published, float* lv_published /* [b_loc, d] dense, mapped */,
+                                  const tcelbo_peer_sync* sync, void* stream);
+int tcelbo_decomp_forward_peer(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv,
+                               const float* const* mu_parts, const float* const* lv_parts, int64_t ld_part,
+                               int b_loc, int n_ranks, int rank, int d, int64_t dataset_size, uint32_t flags, float beta,
+                               float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                               const tcelbo_peer_sync* sync, void* workspace, size_t workspace_bytes, void* stream);
+int tcelbo_decomp_backward_peer(int phase, const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu,
+                                const float* logvar_loc, int64_t ldlv, int b_loc, int n_ranks, int rank, int d,
+                                int64_t dataset_size, uint32_t flags, float beta,
+                                const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                                const float* g_means,
+                                float* grad_z, int64_t ldgz, float* grad_mu_loc, int64_t ldgmu, float* grad_logvar_loc, int64_t ldglv,
+                                const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                                const void* const* scratch_parts, const tcelbo_peer_sync* sync, void* stream);
 
 /* kl_rows[i] = -0.5 * sum_d (1 + logvar - exp(logvar) - mu^2)   (ops.py:161-163; argument order logvar, mu) */
 int tcelbo_kl_forward(const float* logvar, int64_t ldlv, const float* mu, int64_t ldmu,

@@ -131,6 +131,7 @@ struct LossFusion {            // solvers/tc.py:83-89 folded into the finalize k
 // are all mapped into this process (NVLink peer memory); in that mode `mu_all` is this rank's rows only.
 struct Peers {
     const float* const* mu_parts = nullptr; int64_t ld_part = 0;   // forward: device table of every rank's [b_loc, d] rows of mu
+    const float* const* lv_parts = nullptr;                        // forward, column variance: the same for logvar
     const void* const* scratch_parts = nullptr;                    // backward finish: device table of every rank's scratch base
     int n_ranks = 0;
     int phase = 3;                                                 // backward: 1 = sweep into scratch, 2 = finish from the peers' scratch
@@ -147,7 +148,8 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     if (lf.fz.eps && (lf.fz.ldeps < d || (lf.fz.z_out && lf.fz.ldz_out < d))) return fail(TCELBO_ERR_INVALID, "eps / z_out row pitch smaller than d");
     if (lf.fz.eps && (flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_UNSUPPORTED, "the fused reparameterize covers the row-variance density");
     if (lf.fz.expelbo && (!lf.fz.rec_rows || !lf.fz.e_rows)) return fail(TCELBO_ERR_INVALID, "expelbo needs rec_rows and e_rows");
-    if (peers.on() && (flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_UNSUPPORTED, "the peer-memory exchange covers the row-variance density");
+    if (peers.on() && (flags & TCELBO_VAR_COL) && !lf.decomp)
+        return fail(TCELBO_ERR_UNSUPPORTED, "the klloss peer entry points use the row-variance density; the column-variance decomposition has tcelbo_decomp_forward_peer");
     Plan p;
     if (!make_plan(p, b_loc, b_glob, d, flags, sm_count())) return fail(TCELBO_ERR_INVALID, "cannot plan this shape");
     if (!workspace || workspace_bytes < p.total_bytes || !aligned256(workspace))
@@ -169,7 +171,12 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     const tcelbo_fusion& fz = lf.fz;
     unsigned int* ticket = at<unsigned int>(workspace, p.off_red) + 4 * (size_t)p.n_fin_ctas;
     if (p.var_col) {
-        if ((e = launch_colvar_prep(z, ldz, mu_all, ldmu, logvar, ldlv, p, mu_pad, zs, shift, ticket, st)) != cudaSuccess) return fail_cuda(e, "colvar_prep");
+        ColPrepArgs ca;
+        ca.z = z; ca.ldz = ldz; ca.mu_all = mu_all; ca.ldmu = ldmu; ca.lv_all = logvar; ca.ldlv = ldlv;
+        ca.mu_parts = peers.on() ? peers.mu_parts : nullptr; ca.lv_parts = peers.lv_parts; ca.ld_part = peers.ld_part;
+        ca.b_loc = b_loc; ca.b_glob = b_glob; ca.d = d; ca.bl_pad = p.bl_pad; ca.bg_pad = p.bg_pad; ca.dp = p.dp;
+        ca.colpack = mu_pad; ca.zpad = zs; ca.shift = shift; ca.ticket = ticket; ca.sync = peers.sync;
+        if ((e = launch_colvar_prep(ca, st)) != cudaSuccess) return fail_cuda(e, "colvar_prep");
     } else {
         PrepArgs pa;
         pa.mu_all = mu_all; pa.ldmu = ldmu;
@@ -211,6 +218,7 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     fin.dec_loss = fin.dec_mi = fin.dec_tc = fin.dec_dimkl = fin.dec_means = nullptr;
     if (lf.decomp) {
         fin.dz = z; fin.lddz = ldz; fin.dmu = mu_all; fin.lddmu = ldmu; fin.dlv = logvar; fin.lddlv = ldlv;
+        if (peers.on()) fin.row_offset = 0;                                 // mu_all / logvar: this rank's rows only
         fin.dec_loss = lf.loss_rows; fin.dec_mi = lf.mi_rows; fin.dec_tc = lf.tc_rows; fin.dec_dimkl = lf.dimkl_rows;
         if (lf.means) { fin.dec_means = lf.means; fin.red_part = at<float>(workspace, p.off_red); fin.ticket = ticket; }
     }
@@ -234,7 +242,8 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
                          const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream,
                          const Peers& peers = Peers()) {
     if (int rc = check_common(z, mu_all, logvar, b_loc, b_glob, row_offset, d, dataset_size, flags, ldz, ldmu, ldlv, true)) return rc;
-    if (peers.on() && (flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_UNSUPPORTED, "the peer-memory exchange covers the row-variance density");
+    if (peers.on() && (flags & TCELBO_VAR_COL) && !lf.decomp)
+        return fail(TCELBO_ERR_UNSUPPORTED, "the klloss peer entry points use the row-variance density; the column-variance decomposition has tcelbo_decomp_backward_peer");
     if (lf.fz.eps && lf.fz.ldeps < d) return fail(TCELBO_ERR_INVALID, "eps row pitch smaller than d");
     if (lf.fz.g_expelbo && !lf.fz.e_rows) return fail(TCELBO_ERR_INVALID, "g_expelbo needs the e_rows the forward wrote");
     if (!(flags & TCELBO_SAVE_FOR_BACKWARD)) return fail(TCELBO_ERR_INVALID, "backward needs the workspace of a forward run with TCELBO_SAVE_FOR_BACKWARD");
@@ -437,7 +446,8 @@ int tcelbo_klloss_forward_peer(const float* z, int64_t ldz, const float* mu_loc,
 int tcelbo_peer_publish(const float* mu_loc, int64_t ldmu, int b_loc, int d, float* published, const tcelbo_peer_sync* sync, void* stream) {
     if (!mu_loc || !published || b_loc < 1 || d < 1 || ldmu < d) return fail(TCELBO_ERR_INVALID, "bad argument");
     if (sync && !sync->state) return fail(TCELBO_ERR_INVALID, "peer_sync needs the state words");
-    cudaError_t e = launch_publish(mu_loc, ldmu, b_loc, d, published, sync ? sync->state : nullptr, static_cast<cudaStream_t>(stream));
+    cudaError_t e = launch_publish(mu_loc, ldmu, nullptr, 0, b_loc, d, published, nullptr, sync ? sync->state : nullptr,
+                                   static_cast<cudaStream_t>(stream));
     return e == cudaSuccess ? TCELBO_OK : fail_cuda(e, "publish");
 }
 
@@ -460,6 +470,60 @@ int tcelbo_klloss_backward_peer(int phase, const float* z, int64_t ldz, const fl
     if (sync) peers.sync = PeerSync{sync->flag_parts, sync->state, 1, rank, n_ranks};
     return backward_impl(z, ldz, mu_loc, ldmu, logvar, ldlv, b_loc, b_loc * n_ranks, rank * b_loc, d, dataset_size, flags,
                          g_log_qz, g_log_qz_prod, lf, grad_z, ldgz, grad_mu_loc, ldgmu, grad_logvar, ldglv,
+                         workspace, workspace_bytes, scratch, scratch_bytes, stream, peers);
+}
+
+int tcelbo_peer_publish_mu_logvar(const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv, int b_loc, int d,
+                                  float* mu_published, float* lv_published, const tcelbo_peer_sync* sync, void* stream) {
+    if (!mu_loc || !logvar_loc || !mu_published || !lv_published) return fail(TCELBO_ERR_INVALID, "null pointer");
+    if (b_loc < 1 || d < 1 || ldmu < d || ldlv < d) return fail(TCELBO_ERR_INVALID, "bad b_loc / d / row pitch");
+    if (sync && !sync->state) return fail(TCELBO_ERR_INVALID, "peer_sync needs the state words");
+    cudaError_t e = launch_publish(mu_loc, ldmu, logvar_loc, ldlv, b_loc, d, mu_published, lv_published, sync ? sync->state : nullptr,
+                                   static_cast<cudaStream_t>(stream));
+    return e == cudaSuccess ? TCELBO_OK : fail_cuda(e, "publish");
+}
+
+int tcelbo_decomp_forward_peer(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv,
+                               const float* const* mu_parts, const float* const* lv_parts, int64_t ld_part,
+                               int b_loc, int n_ranks, int rank, int d, int64_t dataset_size, uint32_t flags, float beta,
+                               float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                               const tcelbo_peer_sync* sync, void* workspace, size_t workspace_bytes, void* stream) {
+    if (int rc = check_decomp(flags, z, mu_loc, logvar_loc)) return rc;
+    if (!loss_rows || !mi_rows || !tc_rows || !dimkl_rows) return fail(TCELBO_ERR_INVALID, "null output pointer");
+    if (!mu_parts || !lv_parts) return fail(TCELBO_ERR_INVALID, "null pointer table");
+    if (sync && (!sync->flag_parts || !sync->state)) return fail(TCELBO_ERR_INVALID, "peer_sync needs the flag table and the state words");
+    if (n_ranks < 1 || rank < 0 || rank >= n_ranks || ld_part < d) return fail(TCELBO_ERR_INVALID, "bad rank / n_ranks / ld_part");
+    if ((int64_t)b_loc * n_ranks > INT32_MAX) return fail(TCELBO_ERR_INVALID, "global batch too large");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.loss_rows = loss_rows; lf.mi_rows = mi_rows; lf.tc_rows = tc_rows; lf.dimkl_rows = dimkl_rows; lf.means = means;
+    Peers peers; peers.mu_parts = mu_parts; peers.lv_parts = lv_parts; peers.ld_part = ld_part; peers.n_ranks = n_ranks;
+    if (sync) peers.sync = PeerSync{sync->flag_parts, sync->state, 0, rank, n_ranks};
+    return forward_impl(z, ldz, mu_loc, ldmu, logvar_loc, ldlv, b_loc, b_loc * n_ranks, rank * b_loc, d, dataset_size, flags,
+                        nullptr, nullptr, lf, workspace, workspace_bytes, stream, peers);
+}
+
+int tcelbo_decomp_backward_peer(int phase, const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu,
+                                const float* logvar_loc, int64_t ldlv, int b_loc, int n_ranks, int rank, int d,
+                                int64_t dataset_size, uint32_t flags, float beta,
+                                const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                                const float* g_means,
+                                float* grad_z, int64_t ldgz, float* grad_mu_loc, int64_t ldgmu, float* grad_logvar_loc, int64_t ldglv,
+                                const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                                const void* const* scratch_parts, const tcelbo_peer_sync* sync, void* stream) {
+    if (int rc = check_decomp(flags, z, mu_loc, logvar_loc)) return rc;
+    if (!grad_z || !grad_mu_loc || !grad_logvar_loc) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
+    if (!g_loss_rows && !g_mi_rows && !g_tc_rows && !g_dimkl_rows && !g_means) return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
+    if (sync && (!sync->flag_parts || !sync->state)) return fail(TCELBO_ERR_INVALID, "peer_sync needs the flag table and the state words");
+    if (phase != TCELBO_PEER_SWEEP && phase != TCELBO_PEER_FINISH) return fail(TCELBO_ERR_INVALID, "phase must be TCELBO_PEER_SWEEP or TCELBO_PEER_FINISH");
+    if (n_ranks < 1 || rank < 0 || rank >= n_ranks) return fail(TCELBO_ERR_INVALID, "bad rank / n_ranks");
+    if (phase == TCELBO_PEER_FINISH && !scratch_parts) return fail(TCELBO_ERR_INVALID, "null scratch table");
+    if ((int64_t)b_loc * n_ranks > INT32_MAX) return fail(TCELBO_ERR_INVALID, "global batch too large");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.g_loss = g_loss_rows; lf.g_mi = g_mi_rows; lf.g_tc = g_tc_rows; lf.g_dimkl = g_dimkl_rows; lf.g_means = g_means;
+    Peers peers; peers.scratch_parts = scratch_parts; peers.n_ranks = n_ranks; peers.phase = phase;
+    if (sync) peers.sync = PeerSync{sync->flag_parts, sync->state, 1, rank, n_ranks};
+    return backward_impl(z, ldz, mu_loc, ldmu, logvar_loc, ldlv, b_loc, b_loc * n_ranks, rank * b_loc, d, dataset_size, flags,
+                         nullptr, nullptr, lf, grad_z, ldgz, grad_mu_loc, ldgmu, grad_logvar_loc, ldglv,
                          workspace, workspace_bytes, scratch, scratch_bytes, stream, peers);
 }
 

@@ -21,37 +21,66 @@ __device__ __forceinline__ void red_add_v4_cv(float* addr, float a, float b, flo
     asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" :: "l"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
+// (sj, nmus, c2) of one column element, shared by the plain and the peer-gather prologue so that both pack the same bits
+__device__ __forceinline__ void colpack_of(float m, float lv, float& sj, float& nmus, float& c2) {
+    const float iv = expf(-lv);
+    sj = sqrtf(0.5f * kLog2e * iv);
+    c2 = -0.5f * (lv + kLog2Pi) * kLog2e;
+    // logvar < -88.7: exp(-logvar) is +inf in fp32, so ops.py:27-29 yields -inf -> -50 for every z != mu.  Keep that
+    // behaviour with finite operands (dl^2 overflows to +inf and the clamp takes over) instead of inf - inf = NaN,
+    // and keep the unshifted sum S = sum_j rho 2^t finite: c2 stays <= 63 for every column that can be unclamped.
+    if (isinf(iv)) { sj = 1.0e19f; c2 = 0.0f; }
+    nmus = -(m * sj);
+}
+
 // column operands: colpack[j][0..2][dp] = (sj, nmus, c2); rows: zpad[i][dp] (zero padded), shift[i][dp] = 0; zeroes the
-// ticket of the finalize kernel's batch means (the workspace may be fresh, uninitialised memory)
-__global__ void colvar_prep_kernel(const float* __restrict__ z, int64_t ldz, const float* __restrict__ mu_all, int64_t ldmu,
-                                   const float* __restrict__ lv_all, int64_t ldlv, int b_loc, int b_glob, int d,
-                                   int bl_pad, int bg_pad, int dp,
-                                   float* __restrict__ colpack, float* __restrict__ zpad, float* __restrict__ shift,
-                                   unsigned int* __restrict__ ticket) {
-    const int64_t n_col = (int64_t)bg_pad * dp, n_row = (int64_t)bl_pad * dp;
-    if (blockIdx.x == 0 && threadIdx.x == 0) *ticket = 0u;
-    for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n_col + n_row; idx += (int64_t)gridDim.x * blockDim.x) {
-        if (idx < n_col) {
-            const int j = (int)(idx / dp), dd = (int)(idx % dp);
-            float sj = 0.f, nmus = 0.f, c2 = 0.f;
-            if (j < b_glob && dd < d) {
-                const float lv = lv_all[(int64_t)j * ldlv + dd], m = mu_all[(int64_t)j * ldmu + dd];
-                const float iv = expf(-lv);
-                sj = sqrtf(0.5f * kLog2e * iv);
-                c2 = -0.5f * (lv + kLog2Pi) * kLog2e;
-                // logvar < -88.7: exp(-logvar) is +inf in fp32, so ops.py:27-29 yields -inf -> -50 for every z != mu.  Keep that
-                // behaviour with finite operands (dl^2 overflows to +inf and the clamp takes over) instead of inf - inf = NaN,
-                // and keep the unshifted sum S = sum_j rho 2^t finite: c2 stays <= 63 for every column that can be unclamped.
-                if (isinf(iv)) { sj = 1.0e19f; c2 = 0.0f; }
-                nmus = -(m * sj);
+// ticket of the finalize kernel's batch means (the workspace may be fresh, uninitialised memory).  kParts: the columns live in
+// b_loc-row blocks of different allocations (one per rank, peer-mapped); the rows (local data) are written first, then the
+// in-kernel barrier waits for every rank's publish, then the columns are gathered with volatile loads, V (1 or 4) dims per thread.
+template <bool kParts, int V>
+__global__ void colvar_prep_kernel(const ColPrepArgs a) {
+    const int64_t n_row = (int64_t)a.bl_pad * a.dp;
+    const int64_t t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
+    if (blockIdx.x == 0 && threadIdx.x == 0) *a.ticket = 0u;
+    for (int64_t k = t0; k < n_row; k += stride) {
+        const int i = (int)(k / a.dp), dd = (int)(k % a.dp);
+        a.zpad[k] = (i < a.b_loc && dd < a.d) ? a.z[(int64_t)i * a.ldz + dd] : 0.0f;
+        a.shift[k] = 0.0f;
+    }
+    if (kParts && a.sync.on()) peer_barrier(a.sync);
+    const int dpv = a.dp / V;
+    const int64_t n_col = (int64_t)a.bg_pad * dpv;
+    for (int64_t idx = t0; idx < n_col; idx += stride) {
+        const int j = (int)(idx / dpv), dd = V * (int)(idx % dpv);
+        float m[V], l[V];
+        if (kParts && j < a.b_glob && dd < a.d) {
+            const int part = j / a.b_loc;
+            const int64_t o = (int64_t)(j - part * a.b_loc) * a.ld_part + dd;
+            if (V == 4) {                                        // d % 4 == 0: dd < d covers all four
+                const float4 mv = ld_volatile_v4(a.mu_parts[part] + o), lv = ld_volatile_v4(a.lv_parts[part] + o);
+                m[0] = mv.x; m[1] = mv.y; m[2] = mv.z; m[3] = mv.w;
+                l[0] = lv.x; l[1] = lv.y; l[2] = lv.z; l[3] = lv.w;
+            } else {
+                m[0] = *static_cast<const volatile float*>(a.mu_parts[part] + o);
+                l[0] = *static_cast<const volatile float*>(a.lv_parts[part] + o);
             }
-            float* o = colpack + (size_t)j * 3 * dp + dd;
-            o[0] = sj; o[dp] = nmus; o[2 * dp] = c2;
+        } else if (!kParts && j < a.b_glob && dd < a.d) {
+#pragma unroll
+            for (int e = 0; e < V; ++e) { m[e] = a.mu_all[(int64_t)j * a.ldmu + dd + e]; l[e] = a.lv_all[(int64_t)j * a.ldlv + dd + e]; }
+        }
+        float sj[V], nmus[V], c2[V];
+#pragma unroll
+        for (int e = 0; e < V; ++e) {
+            sj[e] = 0.f; nmus[e] = 0.f; c2[e] = 0.f;
+            if (j < a.b_glob && dd + e < a.d) colpack_of(m[e], l[e], sj[e], nmus[e], c2[e]);
+        }
+        float* o = a.colpack + (size_t)j * 3 * a.dp + dd;
+        if (V == 4) {
+            *reinterpret_cast<float4*>(o) = make_float4(sj[0], sj[1], sj[2], sj[3]);
+            *reinterpret_cast<float4*>(o + a.dp) = make_float4(nmus[0], nmus[1], nmus[2], nmus[3]);
+            *reinterpret_cast<float4*>(o + 2 * a.dp) = make_float4(c2[0], c2[1], c2[2], c2[3]);
         } else {
-            const int64_t k = idx - n_col;
-            const int i = (int)(k / dp), dd = (int)(k % dp);
-            zpad[k] = (i < b_loc && dd < d) ? z[(int64_t)i * ldz + dd] : 0.0f;
-            shift[k] = 0.0f;
+            o[0] = sj[0]; o[a.dp] = nmus[0]; o[2 * a.dp] = c2[0];
         }
     }
 }
@@ -383,9 +412,16 @@ tc_bwd_colvar_kernel(const BwdFusedArgs a) {
 // rowdensity_bwd_kernel: condx_i = sum_d lp(z_id; mu_rd, lv_rd) to grad_z[i] and to row r = row_offset + i of grad_mu / grad_lv
 // (the thread that owns (r, d) of the column part adds them, so no two threads write one element), pz_i = sum_d lp(z_id; 0, 0)
 // to grad_z[i].
+// Peer exchange (a.scratch_parts != nullptr): after the barrier that says every rank's sweep is done, the column part covers this
+// rank's rows only; their mu and logvar column sums are added up over all ranks' scratch in rank order (the reduce-scatter is this
+// kernel's load phase), and mu_all / lv / grad_mu / grad_lv are this rank's rows at local indices.
 __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __restrict__ colpack, const float* __restrict__ Glv) {
+    const bool peer = a.scratch_parts != nullptr;
+    if (peer && a.sync.on()) peer_barrier(a.sync);
     const int64_t n_row = (int64_t)a.b_loc * a.d;
-    const int64_t n_col = (int64_t)a.b_glob * a.d;
+    const int64_t n_col = (int64_t)(peer ? a.b_loc : a.b_glob) * a.d;
+    const int64_t mrow0 = peer ? 0 : a.row_offset;                    // row of mu_all / lv that holds local row 0
+    const size_t glv_off = a.g_off + (size_t)a.bg_pad * a.dp * sizeof(float);    // Glv follows Gpart in every rank's scratch
     for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n_row + n_col; idx += (int64_t)gridDim.x * blockDim.x) {
         if (idx < n_row) {
             const int i = (int)(idx / a.d), dd = (int)(idx % a.d);
@@ -394,7 +430,7 @@ __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __re
             for (int s = 0; s < a.n_js; ++s) sa += a.Apart[(size_t)s * a.bl_pad * a.dp + o];
             float gz = -kTwoLn2 * sa;
             if (a.gc != nullptr) {
-                const int64_t r = (int64_t)a.row_offset + i;
+                const int64_t r = mrow0 + i;
                 const float x = a.z[(int64_t)i * a.ldz + dd];
                 float t, iv, t0, iv0;
                 const float lp = lp_unfloored(x, a.mu_all[r * a.ldmu + dd], a.lv[r * a.ldlv + dd], t, iv);
@@ -405,21 +441,41 @@ __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __re
             a.grad_z[(int64_t)i * a.ldgz + dd] = gz;
         } else {
             const int64_t k = idx - n_row;
-            const int j = (int)(k / a.d), dd = (int)(k % a.d);
+            const int j = (int)(k / a.d) + (peer ? a.row_offset : 0), dd = (int)(k % a.d);
             const size_t o = (size_t)j * a.dp + dd;
             const float sj = colpack[(size_t)j * 3 * a.dp + dd];
-            float gmu = kTwoLn2 * sj * a.Gpart[o], glv = Glv[o];
+            float gm, gl;
+            if (peer) {
+                gm = 0.0f; gl = 0.0f;
+                for (int p0 = 0; p0 < a.n_ranks; p0 += 4) {
+                    float vm[4], vl[4];
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const char* base = static_cast<const char*>(a.scratch_parts[p0 + q < a.n_ranks ? p0 + q : p0]);
+                        vm[q] = *reinterpret_cast<const volatile float*>(base + a.g_off + o * sizeof(float));
+                        vl[q] = *reinterpret_cast<const volatile float*>(base + glv_off + o * sizeof(float));
+                    }
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        if (p0 + q < a.n_ranks) { gm += vm[q]; gl += vl[q]; }
+                    }
+                }
+            } else {
+                gm = a.Gpart[o]; gl = Glv[o];
+            }
+            float gmu = kTwoLn2 * sj * gm, glv = gl;
             const int i = j - a.row_offset;
             if (a.gc != nullptr && i >= 0 && i < a.b_loc) {
-                const float m = a.mu_all[(int64_t)j * a.ldmu + dd], l = a.lv[(int64_t)j * a.ldlv + dd];
+                const float m = a.mu_all[(mrow0 + i) * a.ldmu + dd], l = a.lv[(mrow0 + i) * a.ldlv + dd];
                 float t, iv;
                 const float lp = lp_unfloored(a.z[(int64_t)i * a.ldz + dd], m, l, t, iv);
                 const float gc = lp_passes_grad(lp) ? a.gc[i] : 0.0f;
                 gmu += gc * t * iv;
                 glv += gc * 0.5f * (t * t * iv - 1.0f);
             }
-            a.grad_mu[(int64_t)j * a.ldgmu + dd] = gmu;
-            a.grad_lv[(int64_t)j * a.ldglv + dd] = glv;
+            const int64_t grow = peer ? i : j;                        // grad_mu / grad_lv: this rank's rows only in the peer mode
+            a.grad_mu[grow * a.ldgmu + dd] = gmu;
+            a.grad_lv[grow * a.ldglv + dd] = glv;
         }
     }
 }
@@ -427,13 +483,15 @@ __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __re
 // ------------------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------------------
-cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* lv_all, int64_t ldlv,
-                               const Plan& p, float* colpack, float* zpad, float* shift, unsigned int* ticket, cudaStream_t st) {
-    const int64_t n = (int64_t)(p.bg_pad + p.bl_pad) * p.dp;
+cudaError_t launch_colvar_prep(const ColPrepArgs& a, cudaStream_t st) {
+    // the ranks' published buffers are dense, 16-byte aligned allocations: 16-byte gathers when the row pitch keeps them aligned
+    const bool vec = a.mu_parts != nullptr && a.d % 4 == 0 && a.ld_part % 4 == 0;
+    const int64_t n = (int64_t)(a.bg_pad + a.bl_pad) * a.dp;
     int64_t g = (n + 255) / 256; if (g > 148 * 16) g = 148 * 16;
     LaunchScope scope(kKernNone, st);
-    colvar_prep_kernel<<<(int)g, 256, 0, st>>>(z, ldz, mu_all, ldmu, lv_all, ldlv, p.b_loc, p.b_glob, p.d, p.bl_pad, p.bg_pad, p.dp,
-                                                colpack, zpad, shift, ticket);
+    if (a.mu_parts == nullptr) colvar_prep_kernel<false, 1><<<(int)g, 256, 0, st>>>(a);
+    else if (vec)              colvar_prep_kernel<true, 4><<<(int)g, 256, 0, st>>>(a);
+    else                       colvar_prep_kernel<true, 1><<<(int)g, 256, 0, st>>>(a);
     return cudaGetLastError();
 }
 
@@ -483,7 +541,7 @@ cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, cudaStream_t
 }
 
 cudaError_t launch_bwd_colvar_finalize(const Plan& p, const BwdFinArgs& a, const float* colpack, const float* Glv, cudaStream_t st) {
-    const int64_t n = (int64_t)p.b_loc * p.d + (int64_t)p.b_glob * p.d;
+    const int64_t n = (int64_t)p.b_loc * p.d + (int64_t)(a.scratch_parts != nullptr ? p.b_loc : p.b_glob) * p.d;
     int64_t g = (n + 255) / 256; if (g > 148 * 16) g = 148 * 16; if (g < 1) g = 1;
     LaunchScope scope(kKernNone, st);
     bwd_colvar_finalize_kernel<<<(int)g, 256, 0, st>>>(a, colpack, Glv);

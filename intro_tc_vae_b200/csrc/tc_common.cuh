@@ -134,6 +134,12 @@ __device__ __forceinline__ void weight_of(const Weights& w, int i_glob, int j, f
     if (j >= w.b_glob) { rho = 0.0f; l2rho = -INFINITY; }
 }
 
+__device__ __forceinline__ float4 ld_volatile_v4(const float* p) {          // peer-mapped memory: no L1 / nc path
+    float4 v;
+    asm volatile("ld.volatile.global.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
+    return v;
+}
+
 // ---- cross-rank barrier inside a kernel, over peer-mapped flags (one process per GPU, NVLink) --------------------
 // Rank r owns a flag array of n_channels * n_ranks words in memory every rank has mapped.  Barrier number e of a channel:
 // every rank stores e into slot [channel][its rank] of EVERY rank's array (release, system scope) and then waits until all

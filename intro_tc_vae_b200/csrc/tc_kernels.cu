@@ -19,14 +19,18 @@ namespace tcelbo {
 // =====================================================================================================
 // Prologues: pad/copy the column operand, derive the per-(i,d) constants
 // =====================================================================================================
-// Peer exchange, forward: copy this rank's rows of mu into its peer-mapped buffer and open the next forward barrier
-// (the prologue kernel that follows on the stream signals and waits on that number, tc_common.cuh: PeerSync).
-__global__ void publish_kernel(const float* __restrict__ src, int64_t ld, int b_loc, int d, float* __restrict__ dst, unsigned int* epoch) {
+// Peer exchange, forward: copy this rank's rows of mu (and, for the column-variance decomposition, of logvar: src2 -> dst2) into
+// its peer-mapped buffers and open the next forward barrier (the prologue kernel that follows on the stream signals and waits on
+// that number, tc_common.cuh: PeerSync).
+__global__ void publish_kernel(const float* __restrict__ src, int64_t ld, const float* __restrict__ src2, int64_t ld2, int b_loc, int d,
+                               float* __restrict__ dst, float* __restrict__ dst2, unsigned int* epoch) {
     pdl_trigger(); pdl_wait();                               // programmatic dependent launch, tc_common.cuh
     if (blockIdx.x == 0 && threadIdx.x == 0 && epoch != nullptr) atomicAdd(epoch, 1u);
     const int64_t n = (int64_t)b_loc * d;
-    for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (int64_t)gridDim.x * blockDim.x)
+    for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (int64_t)gridDim.x * blockDim.x) {
         dst[idx] = src[(idx / d) * ld + idx % d];
+        if (dst2 != nullptr) dst2[idx] = src2[(idx / d) * ld2 + idx % d];
+    }
 }
 
 template <bool kParts>
@@ -77,12 +81,6 @@ __global__ void prep_scalar_kernel(const PrepArgs a) {
         }
         a.mu_pad[idx] = v;
     }
-}
-
-__device__ __forceinline__ float4 ld_volatile_v4(const float* p) {          // peer-mapped memory: no L1 / nc path
-    float4 v;
-    asm volatile("ld.volatile.global.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
-    return v;
 }
 
 // The same prologue with 16-byte accesses: launched when d % 4 == 0 and every caller-side pitch / pointer is 16-byte aligned
@@ -566,9 +564,11 @@ static cudaError_t launch_fwd_t(const Plan& p, const FwdArgs& a, cudaStream_t st
     return launch_pdl(kern, dim3(p.seg_fwd.n_ctas), dim3(NWF * 32), smem, st, a);
 }
 
-cudaError_t launch_publish(const float* src, int64_t ld, int b_loc, int d, float* dst, unsigned int* epoch, cudaStream_t st) {
+cudaError_t launch_publish(const float* src, int64_t ld, const float* src2, int64_t ld2, int b_loc, int d, float* dst, float* dst2,
+                           unsigned int* epoch, cudaStream_t st) {
     LaunchScope scope(kKernNone, st);
-    return launch_pdl(publish_kernel, dim3(grid_for((int64_t)b_loc * d, 256, 148 * 4)), dim3(256), 0, st, src, ld, b_loc, d, dst, epoch);
+    return launch_pdl(publish_kernel, dim3(grid_for((int64_t)b_loc * d, 256, 148 * 4)), dim3(256), 0, st, src, ld, src2, ld2, b_loc, d,
+                      dst, dst2, epoch);
 }
 
 static inline bool aligned16(const void* p, int64_t ld) { return p == nullptr || ((reinterpret_cast<uintptr_t>(p) & 15u) == 0 && ld % 4 == 0); }

@@ -38,7 +38,8 @@ struct FinArgs {
     //   mi_i = condx_i - log_qz_i, tc_i = log_qz_i - log_qz_prod_i, dimkl_i = log_qz_prod_i - pz_i, loss_i = mi_i + beta*tc_i + dimkl_i
     //   dec_means[0..3] = the batch means of loss, mi, tc, dimkl (nullptr: none)
     const float* dz; int64_t lddz; const float* dmu; int64_t lddmu; const float* dlv; int64_t lddlv;   // z rows; mu / logvar [b_glob]
-    int row_offset;
+    int row_offset;                                              // row of dmu / dlv holding local row 0 (0 with the peer exchange,
+                                                                 // where dmu / dlv are this rank's rows only)
     float* dec_loss; float* dec_mi; float* dec_tc; float* dec_dimkl; float* dec_means;
     float* red_part; unsigned int* ticket;                       // [4][gridDim.x] partial sums, arrival counter (zeroed by the prologue)
 };
@@ -54,6 +55,16 @@ struct PrepArgs {
     int b_loc, b_glob, d, bl_pad, bg_pad, dp;
     float* mu_pad; float* zs; float* ns; float* qmax; float* shift; float* vr;
     unsigned int* ticket;
+    PeerSync sync;                                               // peer exchange: barrier between the ranks' publish and this gather
+};
+
+// Column-variance prologue (tc_colvar.cu): packs (sj, nmus, c2) of every column, zero-pads the local rows of z.
+struct ColPrepArgs {
+    const float* z; int64_t ldz;                                 // this rank's rows
+    const float* mu_all; int64_t ldmu; const float* lv_all; int64_t ldlv;        // [b_glob][d] columns (ignored with parts)
+    const float* const* mu_parts; const float* const* lv_parts; int64_t ld_part;  // peer exchange: one [b_loc][d] block per rank
+    int b_loc, b_glob, d, bl_pad, bg_pad, dp;
+    float* colpack; float* zpad; float* shift; unsigned int* ticket;
     PeerSync sync;                                               // peer exchange: barrier between the ranks' publish and this gather
 };
 
@@ -86,12 +97,16 @@ struct BwdFinArgs {
     const float* eps; int64_t ldeps;
     PeerSync sync;                                               // peer exchange: barrier between the ranks' sweeps and this reduce
     // column-variance decomposition (BwdUpstream::gpz): the row-local gradients of condx_i (coefficient gc_i) and pz_i (gpz_i),
-    // masked where lp < -50, on grad_z[i] and on row r = row_offset + i of grad_mu / grad_lv (nullptr: off)
+    // masked where lp < -50, on grad_z[i] and on row r = row_offset + i of grad_mu / grad_lv (nullptr: off).  With scratch_parts
+    // (peer exchange) the column part covers rows [row_offset, row_offset + b_loc) only, sums the mu and logvar column sums of
+    // every rank's scratch, and mu_all / lv / grad_mu / grad_lv are this rank's rows at local indices.
     const float* gc; const float* gpz; const float* z; int64_t ldz;
 };
 
 cudaError_t launch_prep(const PrepArgs& a, cudaStream_t st);
-cudaError_t launch_publish(const float* src, int64_t ld, int b_loc, int d, float* dst, unsigned int* epoch, cudaStream_t st);
+// src2 / dst2 (may be nullptr): a second [b_loc][d] block copied by the same kernel (logvar of the decomposition)
+cudaError_t launch_publish(const float* src, int64_t ld, const float* src2, int64_t ld2, int b_loc, int d, float* dst, float* dst2,
+                           unsigned int* epoch, cudaStream_t st);
 cudaError_t launch_fwd(const Plan& p, const FwdArgs& a, cudaStream_t st);
 cudaError_t launch_fwd_finalize(const Plan& p, const FinArgs& a, cudaStream_t st);
 // Upstream gradients of the backward prologue.  Per row i (any pointer may be null):
@@ -116,8 +131,7 @@ cudaError_t launch_bwd_prep(const Plan& p, const BwdUpstream& u, const float* S,
                             float* zero, size_t zero_n, cudaStream_t st);
 cudaError_t launch_bwd_fused(const Plan& p, const BwdFusedArgs& a, cudaStream_t st);
 // column-variance ("full" path) variant, tc_colvar.cu
-cudaError_t launch_colvar_prep(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* lv_all, int64_t ldlv,
-                               const Plan& p, float* colpack, float* zpad, float* shift, unsigned int* ticket, cudaStream_t st);
+cudaError_t launch_colvar_prep(const ColPrepArgs& a, cudaStream_t st);
 cudaError_t launch_fwd_colvar(const Plan& p, const FwdArgs& a, cudaStream_t st);
 cudaError_t launch_bwd_colvar(const Plan& p, const BwdFusedArgs& a, cudaStream_t st);
 cudaError_t launch_bwd_colvar_finalize(const Plan& p, const BwdFinArgs& a, const float* colpack, const float* Glv, cudaStream_t st);

@@ -392,7 +392,7 @@ def _decomp_autograd_backward(ctx, g_loss, g_mi, g_tc, g_dimkl, g_means, _g_ws):
 _decomp_forward.register_autograd(_decomp_autograd_backward, setup_context=_decomp_setup_context)
 
 
-def _decomp(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str, group):
+def _decomp(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str, group, exchange):
     """Shared front end of :func:`tc_decomp_loss_terms` / :func:`tc_decomp_loss_mean` -> the op's 5 tensor outputs."""
     for name, t in (("z", z), ("mu", mu), ("logvar", logvar)):
         _check(name, t)
@@ -404,6 +404,11 @@ def _decomp(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: floa
     if torch.is_grad_enabled() and (z.requires_grad or mu.requires_grad or logvar.requires_grad):
         flags |= _lib.SAVE_FOR_BACKWARD
     row_offset, mu_all, lv_all = 0, mu, logvar
+    if exchange is not None:
+        from .peer import tc_decomp_loss_terms_peer
+        if estimator == "mss" and exchange.world * z.shape[0] == 1:
+            raise ZeroDivisionError("float division by zero")
+        return tc_decomp_loss_terms_peer(z, mu, logvar, dataset_size, beta, flags, exchange)
     if group is not None:
         import torch.distributed as dist
         if dist.get_world_size(group) > 1:
@@ -416,7 +421,7 @@ def _decomp(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: floa
 
 
 def tc_decomp_loss_terms(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str = "mss",
-                         group=None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                         group=None, exchange=None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """One fused evaluation of ``TCSovler._compute_kl_loss_full`` (solvers/tc.py:91-144), the beta-TCVAE loss, per sample:
 
         mi_i = log q(z_i|x_i) - log q(z_i),  tc_i = log q(z_i) - sum_d log q(z_id),  dimkl_i = sum_d log q(z_id) - log p(z_i)
@@ -426,17 +431,19 @@ def tc_decomp_loss_terms(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: in
     :func:`row_log_density`).  Returns ``(loss [B], mi [B], tc [B], dimkl [B])``.  The two row densities and the combine are
     folded into the TC kernels' finalize steps, forward and backward: three kernels each way.  ``group`` row-shards the batch
     exactly as :func:`tc_terms` with ``var_of="col"`` does (``mu`` and ``logvar`` all-gathered, column gradients
-    reduce-scattered); outputs cover the local rows.
+    reduce-scattered); outputs cover the local rows.  ``exchange`` (a :class:`intro_tc_vae_b200.peer.PeerExchange`) row-shards
+    it over the exchange's group with both exchange steps, for ``mu`` and ``logvar``, done by the library's kernels over NVLink
+    peer memory instead.
     """
-    return _decomp(z, mu, logvar, dataset_size, beta, estimator, group)[:4]
+    return _decomp(z, mu, logvar, dataset_size, beta, estimator, group, exchange)[:4]
 
 
 def tc_decomp_loss_mean(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, beta: float, estimator: str = "mss",
-                        group=None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+                        group=None, exchange=None) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """``reduce="mean"`` form of :func:`tc_decomp_loss_terms`: 0-d ``(mean loss, mean mi, mean tc, mean dimkl)``.  The means
     come out of the finalize kernel (deterministic last-CTA reduction) and their gradients enter the backward prologue as
-    device scalars.  Row-sharded calls return the means over the local rows."""
-    return tuple(_decomp(z, mu, logvar, dataset_size, beta, estimator, group)[4].unbind(0))
+    device scalars.  Row-sharded calls (``group`` or ``exchange``) return the means over the local rows."""
+    return tuple(_decomp(z, mu, logvar, dataset_size, beta, estimator, group, exchange)[4].unbind(0))
 
 
 def tc_terms(z: Tensor, mu: Tensor, logvar: Tensor, dataset_size: int, estimator: str = "mss",

@@ -31,10 +31,25 @@ def _singleton_writer() -> _WriterView:
     return _WriterView(_utils.SingletonWriter())
 
 
+def _sharding_of(solver, z: Tensor):
+    """(process_group, peer_exchange) for a batch: the exchange only serves the shard shape it was built for; any other shape
+    (e.g. a ragged last batch) falls back on the process group, and without one the call raises rather than silently run the
+    estimator unsharded on the local rows."""
+    group = getattr(solver, "process_group", None)
+    exch = getattr(solver, "peer_exchange", None)
+    if exch is not None and tuple(z.shape) != (exch.b_loc, exch.d):
+        if group is None:
+            raise RuntimeError(
+                f"tcelbo: batch shape {tuple(z.shape)} does not match the peer exchange ({exch.b_loc}, {exch.d}) and no "
+                "process_group is set to fall back on: the estimator would silently run unsharded on the local rows")
+        exch = None                                                  # NCCL path
+    return group, exch
+
+
 class TCLossMixin:
     process_group = None          # set to a torch.distributed group to row-shard the estimator (SURVEY.md 8e)
     peer_exchange = None          # optionally a peer.PeerExchange for that group and shard shape: the all-gather /
-                                  # reduce-scatter of the simple path then run inside the library's kernels over NVLink
+                                  # reduce-scatter of both losses then run inside the library's kernels over NVLink
 
     def compute_kl_loss(self, z: Optional[Tensor], mu: Tensor, logvar: Tensor, reduce: str = "mean",
                         beta: float = None, write: bool = False) -> Tensor:
@@ -47,14 +62,7 @@ class TCLossMixin:
         if beta is None:
             beta = self.beta_kl
         dataset_size = len(self.dataset)
-        group = getattr(self, "process_group", None)
-        exch = getattr(self, "peer_exchange", None)
-        if exch is not None and tuple(z.shape) != (exch.b_loc, exch.d):
-            if group is None:
-                raise RuntimeError(
-                    f"tcelbo: batch shape {tuple(z.shape)} does not match the peer exchange ({exch.b_loc}, {exch.d}) and no "
-                    "process_group is set to fall back on: the estimator would silently run unsharded on the local rows")
-            exch = None                                              # e.g. a ragged last batch: NCCL path
+        group, exch = _sharding_of(self, z)
         if reduce == "mean":                                         # mean((b-1)*tc + kl) == (b-1)*mean(tc) + mean(kl)
             loss, kl = ops.kl_tc_loss_mean(z, mu, logvar, dataset_size, beta, "mss", group, exch)
         else:
@@ -74,17 +82,17 @@ class TCLossMixin:
         if beta is None:
             beta = self.beta_kl
         dataset_size = len(self.dataset)
-        group = getattr(self, "process_group", None)
+        group, exch = _sharding_of(self, z)
         sw = _singleton_writer()
         if reduce == "mean":
-            loss, mi_loss, tc_loss, kl_loss = ops.tc_decomp_loss_mean(z, mu, logvar, dataset_size, beta, "mss", group)
+            loss, mi_loss, tc_loss, kl_loss = ops.tc_decomp_loss_mean(z, mu, logvar, dataset_size, beta, "mss", group, exch)
             if sw.writer:
                 sw.writer.add_scalars(
                     "tc_decomp",
                     {"mi": mi_loss.data.item(), "tc": tc_loss.data.item(), "kl": kl_loss.data.item()},
                     global_step=sw.cur_iter)
         else:
-            loss, mi_loss, tc_loss, kl_loss = ops.tc_decomp_loss_terms(z, mu, logvar, dataset_size, beta, "mss", group)
+            loss, mi_loss, tc_loss, kl_loss = ops.tc_decomp_loss_terms(z, mu, logvar, dataset_size, beta, "mss", group, exch)
         if write:
             self.write_scalar(sw.cur_iter, "kl_loss_unscaled", mi_loss + tc_loss + kl_loss)
         return loss

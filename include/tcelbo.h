@@ -172,8 +172,7 @@ int tcelbo_klloss_backward_ex(const float* z, int64_t ldz, const float* mu_all, 
  * kernel.  The backward takes dLoss/d of the four per-row outputs and g_means (DEVICE float[4], dLoss/d of the four means); each
  * may be NULL (= zero) as long as one is given.  It adds the gradients of condx and pz to grad_z, to grad_logvar [b_glob, D] and to
  * rows [row_offset, row_offset + b_loc) of grad_mu_all, so no row-density or elementwise kernels are launched: 3 kernels forward,
- * 3 backward.  The row-sharded peer-memory form is tcelbo_decomp_forward_peer / _backward_peer below; the fused reparameterize
- * (tcelbo_fusion.eps) covers the row-variance density only.
+ * 3 backward.  The row-sharded peer-memory form is tcelbo_decomp_forward_peer / _backward_peer below.
  */
 int tcelbo_decomp_forward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
                           int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
@@ -185,6 +184,31 @@ int tcelbo_decomp_backward(const float* z, int64_t ldz, const float* mu_all, int
                            const float* g_means,
                            float* grad_z, int64_t ldgz, float* grad_mu_all, int64_t ldgmu, float* grad_logvar, int64_t ldglv,
                            const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream);
+
+/*
+ * tcelbo_decomp_forward / _backward with the fusions of tcelbo_fusion, so that a training step of the decomposition is 3 kernels
+ * each way with nothing around them (the plain entry points are these with fusion = NULL):
+ *   forward   eps, ldeps, z_out, ldz_out: the fused reparameterize; z = mu + eps * exp(logvar / 2) of this rank's rows (rows
+ *             [row_offset, row_offset + b_loc) of mu_all / logvar) is formed in the prologue with the bits of
+ *             tcelbo_reparam_forward, z is not read (pass NULL) and z_out, if given, receives it;
+ *             rec_rows, scale, expelbo, e_rows: the soft-intro exp-ELBO term with kl_i = loss_rows[i], reduced as a fifth batch mean
+ *             next to the four of `means`;
+ *   backward  eps, ldeps: the same eps; grad_logvar and rows [row_offset, row_offset + b_loc) of grad_mu_all are then the
+ *             gradients w.r.t. the ENCODER outputs (grad_z still receives dLoss/dz); scale, e_rows, g_expelbo, g_rec_rows as above
+ *             (g_expelbo counts as an upstream gradient).
+ * The batch means of the decomposition are `means` / `g_means`: fusion.loss_mean, kl_mean, g_loss_mean and g_kl_mean must be NULL
+ * (TCELBO_ERR_INVALID otherwise).  Every argument is checked before any CUDA call.
+ */
+int tcelbo_decomp_forward_ex(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                             int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                             float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                             const tcelbo_fusion* fusion, void* workspace, size_t workspace_bytes, void* stream);
+int tcelbo_decomp_backward_ex(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                              int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                              const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                              const float* g_means, const tcelbo_fusion* fusion,
+                              float* grad_z, int64_t ldgz, float* grad_mu_all, int64_t ldgmu, float* grad_logvar, int64_t ldglv,
+                              const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream);
 
 /*
  * Peer-memory exchange for the row-sharded fused loss (one process per GPU; SURVEY.md 8e).  Replaces the NCCL all-gather of
@@ -270,6 +294,24 @@ int tcelbo_decomp_backward_peer(int phase, const float* z, int64_t ldz, const fl
                                 float* grad_z, int64_t ldgz, float* grad_mu_loc, int64_t ldgmu, float* grad_logvar_loc, int64_t ldglv,
                                 const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
                                 const void* const* scratch_parts, const tcelbo_peer_sync* sync, void* stream);
+/* The peer pair with the fusions of tcelbo_decomp_forward_ex / _backward_ex (same accepted and refused members; the plain peer entry
+ * points are these with fusion = NULL).  With eps, z is formed from mu_loc / logvar_loc and grad_mu_loc / grad_logvar_loc are the
+ * gradients w.r.t. the encoder outputs.  A training step is 7 launches: the publish, 3 forward, 2 in the sweep phase, 1 in the finish. */
+int tcelbo_decomp_forward_peer_ex(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv,
+                                  const float* const* mu_parts, const float* const* lv_parts, int64_t ld_part,
+                                  int b_loc, int n_ranks, int rank, int d, int64_t dataset_size, uint32_t flags, float beta,
+                                  float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                                  const tcelbo_fusion* fusion, const tcelbo_peer_sync* sync, void* workspace, size_t workspace_bytes,
+                                  void* stream);
+int tcelbo_decomp_backward_peer_ex(int phase, const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu,
+                                   const float* logvar_loc, int64_t ldlv, int b_loc, int n_ranks, int rank, int d,
+                                   int64_t dataset_size, uint32_t flags, float beta,
+                                   const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                                   const float* g_means,
+                                   float* grad_z, int64_t ldgz, float* grad_mu_loc, int64_t ldgmu, float* grad_logvar_loc, int64_t ldglv,
+                                   const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                                   const void* const* scratch_parts, const tcelbo_fusion* fusion, const tcelbo_peer_sync* sync,
+                                   void* stream);
 
 /* kl_rows[i] = -0.5 * sum_d (1 + logvar - exp(logvar) - mu^2)   (ops.py:161-163; argument order logvar, mu) */
 int tcelbo_kl_forward(const float* logvar, int64_t ldlv, const float* mu, int64_t ldmu,

@@ -63,6 +63,11 @@ _SIGNATURES = {
     "tcelbo_decomp_backward": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32, c_float,
                                        _f, _f, _f, _f, _f, _f, c_int64, _f, c_int64, _f, c_int64, c_void_p, c_size_t, c_void_p,
                                        c_size_t, c_void_p]),
+    "tcelbo_decomp_forward_ex": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32, c_float,
+                                         _f, _f, _f, _f, _f, POINTER(Fusion), c_void_p, c_size_t, c_void_p]),
+    "tcelbo_decomp_backward_ex": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32, c_float,
+                                          _f, _f, _f, _f, _f, POINTER(Fusion), _f, c_int64, _f, c_int64, _f, c_int64, c_void_p, c_size_t,
+                                          c_void_p, c_size_t, c_void_p]),
     "tcelbo_peer_publish": (c_int, [_f, c_int64, c_int, c_int, _f, POINTER(PeerSyncArgs), c_void_p]),
     "tcelbo_klloss_forward_peer": (c_int, [_f, c_int64, _f, c_int64, c_void_p, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64,
                                            c_uint32, c_float, _f, _f, _f, _f, POINTER(Fusion), POINTER(PeerSyncArgs), c_void_p, c_size_t, c_void_p]),
@@ -76,6 +81,12 @@ _SIGNATURES = {
     "tcelbo_decomp_backward_peer": (c_int, [c_int, _f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64, c_uint32,
                                             c_float, _f, _f, _f, _f, _f, _f, c_int64, _f, c_int64, _f, c_int64, c_void_p, c_size_t,
                                             c_void_p, c_size_t, c_void_p, POINTER(PeerSyncArgs), c_void_p]),
+    "tcelbo_decomp_forward_peer_ex": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_void_p, c_void_p, c_int64, c_int, c_int, c_int,
+                                              c_int, c_int64, c_uint32, c_float, _f, _f, _f, _f, _f, POINTER(Fusion), POINTER(PeerSyncArgs),
+                                              c_void_p, c_size_t, c_void_p]),
+    "tcelbo_decomp_backward_peer_ex": (c_int, [c_int, _f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, c_int, c_int, c_int64,
+                                               c_uint32, c_float, _f, _f, _f, _f, _f, _f, c_int64, _f, c_int64, _f, c_int64, c_void_p,
+                                               c_size_t, c_void_p, c_size_t, c_void_p, POINTER(Fusion), POINTER(PeerSyncArgs), c_void_p]),
     "tcelbo_kl_forward": (c_int, [_f, c_int64, _f, c_int64, c_int, c_int, _f, c_void_p]),
     "tcelbo_kl_backward": (c_int, [_f, c_int64, _f, c_int64, _f, c_int, c_int, _f, c_int64, _f, c_int64, c_void_p]),
     "tcelbo_reparam_forward": (c_int, [_f, c_int64, _f, c_int64, _f, c_int64, c_int, c_int, _f, c_int64, c_void_p]),

@@ -146,7 +146,7 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     if (int rc = check_common(z, mu_all, logvar, b_loc, b_glob, row_offset, d, dataset_size, flags, ldz, ldmu, ldlv, lf.fz.eps != nullptr)) return rc;
     if (!lf.decomp && (!log_qz || !log_qz_prod)) return fail(TCELBO_ERR_INVALID, "null output pointer");
     if (lf.fz.eps && (lf.fz.ldeps < d || (lf.fz.z_out && lf.fz.ldz_out < d))) return fail(TCELBO_ERR_INVALID, "eps / z_out row pitch smaller than d");
-    if (lf.fz.eps && (flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_UNSUPPORTED, "the fused reparameterize covers the row-variance density");
+    if (lf.fz.eps && (flags & TCELBO_VAR_COL) && !lf.decomp) return fail(TCELBO_ERR_UNSUPPORTED, "the fused reparameterize covers the row-variance density");
     if (lf.fz.expelbo && (!lf.fz.rec_rows || !lf.fz.e_rows)) return fail(TCELBO_ERR_INVALID, "expelbo needs rec_rows and e_rows");
     if (peers.on() && (flags & TCELBO_VAR_COL) && !lf.decomp)
         return fail(TCELBO_ERR_UNSUPPORTED, "the klloss peer entry points use the row-variance density; the column-variance decomposition has tcelbo_decomp_forward_peer");
@@ -169,10 +169,13 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     float* Jpart = Spart + (size_t)p.n_part_fwd * p.bl_pad * p.dp;
 
     const tcelbo_fusion& fz = lf.fz;
-    unsigned int* ticket = at<unsigned int>(workspace, p.off_red) + 4 * (size_t)p.n_fin_ctas;
+    unsigned int* ticket = at<unsigned int>(workspace, p.off_red) + kFinRedSlots * (size_t)p.n_fin_ctas;
     if (p.var_col) {
         ColPrepArgs ca;
         ca.z = z; ca.ldz = ldz; ca.mu_all = mu_all; ca.ldmu = ldmu; ca.lv_all = logvar; ca.ldlv = ldlv;
+        ca.eps = fz.eps; ca.ldeps = fz.ldeps; ca.z_out = fz.z_out; ca.ldz_out = fz.ldz_out;
+        ca.mu_loc = peers.on() ? mu_all : mu_all + (int64_t)row_offset * ldmu;        // peer mode: mu_all / logvar are this rank's rows
+        ca.lv_loc = peers.on() ? logvar : logvar + (int64_t)row_offset * ldlv;
         ca.mu_parts = peers.on() ? peers.mu_parts : nullptr; ca.lv_parts = peers.lv_parts; ca.ld_part = peers.ld_part;
         ca.b_loc = b_loc; ca.b_glob = b_glob; ca.d = d; ca.bl_pad = p.bl_pad; ca.bg_pad = p.bg_pad; ca.dp = p.dp;
         ca.colpack = mu_pad; ca.zpad = zs; ca.shift = shift; ca.ticket = ticket; ca.sync = peers.sync;
@@ -217,10 +220,13 @@ static int forward_impl(const float* z, int64_t ldz, const float* mu_all, int64_
     fin.dz = nullptr; fin.lddz = 0; fin.dmu = nullptr; fin.lddmu = 0; fin.dlv = nullptr; fin.lddlv = 0; fin.row_offset = row_offset;
     fin.dec_loss = fin.dec_mi = fin.dec_tc = fin.dec_dimkl = fin.dec_means = nullptr;
     if (lf.decomp) {
-        fin.dz = z; fin.lddz = ldz; fin.dmu = mu_all; fin.lddmu = ldmu; fin.dlv = logvar; fin.lddlv = ldlv;
+        fin.dz = fz.eps ? zs : z; fin.lddz = fz.eps ? p.dp : ldz;          // with eps: the z the prologue formed
+        fin.dmu = mu_all; fin.lddmu = ldmu; fin.dlv = logvar; fin.lddlv = ldlv;
         if (peers.on()) fin.row_offset = 0;                                 // mu_all / logvar: this rank's rows only
         fin.dec_loss = lf.loss_rows; fin.dec_mi = lf.mi_rows; fin.dec_tc = lf.tc_rows; fin.dec_dimkl = lf.dimkl_rows;
-        if (lf.means) { fin.dec_means = lf.means; fin.red_part = at<float>(workspace, p.off_red); fin.ticket = ticket; }
+        fin.dec_means = lf.means;
+        if (lf.means || fz.expelbo) { fin.red_part = at<float>(workspace, p.off_red); fin.ticket = ticket; }
+        if (fz.expelbo) { fin.rec_rows = fz.rec_rows; fin.scale = fz.scale; fin.expelbo = fz.expelbo; fin.e_rows = fz.e_rows; }
     }
     if (lf.on) {
         fin.lv = logvar; fin.ldlv = ldlv; fin.mu_loc = peers.on() ? mu_all : mu_all + (int64_t)row_offset * ldmu; fin.ldmu = ldmu;
@@ -317,7 +323,8 @@ static int backward_impl(const float* z, int64_t ldz, const float* mu_all, int64
         fa.scratch_parts = peers.on() ? peers.scratch_parts : nullptr; fa.g_off = p.boff_G; fa.n_ranks = peers.n_ranks;
         fa.eps = lf.fz.eps; fa.ldeps = lf.fz.ldeps;
         fa.sync = peers.sync;
-        fa.gc = lf.decomp ? gk : nullptr; fa.gpz = lf.decomp ? gpz : nullptr; fa.z = z; fa.ldz = ldz;   // gk holds gc (bwd_prep)
+        fa.gc = lf.decomp ? gk : nullptr; fa.gpz = lf.decomp ? gpz : nullptr;                           // gk holds gc (bwd_prep)
+        fa.z = (lf.decomp && lf.fz.eps) ? zs : z; fa.ldz = (lf.decomp && lf.fz.eps) ? p.dp : ldz;   // with eps: the prologue's z
         if (p.var_col) {
             if ((e = launch_bwd_colvar_finalize(p, fa, mu_pad, Glv, st)) != cudaSuccess) return fail_cuda(e, "bwd_colvar_finalize");
         } else {
@@ -392,23 +399,58 @@ int tcelbo_klloss_backward_ex(const float* z, int64_t ldz, const float* mu_all, 
                          workspace, workspace_bytes, scratch, scratch_bytes, stream);
 }
 
-// Checked before anything touches the device, so that a wrong call fails the same way on a machine without a GPU.
-static int check_decomp(uint32_t flags, const void* z, const void* mu_all, const void* logvar) {
+// Checked before anything touches the device, so that a wrong call fails the same way on a machine without a GPU.  With the fused
+// reparameterize (fusion->eps) z is not read and may be NULL.  The decomposition reports its batch means through `means` /
+// `g_means` only, so the klloss mean members of the fusion are refused.
+static int check_decomp(uint32_t flags, const void* z, const void* mu_all, const void* logvar, const tcelbo_fusion* fusion) {
     if (!(flags & TCELBO_VAR_COL)) return fail(TCELBO_ERR_INVALID, "the decomposition uses the column-variance density: flags need TCELBO_VAR_COL");
-    if (!z || !mu_all || !logvar) return fail(TCELBO_ERR_INVALID, "null input pointer");
+    if ((!z && !(fusion && fusion->eps)) || !mu_all || !logvar) return fail(TCELBO_ERR_INVALID, "null input pointer");
+    if (fusion && (fusion->loss_mean || fusion->kl_mean || fusion->g_loss_mean || fusion->g_kl_mean))
+        return fail(TCELBO_ERR_INVALID, "the decomposition's batch means are `means` / `g_means`: fusion.loss_mean, kl_mean, g_loss_mean and g_kl_mean must be NULL");
     return TCELBO_OK;
+}
+
+static bool decomp_has_upstream(const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                                const float* g_means, const tcelbo_fusion* fusion) {
+    return g_loss_rows || g_mi_rows || g_tc_rows || g_dimkl_rows || g_means || (fusion && fusion->g_expelbo);
+}
+
+int tcelbo_decomp_forward_ex(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                             int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                             float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                             const tcelbo_fusion* fusion, void* workspace, size_t workspace_bytes, void* stream) {
+    if (int rc = check_decomp(flags, z, mu_all, logvar, fusion)) return rc;
+    if (!loss_rows || !mi_rows || !tc_rows || !dimkl_rows) return fail(TCELBO_ERR_INVALID, "null output pointer");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.loss_rows = loss_rows; lf.mi_rows = mi_rows; lf.tc_rows = tc_rows; lf.dimkl_rows = dimkl_rows; lf.means = means;
+    if (fusion) lf.fz = *fusion;
+    return forward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
+                        nullptr, nullptr, lf, workspace, workspace_bytes, stream);
+}
+
+int tcelbo_decomp_backward_ex(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
+                              int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
+                              const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                              const float* g_means, const tcelbo_fusion* fusion,
+                              float* grad_z, int64_t ldgz, float* grad_mu_all, int64_t ldgmu, float* grad_logvar, int64_t ldglv,
+                              const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream) {
+    if (int rc = check_decomp(flags, z, mu_all, logvar, fusion)) return rc;
+    if (!grad_z || !grad_mu_all || !grad_logvar) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
+    if (!decomp_has_upstream(g_loss_rows, g_mi_rows, g_tc_rows, g_dimkl_rows, g_means, fusion)) return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.g_loss = g_loss_rows; lf.g_mi = g_mi_rows; lf.g_tc = g_tc_rows; lf.g_dimkl = g_dimkl_rows; lf.g_means = g_means;
+    if (fusion) lf.fz = *fusion;
+    return backward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
+                         nullptr, nullptr, lf, grad_z, ldgz, grad_mu_all, ldgmu, grad_logvar, ldglv,
+                         workspace, workspace_bytes, scratch, scratch_bytes, stream);
 }
 
 int tcelbo_decomp_forward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
                           int b_loc, int b_glob, int row_offset, int d, int64_t dataset_size, uint32_t flags, float beta,
                           float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
                           void* workspace, size_t workspace_bytes, void* stream) {
-    if (int rc = check_decomp(flags, z, mu_all, logvar)) return rc;
-    if (!loss_rows || !mi_rows || !tc_rows || !dimkl_rows) return fail(TCELBO_ERR_INVALID, "null output pointer");
-    LossFusion lf; lf.decomp = true; lf.beta = beta;
-    lf.loss_rows = loss_rows; lf.mi_rows = mi_rows; lf.tc_rows = tc_rows; lf.dimkl_rows = dimkl_rows; lf.means = means;
-    return forward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
-                        nullptr, nullptr, lf, workspace, workspace_bytes, stream);
+    return tcelbo_decomp_forward_ex(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags, beta,
+                                    loss_rows, mi_rows, tc_rows, dimkl_rows, means, nullptr, workspace, workspace_bytes, stream);
 }
 
 int tcelbo_decomp_backward(const float* z, int64_t ldz, const float* mu_all, int64_t ldmu, const float* logvar, int64_t ldlv,
@@ -417,14 +459,10 @@ int tcelbo_decomp_backward(const float* z, int64_t ldz, const float* mu_all, int
                            const float* g_means,
                            float* grad_z, int64_t ldgz, float* grad_mu_all, int64_t ldgmu, float* grad_logvar, int64_t ldglv,
                            const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes, void* stream) {
-    if (int rc = check_decomp(flags, z, mu_all, logvar)) return rc;
-    if (!grad_z || !grad_mu_all || !grad_logvar) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
-    if (!g_loss_rows && !g_mi_rows && !g_tc_rows && !g_dimkl_rows && !g_means) return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
-    LossFusion lf; lf.decomp = true; lf.beta = beta;
-    lf.g_loss = g_loss_rows; lf.g_mi = g_mi_rows; lf.g_tc = g_tc_rows; lf.g_dimkl = g_dimkl_rows; lf.g_means = g_means;
-    return backward_impl(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags,
-                         nullptr, nullptr, lf, grad_z, ldgz, grad_mu_all, ldgmu, grad_logvar, ldglv,
-                         workspace, workspace_bytes, scratch, scratch_bytes, stream);
+    return tcelbo_decomp_backward_ex(z, ldz, mu_all, ldmu, logvar, ldlv, b_loc, b_glob, row_offset, d, dataset_size, flags, beta,
+                                     g_loss_rows, g_mi_rows, g_tc_rows, g_dimkl_rows, g_means, nullptr,
+                                     grad_z, ldgz, grad_mu_all, ldgmu, grad_logvar, ldglv,
+                                     workspace, workspace_bytes, scratch, scratch_bytes, stream);
 }
 
 int tcelbo_klloss_forward_peer(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* const* mu_parts, int64_t ld_part,
@@ -483,12 +521,13 @@ int tcelbo_peer_publish_mu_logvar(const float* mu_loc, int64_t ldmu, const float
     return e == cudaSuccess ? TCELBO_OK : fail_cuda(e, "publish");
 }
 
-int tcelbo_decomp_forward_peer(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv,
-                               const float* const* mu_parts, const float* const* lv_parts, int64_t ld_part,
-                               int b_loc, int n_ranks, int rank, int d, int64_t dataset_size, uint32_t flags, float beta,
-                               float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
-                               const tcelbo_peer_sync* sync, void* workspace, size_t workspace_bytes, void* stream) {
-    if (int rc = check_decomp(flags, z, mu_loc, logvar_loc)) return rc;
+int tcelbo_decomp_forward_peer_ex(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv,
+                                  const float* const* mu_parts, const float* const* lv_parts, int64_t ld_part,
+                                  int b_loc, int n_ranks, int rank, int d, int64_t dataset_size, uint32_t flags, float beta,
+                                  float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                                  const tcelbo_fusion* fusion, const tcelbo_peer_sync* sync, void* workspace, size_t workspace_bytes,
+                                  void* stream) {
+    if (int rc = check_decomp(flags, z, mu_loc, logvar_loc, fusion)) return rc;
     if (!loss_rows || !mi_rows || !tc_rows || !dimkl_rows) return fail(TCELBO_ERR_INVALID, "null output pointer");
     if (!mu_parts || !lv_parts) return fail(TCELBO_ERR_INVALID, "null pointer table");
     if (sync && (!sync->flag_parts || !sync->state)) return fail(TCELBO_ERR_INVALID, "peer_sync needs the flag table and the state words");
@@ -496,10 +535,48 @@ int tcelbo_decomp_forward_peer(const float* z, int64_t ldz, const float* mu_loc,
     if ((int64_t)b_loc * n_ranks > INT32_MAX) return fail(TCELBO_ERR_INVALID, "global batch too large");
     LossFusion lf; lf.decomp = true; lf.beta = beta;
     lf.loss_rows = loss_rows; lf.mi_rows = mi_rows; lf.tc_rows = tc_rows; lf.dimkl_rows = dimkl_rows; lf.means = means;
+    if (fusion) lf.fz = *fusion;
     Peers peers; peers.mu_parts = mu_parts; peers.lv_parts = lv_parts; peers.ld_part = ld_part; peers.n_ranks = n_ranks;
     if (sync) peers.sync = PeerSync{sync->flag_parts, sync->state, 0, rank, n_ranks};
     return forward_impl(z, ldz, mu_loc, ldmu, logvar_loc, ldlv, b_loc, b_loc * n_ranks, rank * b_loc, d, dataset_size, flags,
                         nullptr, nullptr, lf, workspace, workspace_bytes, stream, peers);
+}
+
+int tcelbo_decomp_backward_peer_ex(int phase, const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu,
+                                   const float* logvar_loc, int64_t ldlv, int b_loc, int n_ranks, int rank, int d,
+                                   int64_t dataset_size, uint32_t flags, float beta,
+                                   const float* g_loss_rows, const float* g_mi_rows, const float* g_tc_rows, const float* g_dimkl_rows,
+                                   const float* g_means,
+                                   float* grad_z, int64_t ldgz, float* grad_mu_loc, int64_t ldgmu, float* grad_logvar_loc, int64_t ldglv,
+                                   const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
+                                   const void* const* scratch_parts, const tcelbo_fusion* fusion, const tcelbo_peer_sync* sync,
+                                   void* stream) {
+    if (int rc = check_decomp(flags, z, mu_loc, logvar_loc, fusion)) return rc;
+    if (!grad_z || !grad_mu_loc || !grad_logvar_loc) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
+    if (!decomp_has_upstream(g_loss_rows, g_mi_rows, g_tc_rows, g_dimkl_rows, g_means, fusion)) return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
+    if (sync && (!sync->flag_parts || !sync->state)) return fail(TCELBO_ERR_INVALID, "peer_sync needs the flag table and the state words");
+    if (phase != TCELBO_PEER_SWEEP && phase != TCELBO_PEER_FINISH) return fail(TCELBO_ERR_INVALID, "phase must be TCELBO_PEER_SWEEP or TCELBO_PEER_FINISH");
+    if (n_ranks < 1 || rank < 0 || rank >= n_ranks) return fail(TCELBO_ERR_INVALID, "bad rank / n_ranks");
+    if (phase == TCELBO_PEER_FINISH && !scratch_parts) return fail(TCELBO_ERR_INVALID, "null scratch table");
+    if ((int64_t)b_loc * n_ranks > INT32_MAX) return fail(TCELBO_ERR_INVALID, "global batch too large");
+    LossFusion lf; lf.decomp = true; lf.beta = beta;
+    lf.g_loss = g_loss_rows; lf.g_mi = g_mi_rows; lf.g_tc = g_tc_rows; lf.g_dimkl = g_dimkl_rows; lf.g_means = g_means;
+    if (fusion) lf.fz = *fusion;
+    Peers peers; peers.scratch_parts = scratch_parts; peers.n_ranks = n_ranks; peers.phase = phase;
+    if (sync) peers.sync = PeerSync{sync->flag_parts, sync->state, 1, rank, n_ranks};
+    return backward_impl(z, ldz, mu_loc, ldmu, logvar_loc, ldlv, b_loc, b_loc * n_ranks, rank * b_loc, d, dataset_size, flags,
+                         nullptr, nullptr, lf, grad_z, ldgz, grad_mu_loc, ldgmu, grad_logvar_loc, ldglv,
+                         workspace, workspace_bytes, scratch, scratch_bytes, stream, peers);
+}
+
+int tcelbo_decomp_forward_peer(const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu, const float* logvar_loc, int64_t ldlv,
+                               const float* const* mu_parts, const float* const* lv_parts, int64_t ld_part,
+                               int b_loc, int n_ranks, int rank, int d, int64_t dataset_size, uint32_t flags, float beta,
+                               float* loss_rows, float* mi_rows, float* tc_rows, float* dimkl_rows, float* means,
+                               const tcelbo_peer_sync* sync, void* workspace, size_t workspace_bytes, void* stream) {
+    return tcelbo_decomp_forward_peer_ex(z, ldz, mu_loc, ldmu, logvar_loc, ldlv, mu_parts, lv_parts, ld_part, b_loc, n_ranks, rank, d,
+                                         dataset_size, flags, beta, loss_rows, mi_rows, tc_rows, dimkl_rows, means, nullptr, sync,
+                                         workspace, workspace_bytes, stream);
 }
 
 int tcelbo_decomp_backward_peer(int phase, const float* z, int64_t ldz, const float* mu_loc, int64_t ldmu,
@@ -510,21 +587,10 @@ int tcelbo_decomp_backward_peer(int phase, const float* z, int64_t ldz, const fl
                                 float* grad_z, int64_t ldgz, float* grad_mu_loc, int64_t ldgmu, float* grad_logvar_loc, int64_t ldglv,
                                 const void* workspace, size_t workspace_bytes, void* scratch, size_t scratch_bytes,
                                 const void* const* scratch_parts, const tcelbo_peer_sync* sync, void* stream) {
-    if (int rc = check_decomp(flags, z, mu_loc, logvar_loc)) return rc;
-    if (!grad_z || !grad_mu_loc || !grad_logvar_loc) return fail(TCELBO_ERR_INVALID, "null gradient pointer");
-    if (!g_loss_rows && !g_mi_rows && !g_tc_rows && !g_dimkl_rows && !g_means) return fail(TCELBO_ERR_INVALID, "no upstream gradient given");
-    if (sync && (!sync->flag_parts || !sync->state)) return fail(TCELBO_ERR_INVALID, "peer_sync needs the flag table and the state words");
-    if (phase != TCELBO_PEER_SWEEP && phase != TCELBO_PEER_FINISH) return fail(TCELBO_ERR_INVALID, "phase must be TCELBO_PEER_SWEEP or TCELBO_PEER_FINISH");
-    if (n_ranks < 1 || rank < 0 || rank >= n_ranks) return fail(TCELBO_ERR_INVALID, "bad rank / n_ranks");
-    if (phase == TCELBO_PEER_FINISH && !scratch_parts) return fail(TCELBO_ERR_INVALID, "null scratch table");
-    if ((int64_t)b_loc * n_ranks > INT32_MAX) return fail(TCELBO_ERR_INVALID, "global batch too large");
-    LossFusion lf; lf.decomp = true; lf.beta = beta;
-    lf.g_loss = g_loss_rows; lf.g_mi = g_mi_rows; lf.g_tc = g_tc_rows; lf.g_dimkl = g_dimkl_rows; lf.g_means = g_means;
-    Peers peers; peers.scratch_parts = scratch_parts; peers.n_ranks = n_ranks; peers.phase = phase;
-    if (sync) peers.sync = PeerSync{sync->flag_parts, sync->state, 1, rank, n_ranks};
-    return backward_impl(z, ldz, mu_loc, ldmu, logvar_loc, ldlv, b_loc, b_loc * n_ranks, rank * b_loc, d, dataset_size, flags,
-                         nullptr, nullptr, lf, grad_z, ldgz, grad_mu_loc, ldgmu, grad_logvar_loc, ldglv,
-                         workspace, workspace_bytes, scratch, scratch_bytes, stream, peers);
+    return tcelbo_decomp_backward_peer_ex(phase, z, ldz, mu_loc, ldmu, logvar_loc, ldlv, b_loc, n_ranks, rank, d, dataset_size, flags, beta,
+                                          g_loss_rows, g_mi_rows, g_tc_rows, g_dimkl_rows, g_means,
+                                          grad_z, ldgz, grad_mu_loc, ldgmu, grad_logvar_loc, ldglv,
+                                          workspace, workspace_bytes, scratch, scratch_bytes, scratch_parts, nullptr, sync, stream);
 }
 
 #define ROWOP_CHECK(cond, msg) do { if (!(cond)) return fail(TCELBO_ERR_INVALID, msg); } while (0)

@@ -37,6 +37,7 @@ __device__ __forceinline__ void colpack_of(float m, float lv, float& sj, float& 
 // ticket of the finalize kernel's batch means (the workspace may be fresh, uninitialised memory).  kParts: the columns live in
 // b_loc-row blocks of different allocations (one per rank, peer-mapped); the rows (local data) are written first, then the
 // in-kernel barrier waits for every rank's publish, then the columns are gathered with volatile loads, V (1 or 4) dims per thread.
+// With eps the local rows of z are formed here from mu_loc / lv_loc (fused reparameterize) and stored to z_out if given.
 template <bool kParts, int V>
 __global__ void colvar_prep_kernel(const ColPrepArgs a) {
     const int64_t n_row = (int64_t)a.bl_pad * a.dp;
@@ -44,7 +45,16 @@ __global__ void colvar_prep_kernel(const ColPrepArgs a) {
     if (blockIdx.x == 0 && threadIdx.x == 0) *a.ticket = 0u;
     for (int64_t k = t0; k < n_row; k += stride) {
         const int i = (int)(k / a.dp), dd = (int)(k % a.dp);
-        a.zpad[k] = (i < a.b_loc && dd < a.d) ? a.z[(int64_t)i * a.ldz + dd] : 0.0f;
+        float zv = 0.0f;
+        if (i < a.b_loc && dd < a.d) {
+            if (a.eps != nullptr) {
+                zv = reparam_z(a.mu_loc[(int64_t)i * a.ldmu + dd], a.lv_loc[(int64_t)i * a.ldlv + dd], a.eps[(int64_t)i * a.ldeps + dd]);
+                if (a.z_out != nullptr) a.z_out[(int64_t)i * a.ldz_out + dd] = zv;
+            } else {
+                zv = a.z[(int64_t)i * a.ldz + dd];
+            }
+        }
+        a.zpad[k] = zv;
         a.shift[k] = 0.0f;
     }
     if (kParts && a.sync.on()) peer_barrier(a.sync);
@@ -415,13 +425,51 @@ tc_bwd_colvar_kernel(const BwdFusedArgs a) {
 // Peer exchange (a.scratch_parts != nullptr): after the barrier that says every rank's sweep is done, the column part covers this
 // rank's rows only; their mu and logvar column sums are added up over all ranks' scratch in rank order (the reduce-scatter is this
 // kernel's load phase), and mu_all / lv / grad_mu / grad_lv are this rank's rows at local indices.
+// Fused reparameterize (a.eps != nullptr, z = mu + eps * exp(lv / 2) of the local rows): the thread of local element (i, d) writes
+// grad_z[i] and also row r = row_offset + i of grad_mu / grad_lv with its own grad_z chained through z (as rows_own_mu does in
+// bwd_fused_finalize_kernel), so no thread reads another's output; the column part then skips the local rows.
 __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __restrict__ colpack, const float* __restrict__ Glv) {
     const bool peer = a.scratch_parts != nullptr;
+    const bool rows_own = a.eps != nullptr;
     if (peer && a.sync.on()) peer_barrier(a.sync);
     const int64_t n_row = (int64_t)a.b_loc * a.d;
     const int64_t n_col = (int64_t)(peer ? a.b_loc : a.b_glob) * a.d;
     const int64_t mrow0 = peer ? 0 : a.row_offset;                    // row of mu_all / lv that holds local row 0
     const size_t glv_off = a.g_off + (size_t)a.bg_pad * a.dp * sizeof(float);    // Glv follows Gpart in every rank's scratch
+    // gradients of mu / logvar at global row j (column sums, plus the condx terms of a local row)
+    auto col_grad = [&](int j, int dd, float& gmu, float& glv) {
+        const size_t o = (size_t)j * a.dp + dd;
+        const float sj = colpack[(size_t)j * 3 * a.dp + dd];
+        float gm, gl;
+        if (peer) {
+            gm = 0.0f; gl = 0.0f;
+            for (int p0 = 0; p0 < a.n_ranks; p0 += 4) {
+                float vm[4], vl[4];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const char* base = static_cast<const char*>(a.scratch_parts[p0 + q < a.n_ranks ? p0 + q : p0]);
+                    vm[q] = *reinterpret_cast<const volatile float*>(base + a.g_off + o * sizeof(float));
+                    vl[q] = *reinterpret_cast<const volatile float*>(base + glv_off + o * sizeof(float));
+                }
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    if (p0 + q < a.n_ranks) { gm += vm[q]; gl += vl[q]; }
+                }
+            }
+        } else {
+            gm = a.Gpart[o]; gl = Glv[o];
+        }
+        gmu = kTwoLn2 * sj * gm; glv = gl;
+        const int i = j - a.row_offset;
+        if (a.gc != nullptr && i >= 0 && i < a.b_loc) {
+            const float m = a.mu_all[(mrow0 + i) * a.ldmu + dd], l = a.lv[(mrow0 + i) * a.ldlv + dd];
+            float t, iv;
+            const float lp = lp_unfloored(a.z[(int64_t)i * a.ldz + dd], m, l, t, iv);
+            const float gc = lp_passes_grad(lp) ? a.gc[i] : 0.0f;
+            gmu += gc * t * iv;
+            glv += gc * 0.5f * (t * t * iv - 1.0f);
+        }
+    };
     for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n_row + n_col; idx += (int64_t)gridDim.x * blockDim.x) {
         if (idx < n_row) {
             const int i = (int)(idx / a.d), dd = (int)(idx % a.d);
@@ -439,40 +487,23 @@ __global__ void bwd_colvar_finalize_kernel(const BwdFinArgs a, const float* __re
                 gz += -gc * t * iv + -gp * t0 * iv0;
             }
             a.grad_z[(int64_t)i * a.ldgz + dd] = gz;
+            if (rows_own) {                                           // through z = mu + eps * std
+                float gmu, glv;
+                col_grad(a.row_offset + i, dd, gmu, glv);
+                const float lv = a.lv[(mrow0 + i) * a.ldlv + dd];
+                gmu += gz;
+                glv += gz * a.eps[(int64_t)i * a.ldeps + dd] * (0.5f * expf(0.5f * lv));
+                const int64_t grow = peer ? i : a.row_offset + i;
+                a.grad_mu[grow * a.ldgmu + dd] = gmu;
+                a.grad_lv[grow * a.ldglv + dd] = glv;
+            }
         } else {
             const int64_t k = idx - n_row;
             const int j = (int)(k / a.d) + (peer ? a.row_offset : 0), dd = (int)(k % a.d);
-            const size_t o = (size_t)j * a.dp + dd;
-            const float sj = colpack[(size_t)j * 3 * a.dp + dd];
-            float gm, gl;
-            if (peer) {
-                gm = 0.0f; gl = 0.0f;
-                for (int p0 = 0; p0 < a.n_ranks; p0 += 4) {
-                    float vm[4], vl[4];
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const char* base = static_cast<const char*>(a.scratch_parts[p0 + q < a.n_ranks ? p0 + q : p0]);
-                        vm[q] = *reinterpret_cast<const volatile float*>(base + a.g_off + o * sizeof(float));
-                        vl[q] = *reinterpret_cast<const volatile float*>(base + glv_off + o * sizeof(float));
-                    }
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        if (p0 + q < a.n_ranks) { gm += vm[q]; gl += vl[q]; }
-                    }
-                }
-            } else {
-                gm = a.Gpart[o]; gl = Glv[o];
-            }
-            float gmu = kTwoLn2 * sj * gm, glv = gl;
             const int i = j - a.row_offset;
-            if (a.gc != nullptr && i >= 0 && i < a.b_loc) {
-                const float m = a.mu_all[(mrow0 + i) * a.ldmu + dd], l = a.lv[(mrow0 + i) * a.ldlv + dd];
-                float t, iv;
-                const float lp = lp_unfloored(a.z[(int64_t)i * a.ldz + dd], m, l, t, iv);
-                const float gc = lp_passes_grad(lp) ? a.gc[i] : 0.0f;
-                gmu += gc * t * iv;
-                glv += gc * 0.5f * (t * t * iv - 1.0f);
-            }
+            if (rows_own && i >= 0 && i < a.b_loc) continue;          // written by the row part
+            float gmu, glv;
+            col_grad(j, dd, gmu, glv);
             const int64_t grow = peer ? i : j;                        // grad_mu / grad_lv: this rank's rows only in the peer mode
             a.grad_mu[grow * a.ldgmu + dd] = gmu;
             a.grad_lv[grow * a.ldglv + dd] = glv;

@@ -69,6 +69,10 @@ __device__ __forceinline__ float lp_unfloored(float x, float mu, float lv, float
 __device__ __forceinline__ float lp_clamped(float lp) { return fmax_nan(lp, kLogpFloor); }
 __device__ __forceinline__ bool lp_passes_grad(float lp) { return lp >= kLogpFloor; }
 
+// z = mu + eps * exp(logvar / 2) (ops.py:183-185): the one formula of tcelbo_reparam_forward and of every prologue that fuses the
+// reparameterize, so that a fused z has the bits of the standalone one
+__device__ __forceinline__ float reparam_z(float mu, float lv, float eps) { return mu + eps * expf(0.5f * lv); }
+
 // ---- mbarrier + 1-D bulk TMA (cp.async.bulk -> UBLKCP) -------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));

@@ -46,7 +46,7 @@ __global__ void prep_scalar_kernel(const PrepArgs a) {
             const float lv = a.logvar[(int64_t)i * a.ldlv + dd];
             float zv;
             if (a.eps != nullptr) {                                     // fused reparameterize, ops.py:183-185
-                zv = a.mu_loc[(int64_t)i * a.ldmu_loc + dd] + a.eps[(int64_t)i * a.ldeps + dd] * expf(0.5f * lv);
+                zv = reparam_z(a.mu_loc[(int64_t)i * a.ldmu_loc + dd], lv, a.eps[(int64_t)i * a.ldeps + dd]);
                 if (a.z_out != nullptr) a.z_out[(int64_t)i * a.ldz_out + dd] = zv;
             } else {
                 zv = a.z[(int64_t)i * a.ldz + dd];
@@ -104,7 +104,7 @@ __global__ void prep_kernel(const PrepArgs a) {
                 const float4 m4 = ld4(a.mu_loc + (int64_t)i * a.ldmu_loc + dd), e4 = ld4(a.eps + (int64_t)i * a.ldeps + dd);
                 const float mv[4] = {m4.x, m4.y, m4.z, m4.w}, ev[4] = {e4.x, e4.y, e4.z, e4.w};
 #pragma unroll
-                for (int e = 0; e < 4; ++e) zv[e] = mv[e] + ev[e] * expf(0.5f * lvv[e]);
+                for (int e = 0; e < 4; ++e) zv[e] = reparam_z(mv[e], lvv[e], ev[e]);
                 if (a.z_out != nullptr) *reinterpret_cast<float4*>(a.z_out + (int64_t)i * a.ldz_out + dd) = make_float4(zv[0], zv[1], zv[2], zv[3]);
             } else {
                 const float4 z4 = ld4(a.z + (int64_t)i * a.ldz + dd);
@@ -401,7 +401,7 @@ __global__ void fwd_finalize_kernel(const FinArgs a) {
         condx += __shfl_xor_sync(0xffffffffu, condx, o);
         pz += __shfl_xor_sync(0xffffffffu, pz, o);
     }
-    float red[4] = {0.0f, 0.0f, 0.0f, 0.0f};                // this row's share of the batch means
+    float red[kFinRedSlots] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f};   // this row's share of the batch means
     if (lane == 0 && row_ok) {
         const float2* pj = reinterpret_cast<const float2*>(a.Jpart);
         float m = kNegBig, s = 0.0f;
@@ -416,34 +416,34 @@ __global__ void fwd_finalize_kernel(const FinArgs a) {
         a.J2[row] = J2;
         if (a.log_qz != nullptr) a.log_qz[row] = lq;
         if (a.log_qz_prod != nullptr) a.log_qz_prod[row] = P;
-        if (a.lv != nullptr) {                               // red = (loss, kl, exp-ELBO, -)
+        if (a.lv != nullptr) {                               // red = (loss, kl, -, -, exp-ELBO)
             kl *= -0.5f;
             a.kl_rows[row] = kl;
             const float loss_i = (a.beta - 1.0f) * (lq - P) + kl;
             red[0] = loss_i; red[1] = kl;
             a.loss_rows[row] = loss_i;
-            if (a.rec_rows != nullptr) {
-                red[2] = expf(-2.0f * a.scale * (a.rec_rows[row] + loss_i));
-                a.e_rows[row] = red[2];
-            }
-        } else if (a.dz != nullptr) {                        // red = (loss, mi, tc, dimkl)
+        } else if (a.dz != nullptr) {                        // red = (loss, mi, tc, dimkl, exp-ELBO)
             const float mi = condx - lq, tc = lq - P, dimkl = P - pz;
             red[0] = mi + a.beta * tc + dimkl; red[1] = mi; red[2] = tc; red[3] = dimkl;
             a.dec_loss[row] = red[0]; a.dec_mi[row] = mi; a.dec_tc[row] = tc; a.dec_dimkl[row] = dimkl;
         }
+        if (a.rec_rows != nullptr) {                         // soft-intro exp-ELBO term of either loss (red[0] = loss_i)
+            red[4] = expf(-2.0f * a.scale * (a.rec_rows[row] + red[0]));
+            a.e_rows[row] = red[4];
+        }
     }
     if (a.red_part == nullptr) return;
     // ---- batch means: per-CTA partials in a fixed slot, summed in fixed order by the last CTA to arrive (deterministic)
-    __shared__ float sh[4][kFinWarps];
+    __shared__ float sh[kFinRedSlots][kFinWarps];
     __shared__ bool last;
     if (lane == 0) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) sh[q][warp] = red[q];
+        for (int q = 0; q < kFinRedSlots; ++q) sh[q][warp] = red[q];
     }
     __syncthreads();
     if (threadIdx.x == 0) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) {
+        for (int q = 0; q < kFinRedSlots; ++q) {
             float tq = 0.0f;
             for (int w = 0; w < kFinWarps; ++w) tq += sh[q][w];
             a.red_part[q * gridDim.x + blockIdx.x] = tq;
@@ -454,21 +454,21 @@ __global__ void fwd_finalize_kernel(const FinArgs a) {
     __syncthreads();
     if (!last || warp != 0) return;
     __threadfence();
-    float t[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    float t[kFinRedSlots] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f};
     for (int k = lane; k < (int)gridDim.x; k += 32) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) t[q] += *(volatile float*)(a.red_part + q * gridDim.x + k);
+        for (int q = 0; q < kFinRedSlots; ++q) t[q] += *(volatile float*)(a.red_part + q * gridDim.x + k);
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q) t[q] += __shfl_xor_sync(0xffffffffu, t[q], o);
+        for (int q = 0; q < kFinRedSlots; ++q) t[q] += __shfl_xor_sync(0xffffffffu, t[q], o);
     }
     if (lane == 0) {
         const float inv_b = 1.0f / (float)a.b_loc;
         if (a.loss_mean) a.loss_mean[0] = t[0] * inv_b;
         if (a.kl_mean) a.kl_mean[0] = t[1] * inv_b;
-        if (a.expelbo) a.expelbo[0] = t[2] * inv_b;
+        if (a.expelbo) a.expelbo[0] = t[4] * inv_b;
         if (a.dec_means) {
 #pragma unroll
             for (int q = 0; q < 4; ++q) a.dec_means[q] = t[q] * inv_b;

@@ -30,18 +30,20 @@ struct FinArgs {
     float beta; float* loss_rows; float* kl_rows;
     // optional batch-level epilogue, reduced deterministically by the last CTA to finish (fixed summation order):
     //   loss_mean = mean_i loss_rows[i], kl_mean = mean_i kl_rows[i]               (solvers/tc.py:83-89 with reduce="mean")
-    //   e_rows[i] = exp(-2*scale*(rec_rows[i] + loss_rows[i])), expelbo = mean_i e_rows[i]   (solvers/intro.py:102-103)
+    //   e_rows[i] = exp(-2*scale*(rec_rows[i] + loss_rows[i])), expelbo = mean_i e_rows[i]   (solvers/intro.py:102-103; with the
+    //   loss_rows of either the fused KL loss or the decomposition)
     float* loss_mean; float* kl_mean; const float* rec_rows; float scale; float* expelbo; float* e_rows;
     // optional MI / TC / dimension-wise KL decomposition of solvers/tc.py:91-144 (column-variance plans; dz == nullptr: off),
     // per local row i with global row r = row_offset + i:
     //   condx_i = sum_d lp(z_id; mu_rd, lv_rd), pz_i = sum_d lp(z_id; 0, 0)      (lp: tc_common.cuh lp_unfloored, clamped)
     //   mi_i = condx_i - log_qz_i, tc_i = log_qz_i - log_qz_prod_i, dimkl_i = log_qz_prod_i - pz_i, loss_i = mi_i + beta*tc_i + dimkl_i
     //   dec_means[0..3] = the batch means of loss, mi, tc, dimkl (nullptr: none)
+    // dz: the caller's z, or with the fused reparameterize the prologue's zero-padded z (the workspace's zpad, pitch dp)
     const float* dz; int64_t lddz; const float* dmu; int64_t lddmu; const float* dlv; int64_t lddlv;   // z rows; mu / logvar [b_glob]
     int row_offset;                                              // row of dmu / dlv holding local row 0 (0 with the peer exchange,
                                                                  // where dmu / dlv are this rank's rows only)
     float* dec_loss; float* dec_mi; float* dec_tc; float* dec_dimkl; float* dec_means;
-    float* red_part; unsigned int* ticket;                       // [4][gridDim.x] partial sums, arrival counter (zeroed by the prologue)
+    float* red_part; unsigned int* ticket;                       // [kFinRedSlots][gridDim.x] partial sums, arrival counter (zeroed by the prologue)
 };
 
 // One prologue kernel: pads / gathers the column operand, derives the per-(i,d) row constants, optionally forms
@@ -58,9 +60,12 @@ struct PrepArgs {
     PeerSync sync;                                               // peer exchange: barrier between the ranks' publish and this gather
 };
 
-// Column-variance prologue (tc_colvar.cu): packs (sj, nmus, c2) of every column, zero-pads the local rows of z.
+// Column-variance prologue (tc_colvar.cu): packs (sj, nmus, c2) of every column, zero-pads the local rows of z, optionally forming
+// them as z = mu + eps * exp(logvar / 2) (ops.py:183-185).
 struct ColPrepArgs {
-    const float* z; int64_t ldz;                                 // this rank's rows
+    const float* z; int64_t ldz;                                 // this rank's rows, or nullptr with eps set
+    const float* eps; int64_t ldeps; float* z_out; int64_t ldz_out;   // fused reparameterize (eps == nullptr: off; z_out optional)
+    const float* mu_loc; const float* lv_loc;                    // this rank's rows of mu / logvar (pitches ldmu / ldlv), read with eps
     const float* mu_all; int64_t ldmu; const float* lv_all; int64_t ldlv;        // [b_glob][d] columns (ignored with parts)
     const float* const* mu_parts; const float* const* lv_parts; int64_t ld_part;  // peer exchange: one [b_loc][d] block per rank
     int b_loc, b_glob, d, bl_pad, bg_pad, dp;
@@ -99,7 +104,8 @@ struct BwdFinArgs {
     // column-variance decomposition (BwdUpstream::gpz): the row-local gradients of condx_i (coefficient gc_i) and pz_i (gpz_i),
     // masked where lp < -50, on grad_z[i] and on row r = row_offset + i of grad_mu / grad_lv (nullptr: off).  With scratch_parts
     // (peer exchange) the column part covers rows [row_offset, row_offset + b_loc) only, sums the mu and logvar column sums of
-    // every rank's scratch, and mu_all / lv / grad_mu / grad_lv are this rank's rows at local indices.
+    // every rank's scratch, and mu_all / lv / grad_mu / grad_lv are this rank's rows at local indices.  With eps, z is the
+    // prologue's zpad (pitch dp) and the thread of (i, d) also writes row r of grad_mu / grad_lv, adding its own grad_z.
     const float* gc; const float* gpz; const float* z; int64_t ldz;
 };
 

@@ -14,6 +14,7 @@ constexpr int kSmallTile  = 4;        // forward column tile of the small-proble
 constexpr int kFwdWarps   = 4;
 constexpr int kBwdWarps   = 8;
 constexpr int kFinWarps   = 8;        // rows (one warp each) per CTA of the forward finalize kernel
+constexpr int kFinRedSlots = 5;       // batch means the forward finalize kernel reduces: (loss, kl | mi, -| tc, -| dimkl, exp-ELBO)
 
 inline int64_t round_up(int64_t x, int64_t m) { return (x + m - 1) / m * m; }
 
@@ -194,7 +195,7 @@ inline bool make_plan(Plan& p, int b_loc, int b_glob, int d, uint32_t flags, int
     p.off_S = off;     off = align256(off + row_arr);
     p.off_J2 = off;    off = align256(off + (size_t)p.bl_pad * sizeof(float));
     p.n_fin_ctas = (b_loc + kFinWarps - 1) / kFinWarps;
-    p.off_red = off;   off = align256(off + ((size_t)4 * p.n_fin_ctas + 4) * sizeof(float));    // 4 means per CTA, then the ticket
+    p.off_red = off;   off = align256(off + ((size_t)kFinRedSlots * p.n_fin_ctas + 4) * sizeof(float));   // the means per CTA, then the ticket
     p.ld_s2 = p.bg_pad;
     p.off_s2 = off;    off = align256(off + (p.save ? (size_t)p.bl_pad * p.ld_s2 * sizeof(float) : 0));
     const int n_part = p.n_js_fwd > p.slots_fwd ? p.n_js_fwd : p.slots_fwd;

@@ -47,8 +47,7 @@ __global__ void reparam_fwd_kernel(const float* __restrict__ mu, int64_t ldmu, c
     const int64_t n = (int64_t)b * d;
     for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < n; idx += (int64_t)gridDim.x * blockDim.x) {
         const int i = (int)(idx / d), dd = (int)(idx % d);
-        const float std = expf(0.5f * lv[(int64_t)i * ldlv + dd]);
-        z[(int64_t)i * ldz + dd] = mu[(int64_t)i * ldmu + dd] + eps[(int64_t)i * ldeps + dd] * std;
+        z[(int64_t)i * ldz + dd] = reparam_z(mu[(int64_t)i * ldmu + dd], lv[(int64_t)i * ldlv + dd], eps[(int64_t)i * ldeps + dd]);
     }
 }
 

@@ -18,7 +18,8 @@ class GraphedKLLoss:
     """``loss, dmu, dlogvar = graphed(mu, logvar, eps)`` with
 
         z    = mu + eps * exp(0.5 * logvar)                       (ops.py:183-185)
-        loss = mean_i[(beta - 1) * tc_i + kl_i]                   (solvers/tc.py:69-89, reduce="mean")
+        loss = mean_i[(beta - 1) * tc_i + kl_i]                   (loss="simple": solvers/tc.py:69-89, reduce="mean")
+        loss = mean_i[mi_i + beta * tc_i + dimkl_i]               (loss="decomp": solvers/tc.py:91-144, reduce="mean")
 
     evaluated and differentiated inside one CUDA graph.  ``mu``/``logvar``/``eps`` are ``[b_loc, d]`` fp32 CUDA
     tensors (or pinned host tensors: they are copied into the graph's static inputs on the current stream);
@@ -28,17 +29,23 @@ class GraphedKLLoss:
     ``exchange``: how the column operand and its gradient cross ranks -- ``"nccl"`` (all-gather / reduce-scatter,
     captured in the graph), ``"peer"`` (the library's own kernels over NVLink peer memory,
     :mod:`intro_tc_vae_b200.peer`), or ``"auto"`` (peer memory when it can be set up, NCCL otherwise).
-    ``mode``: ``"direct"`` drives the C ABI itself (tcelbo_klloss_forward_ex / _backward_ex with the reparameterize and
-    batch-mean fusions: 6 launches for the whole step); ``"autograd"`` records the same step through ``torch.autograd`` (the
-    public ops plus autograd's fill / accumulate kernels) and exists to cross-check the direct path.
+    ``mode``: ``"direct"`` drives the C ABI itself (tcelbo_klloss_forward_ex / _backward_ex, or for loss="decomp"
+    tcelbo_decomp_forward_ex / _backward_ex, with the reparameterize and batch-mean fusions: 6 launches for the whole step on one
+    GPU, 7 with the peer exchange); ``"autograd"`` records the same step through ``torch.autograd`` (the public ops plus autograd's
+    fill / accumulate kernels) and exists to cross-check the direct path.  ``loss="decomp"`` exchanges ``logvar`` (and its
+    gradient) as well as ``mu``, since the column-variance density of the decomposition reads every row's variance.
     ``capture=False`` issues the same launches eagerly on every call instead of replaying a graph (for profilers that
     want to see individual launches).
     """
 
     def __init__(self, b_loc: int, d: int, dataset_size: int, beta: float, device, group=None,
-                 estimator: str = "mss", warmup: int = 3, exchange: str = "nccl", mode: str = "direct", capture: bool = True):
+                 estimator: str = "mss", warmup: int = 3, exchange: str = "nccl", mode: str = "direct", capture: bool = True,
+                 loss: str = "simple"):
         if mode not in ("direct", "autograd"):
             raise ValueError(f"mode must be 'direct' or 'autograd', got {mode!r}")
+        if loss not in ("simple", "decomp"):
+            raise ValueError(f"loss must be 'simple' or 'decomp', got {loss!r}")
+        self.loss_form = loss
         if estimator not in ("mss", "mws"):
             raise ValueError(f"estimator must be 'mss' or 'mws', got {estimator!r}")
         self.device = torch.device(device)
@@ -83,7 +90,9 @@ class GraphedKLLoss:
             self.logvar.fill_(-2.0)
         if mode == "direct":
             self._alloc_direct()
-        step = self._direct_step if mode == "direct" else self._autograd_step
+            step = self._direct_step if loss == "simple" else self._direct_decomp_step
+        else:
+            step = self._autograd_step
         side = torch.cuda.Stream(device=self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
@@ -111,7 +120,10 @@ class GraphedKLLoss:
         self.mu.grad = None
         self.logvar.grad = None
         z = ops.reparameterize(self.mu, self.logvar, self.eps)
-        loss = ops.kl_tc_loss_terms(z, self.mu, self.logvar, n, beta, estimator, group, self.exchange)[0].mean()
+        if self.loss_form == "decomp":
+            loss = ops.tc_decomp_loss_mean(z, self.mu, self.logvar, n, beta, estimator, group, self.exchange)[0]
+        else:
+            loss = ops.kl_tc_loss_terms(z, self.mu, self.logvar, n, beta, estimator, group, self.exchange)[0].mean()
         loss.backward()
         return loss.detach()
 
@@ -120,7 +132,8 @@ class GraphedKLLoss:
         lib = _lib.load()
         n, beta, estimator, _ = self._args
         dev, b_loc, d = self.device, self.b_loc, self.d
-        self._flags = (_lib.EST_MSS if estimator == "mss" else _lib.EST_MWS) | _lib.VAR_ROW | _lib.SAVE_FOR_BACKWARD
+        decomp = self.loss_form == "decomp"
+        self._flags = (_lib.EST_MSS if estimator == "mss" else _lib.EST_MWS) | (_lib.VAR_COL if decomp else _lib.VAR_ROW) | _lib.SAVE_FOR_BACKWARD
         b_glob = b_loc * self.world
         if estimator == "mss" and b_glob == 1:
             raise ZeroDivisionError("float division by zero")       # ops.py:44 with M = B-1 = 0
@@ -143,6 +156,11 @@ class GraphedKLLoss:
         nccl = self.world > 1 and self.exchange is None
         self._mu_all = torch.empty(b_glob, d, **f32) if nccl else None
         self._gmu_all = torch.empty(b_glob, d, **f32) if nccl else None
+        if decomp:
+            self._means = torch.zeros(4, **f32)                           # loss, mi, tc, dimkl means, written by the finalize kernel
+            self._g_means = torch.tensor([1.0, 0.0, 0.0, 0.0], **f32)     # dLoss / d means
+            self._lv_all = torch.empty(b_glob, d, **f32) if nccl else None
+            self._glv_all = torch.empty(b_glob, d, **f32) if nccl else None
 
     def _direct_step(self) -> Tensor:
         import torch.distributed as dist
@@ -197,6 +215,62 @@ class GraphedKLLoss:
                 if phase == _lib.PEER_SWEEP:
                     exch.barrier_backward()
         return self._loss
+
+    def _direct_decomp_step(self) -> Tensor:
+        import ctypes
+        import torch.distributed as dist
+        lib = _lib.load()
+        n, beta, _, group = self._args
+        b_loc, d, flags = self.b_loc, self.d, self._flags
+        mu, lv, eps, z = self.mu, self.logvar, self.eps, self._z
+        P = lambda t: t.data_ptr()                                       # noqa: E731
+        rows = [P(t) for t in self._rows]                                # loss, mi, tc, dimkl
+        exch = self.exchange
+        fz = _lib.Fusion(eps=P(eps), ldeps=d, z_out=P(z), ldz_out=d)
+        fb = _lib.Fusion(eps=P(eps), ldeps=d)
+        with torch.cuda.device(self.device), torch.no_grad():
+            st = torch.cuda.current_stream(self.device).cuda_stream
+            if exch is None:
+                # 6 launches: prologue (reparameterize + column packing), forward sweep, finalize (+ the four means), backward
+                # prologue, sweep, finalize (+ the chain rule through z = mu + eps * std); NCCL: mu and logvar gathered around them
+                mu_all, lv_all, row_offset = mu, lv, 0
+                if self._mu_all is not None:
+                    dist.all_gather_into_tensor(self._mu_all, mu, group=group)
+                    dist.all_gather_into_tensor(self._lv_all, lv, group=group)
+                    mu_all, lv_all, row_offset = self._mu_all, self._lv_all, self.rank * b_loc
+                b_glob = mu_all.shape[0]
+                _lib.check(lib.tcelbo_decomp_forward_ex(None, 0, P(mu_all), d, P(lv_all), d, b_loc, b_glob, row_offset, d, n, flags, beta,
+                                                        *rows, P(self._means), ctypes.byref(fz), P(self._ws), self._ws.numel(), st),
+                           "tcelbo_decomp_forward_ex")
+                gmu = self._gmu_all if self._gmu_all is not None else self.dmu
+                glv = self._glv_all if self._glv_all is not None else self.dlogvar
+                _lib.check(lib.tcelbo_decomp_backward_ex(None, 0, P(mu_all), d, P(lv_all), d, b_loc, b_glob, row_offset, d, n, flags, beta,
+                                                         None, None, None, None, P(self._g_means), ctypes.byref(fb), P(self._gz), d,
+                                                         P(gmu), d, P(glv), d, P(self._ws), self._ws.numel(), P(self._scratch),
+                                                         self._sc_bytes, st), "tcelbo_decomp_backward_ex")
+                if self._gmu_all is not None:
+                    dist.reduce_scatter_tensor(self.dmu, self._gmu_all, op=dist.ReduceOp.SUM, group=group)
+                    dist.reduce_scatter_tensor(self.dlogvar, self._glv_all, op=dist.ReduceOp.SUM, group=group)
+                return self._means[0]
+            # peer-memory exchange: 7 launches (publish of mu and logvar, 3 forward, 2 in the sweep phase, 1 in the finish)
+            k = exch.next_forward()
+            exch.publish(mu, k, lv)
+            _lib.check(lib.tcelbo_decomp_forward_peer_ex(None, 0, P(mu), d, P(lv), d, P(exch.mu_tables[k]), P(exch.lv_tables[k]), d,
+                                                         b_loc, self.world, self.rank, d, n, flags, beta, *rows, P(self._means),
+                                                         ctypes.byref(fz), exch.sync_arg(), P(self._ws), self._ws.numel(), st),
+                       "tcelbo_decomp_forward_peer_ex")
+            k = exch.next_backward()
+            scratch = exch.scratch_sym[k]
+            for phase in (_lib.PEER_SWEEP, _lib.PEER_FINISH):
+                _lib.check(lib.tcelbo_decomp_backward_peer_ex(phase, None, 0, P(mu), d, P(lv), d, b_loc, self.world, self.rank, d, n,
+                                                              flags, beta, None, None, None, None, P(self._g_means),
+                                                              P(self._gz), d, P(self.dmu), d, P(self.dlogvar), d,
+                                                              P(self._ws), self._ws.numel(), P(scratch), exch.scratch_bytes,
+                                                              P(exch.scratch_tables[k]), ctypes.byref(fb), exch.sync_arg(), st),
+                           "tcelbo_decomp_backward_peer_ex")
+                if phase == _lib.PEER_SWEEP:
+                    exch.barrier_backward()
+        return self._means[0]
 
     def __call__(self, mu: Tensor, logvar: Tensor, eps: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
         with torch.no_grad():

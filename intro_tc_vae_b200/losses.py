@@ -104,13 +104,16 @@ def exp_elbo(rec_per_sample: Tensor, kl_per_sample: Tensor, scale: float) -> Ten
     return _ExpElbo.apply(rec_per_sample, kl_per_sample, float(scale))
 
 
-class _KLTCExpElbo(torch.autograd.Function):
-    """solvers/intro.py:84-89 + 102-103 in one forward / one backward evaluation of the fused loss: the per-sample
-    ``kl_i = (beta-1)*tc_i + KL_i`` of ``compute_kl_loss(reduce="none", beta=beta_neg)`` never leaves the kernels; the
-    exp-ELBO mean comes out of the forward finalize kernel and its gradient enters the backward prologue as a scalar."""
+class _FusedExpElbo(torch.autograd.Function):
+    """solvers/intro.py:84-89 + 102-103 in one forward / one backward evaluation of a fused loss: the per-sample ``kl_i`` of
+    ``compute_kl_loss(reduce="none", beta=beta_neg)`` never leaves the kernels; the exp-ELBO mean comes out of the forward finalize
+    kernel and its gradient enters the backward prologue as a scalar.  ``decomp`` selects the loss form: False is the simple
+    ``(beta-1)*tc_i + KL_i`` (solvers/tc.py:69-89, tcelbo_klloss_*_ex), True the decomposition ``mi_i + beta*tc_i + dimkl_i``
+    (solvers/tc.py:91-144, tcelbo_decomp_*_ex).  Either way the op returns 4 per-row outputs, the first of which is kl_i."""
 
     @staticmethod
-    def forward(ctx, z: Tensor, mu: Tensor, logvar: Tensor, rec_rows: Tensor, dataset_size: int, beta: float, scale: float, flags: int):
+    def forward(ctx, z: Tensor, mu: Tensor, logvar: Tensor, rec_rows: Tensor, dataset_size: int, beta: float, scale: float, flags: int,
+                decomp: bool):
         import ctypes
         lib = _lib.load()
         z, mu, logvar, rec_rows = z.contiguous(), mu.contiguous(), logvar.contiguous(), rec_rows.contiguous()
@@ -120,15 +123,18 @@ class _KLTCExpElbo(torch.autograd.Function):
         if nbytes == 0:
             raise NotImplementedError(f"tcelbo: unsupported shape b={b} d={d} (d must be <= 512)")
         ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        rows = [torch.empty(b, dtype=torch.float32, device=dev) for _ in range(5)]        # loss, kl, log_qz, log_qz_prod, e
+        rows = [torch.empty(b, dtype=torch.float32, device=dev) for _ in range(5)]        # loss, (kl, log_qz, log_qz_prod | mi, tc, dimkl), e
         out = torch.empty((), dtype=torch.float32, device=dev)
         fz = _lib.Fusion(rec_rows=rec_rows.data_ptr(), scale=scale, expelbo=out.data_ptr(), e_rows=rows[4].data_ptr())
+        args = (z.data_ptr(), d, mu.data_ptr(), d, logvar.data_ptr(), d, b, b, 0, d, dataset_size, flags, beta, *(t.data_ptr() for t in rows[:4]))
         with torch.cuda.device(dev):
-            st = lib.tcelbo_klloss_forward_ex(z.data_ptr(), d, mu.data_ptr(), d, logvar.data_ptr(), d, b, b, 0, d, dataset_size, flags, beta,
-                                              *(t.data_ptr() for t in rows[:4]), ctypes.byref(fz), ws.data_ptr(), nbytes, _stream(z))
-        _lib.check(st, "tcelbo_klloss_forward_ex")
+            if decomp:
+                st = lib.tcelbo_decomp_forward_ex(*args, None, ctypes.byref(fz), ws.data_ptr(), nbytes, _stream(z))
+            else:
+                st = lib.tcelbo_klloss_forward_ex(*args, ctypes.byref(fz), ws.data_ptr(), nbytes, _stream(z))
+        _lib.check(st, "tcelbo_decomp_forward_ex" if decomp else "tcelbo_klloss_forward_ex")
         ctx.save_for_backward(z, mu, logvar, rows[4], ws)
-        ctx.meta = (dataset_size, beta, scale, flags)
+        ctx.meta = (dataset_size, beta, scale, flags, decomp)
         ctx.mark_non_differentiable(rows[0])
         return out, rows[0]
 
@@ -137,7 +143,7 @@ class _KLTCExpElbo(torch.autograd.Function):
         import ctypes
         lib = _lib.load()
         z, mu, logvar, e_rows, ws = ctx.saved_tensors
-        dataset_size, beta, scale, flags = ctx.meta
+        dataset_size, beta, scale, flags, decomp = ctx.meta
         b, d = z.shape
         dev = z.device
         g_out = g_out.reshape(()).contiguous()
@@ -146,18 +152,18 @@ class _KLTCExpElbo(torch.autograd.Function):
         nscratch = lib.tcelbo_backward_scratch_bytes(b, b, d, flags)
         scratch = torch.empty(nscratch, dtype=torch.uint8, device=dev)
         fz = _lib.Fusion(scale=scale, e_rows=e_rows.data_ptr(), g_expelbo=g_out.data_ptr(), g_rec_rows=g_rec.data_ptr())
+        args = (z.data_ptr(), d, mu.data_ptr(), d, logvar.data_ptr(), d, b, b, 0, d, dataset_size, flags, beta)
+        tail = (gz.data_ptr(), d, gmu.data_ptr(), d, glv.data_ptr(), d, ws.data_ptr(), ws.numel(), scratch.data_ptr(), nscratch, _stream(z))
         with torch.cuda.device(dev):
-            st = lib.tcelbo_klloss_backward_ex(z.data_ptr(), d, mu.data_ptr(), d, logvar.data_ptr(), d, b, b, 0, d, dataset_size, flags, beta,
-                                               None, None, None, None, ctypes.byref(fz), gz.data_ptr(), d, gmu.data_ptr(), d, glv.data_ptr(), d,
-                                               ws.data_ptr(), ws.numel(), scratch.data_ptr(), nscratch, _stream(z))
-        _lib.check(st, "tcelbo_klloss_backward_ex")
-        return gz, gmu, glv, g_rec, None, None, None, None
+            if decomp:
+                st = lib.tcelbo_decomp_backward_ex(*args, None, None, None, None, None, ctypes.byref(fz), *tail)
+            else:
+                st = lib.tcelbo_klloss_backward_ex(*args, None, None, None, None, ctypes.byref(fz), *tail)
+        _lib.check(st, "tcelbo_decomp_backward_ex" if decomp else "tcelbo_klloss_backward_ex")
+        return gz, gmu, glv, g_rec, None, None, None, None, None
 
 
-def kl_tc_exp_elbo(z: Tensor, mu: Tensor, logvar: Tensor, rec_per_sample: Tensor, dataset_size: int, beta: float, scale: float):
-    """``exp(-2*scale*(rec_i + kl_i)).mean()`` with ``kl_i = compute_kl_loss(z, mu, logvar, reduce="none", beta=beta)``
-    (solvers/intro.py:84-89, 102-103; TC solver: solvers/tc.py:69-89) as ONE fused evaluation.  Returns
-    ``(expelbo [], kl_rows [B] (detached))``; gradients flow to z, mu, logvar and rec_per_sample.  Single GPU."""
+def _check_exp_elbo_args(z: Tensor, mu: Tensor, logvar: Tensor, rec_per_sample: Tensor) -> None:
     for name, t in (("z", z), ("mu", mu), ("logvar", logvar), ("rec_per_sample", rec_per_sample)):
         if not t.is_cuda or t.dtype != torch.float32:
             raise RuntimeError(f"{name} must be an fp32 CUDA tensor: the B200 path has no CPU fallback")
@@ -165,5 +171,22 @@ def kl_tc_exp_elbo(z: Tensor, mu: Tensor, logvar: Tensor, rec_per_sample: Tensor
         raise ValueError("z, mu, logvar must be [B, D] of one shape and rec_per_sample [B]")
     if z.shape[0] == 1:
         raise ZeroDivisionError("float division by zero")       # ops.py:44 with M = B-1 = 0
+
+
+def kl_tc_exp_elbo(z: Tensor, mu: Tensor, logvar: Tensor, rec_per_sample: Tensor, dataset_size: int, beta: float, scale: float):
+    """``exp(-2*scale*(rec_i + kl_i)).mean()`` with ``kl_i = compute_kl_loss(z, mu, logvar, reduce="none", beta=beta)``
+    (solvers/intro.py:84-89, 102-103; TC solver: solvers/tc.py:69-89) as ONE fused evaluation.  Returns
+    ``(expelbo [], kl_rows [B] (detached))``; gradients flow to z, mu, logvar and rec_per_sample.  Single GPU."""
+    _check_exp_elbo_args(z, mu, logvar, rec_per_sample)
     flags = _lib.EST_MSS | _lib.VAR_ROW | _lib.SAVE_FOR_BACKWARD
-    return _KLTCExpElbo.apply(z, mu, logvar, rec_per_sample, int(dataset_size), float(beta), float(scale), flags)
+    return _FusedExpElbo.apply(z, mu, logvar, rec_per_sample, int(dataset_size), float(beta), float(scale), flags, False)
+
+
+def tc_decomp_exp_elbo(z: Tensor, mu: Tensor, logvar: Tensor, rec_per_sample: Tensor, dataset_size: int, beta: float, scale: float):
+    """The decomposition counterpart of :func:`kl_tc_exp_elbo`: ``exp(-2*scale*(rec_i + loss_i)).mean()`` with
+    ``loss_i = mi_i + beta*tc_i + dimkl_i``, the per-sample loss of ``TCSovler._compute_kl_loss_full`` (solvers/tc.py:91-144,
+    column-variance density, MSS), as ONE forward and ONE backward evaluation.  Returns ``(expelbo [], loss_rows [B] (detached))``;
+    gradients flow to z, mu, logvar and rec_per_sample.  Single GPU."""
+    _check_exp_elbo_args(z, mu, logvar, rec_per_sample)
+    flags = _lib.EST_MSS | _lib.VAR_COL | _lib.SAVE_FOR_BACKWARD
+    return _FusedExpElbo.apply(z, mu, logvar, rec_per_sample, int(dataset_size), float(beta), float(scale), flags, True)

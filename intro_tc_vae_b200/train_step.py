@@ -12,6 +12,10 @@ host synchronisation at all:
   loss term on the library's kernels: ``reparameterize``, the fused ``(beta-1)*TC + KL`` mean (solvers/tc.py:69-89), the
   per-sample reconstruction loss (ops.py:188-236) and the exp-ELBO terms with the TC loss folded in
   (solvers/intro.py:84-103, one fused evaluation per batch);
+* ``kl_loss="full"`` trains with the beta-TCVAE decomposition ``mi + beta*tc + dimkl`` (``TCSovler._compute_kl_loss_full``,
+  solvers/tc.py:91-144) instead of the simple ``(beta-1)*TC + KL``: the KL means and the exp-ELBO terms then run on the fused
+  decomposition, and ``out`` also carries the encoder phase's ``mi`` / ``tc`` / ``dimkl`` means of the real batch (what the
+  reference writes to ``tc_decomp``);
 * data parallel: pass ``group`` -- the TC estimator is row-sharded over it (``exchange`` selects NCCL or the peer-memory
   kernels) and parameter gradients are averaged with one flattened all-reduce per phase, captured inside the graphs;
   ``SyncBatchNorm`` conversion is the caller's choice (``torch.nn.SyncBatchNorm.convert_sync_batchnorm``).
@@ -30,13 +34,17 @@ from torch import Tensor
 from torch._utils import _flatten_dense_tensors, _unflatten_dense_tensors
 
 from . import ops
-from .losses import exp_elbo, kl_tc_exp_elbo, reconstruction_loss
+from .losses import exp_elbo, kl_tc_exp_elbo, reconstruction_loss, tc_decomp_exp_elbo
 
 
 class SoftIntroTCStep:
     def __init__(self, model, optimizer_e, optimizer_d, dataset_size: int, batch_shape, *, recon_loss_type: str = "mse",
                  beta_kl: float = 1.0, beta_rec: float = 1.0, beta_neg: float = 256.0, gamma_r: float = 1e-8,
-                 clip: Optional[float] = None, group=None, exchange=None, capture: bool = True, warmup: int = 3):
+                 clip: Optional[float] = None, group=None, exchange=None, capture: bool = True, warmup: int = 3,
+                 kl_loss: str = "simple"):
+        if kl_loss not in ("simple", "full"):
+            raise ValueError(f"kl_loss must be 'simple' or 'full', got {kl_loss!r}")
+        self.kl_loss = kl_loss
         self.model, self.opt_e, self.opt_d = model, optimizer_e, optimizer_d
         self.n = int(dataset_size)
         self.kind = recon_loss_type
@@ -105,16 +113,25 @@ class SoftIntroTCStep:
         for p in self.model.decoder.parameters():
             p.requires_grad = not encoder
 
-    def _kl_mean(self, z: Tensor, mu: Tensor, logvar: Tensor) -> Tensor:
-        """compute_kl_loss(z, mu, logvar) of the TC solver with the default reduce="mean" (solvers/tc.py:58-89)."""
-        return ops.kl_tc_loss_mean(z, mu, logvar, self.n, self.beta_kl, "mss", self.group, self.exchange)[0]
+    def _kl_mean(self, z: Tensor, mu: Tensor, logvar: Tensor, record: bool = False) -> Tensor:
+        """compute_kl_loss(z, mu, logvar) of the TC solver with the default reduce="mean" (solvers/tc.py:58-144); with
+        kl_loss="full" and ``record``, the mi / tc / dimkl means go to ``out`` as the reference's tc_decomp scalars."""
+        if self.kl_loss == "simple":
+            return ops.kl_tc_loss_mean(z, mu, logvar, self.n, self.beta_kl, "mss", self.group, self.exchange)[0]
+        loss, mi, tc, dimkl = ops.tc_decomp_loss_mean(z, mu, logvar, self.n, self.beta_kl, "mss", self.group, self.exchange)
+        if record:
+            self.out.update(mi=mi.detach(), tc=tc.detach(), dimkl=dimkl.detach())
+        return loss
 
     def _exp_elbo(self, x: Tensor, recon: Tensor, z: Tensor, mu: Tensor, logvar: Tensor) -> Tensor:
         """mean_i exp(-2*scale*(beta_rec*rec_i + kl_i)), kl_i = compute_kl_loss(reduce="none", beta=beta_neg)  (solvers/intro.py:84-103)."""
         rec_rows = self.beta_rec * reconstruction_loss(x, recon, self.kind, "none")
+        full = self.kl_loss == "full"
         if self.world == 1:
-            return kl_tc_exp_elbo(z, mu, logvar, rec_rows, self.n, self.beta_neg, self.scale)[0]
-        kl_rows = ops.kl_tc_loss_terms(z, mu, logvar, self.n, self.beta_neg, "mss", self.group, self.exchange)[0]
+            fused = tc_decomp_exp_elbo if full else kl_tc_exp_elbo
+            return fused(z, mu, logvar, rec_rows, self.n, self.beta_neg, self.scale)[0]
+        terms = ops.tc_decomp_loss_terms if full else ops.kl_tc_loss_terms
+        kl_rows = terms(z, mu, logvar, self.n, self.beta_neg, "mss", self.group, self.exchange)[0]
         return exp_elbo(rec_rows, kl_rows, self.scale)
 
     def _finish(self, loss: Tensor, optimizer, params, tag: str) -> None:
@@ -141,7 +158,7 @@ class SoftIntroTCStep:
         z = ops.reparameterize(mu, logvar)
         rec = m.decoder(z)
         loss_rec = self.beta_rec * reconstruction_loss(real, rec, self.kind, "mean")
-        loss_kl = self._kl_mean(z, mu, logvar)
+        loss_kl = self._kl_mean(z, mu, logvar, record=True)
         rec_mu, rec_lv, z_rec, rec_rec = m(rec.detach())
         fake_mu, fake_lv, z_fake, rec_fake = m(fake.detach())
         ee_rec = self._exp_elbo(rec, rec_rec, z_rec, rec_mu, rec_lv)
@@ -176,7 +193,7 @@ class SoftIntroTCStep:
     def __call__(self, real: Tensor, noise: Tensor) -> Dict[str, Tensor]:
         """One update on ``real`` [B,C,H,W] with the fake-batch latents ``noise`` [B,zdim] (solvers/intro.py:61 draws them with
         ``torch.randn`` on the host).  Returns device scalars: loss_enc, loss_dec, loss_kl, loss_rec, expelbo_fake, diff_kl,
-        norm_e / norm_d (with ``clip``)."""
+        norm_e / norm_d (with ``clip``), mi / tc / dimkl (with kl_loss="full")."""
         self.real.copy_(real, non_blocking=True)
         self.noise.copy_(noise, non_blocking=True)
         if self.graph_e is not None:
